@@ -5,7 +5,7 @@ Headline (BASELINE.json configs[1], "C2"): hg19 chr1-22,X intra-chromosomal matr
 synthetic cis valid pairs, binned on the GPU and ICE-balanced (`cooler balance --ignore-diags 1
 --cis-only` semantics) to convergence.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = zero the dense tiles, bin all pairs, run the bin filters and iterate every chromosome to
 convergence.  `value` = device-resident step time (ms, lower is better); `e2e` = the same through the
@@ -25,6 +25,9 @@ The same JSON line also carries
 
 `--impl reference` times the reference's CPU path (the oracle port: the Python-2 reference cannot be
 installed) on the FULL C2 workload over all host cores -- nothing is extrapolated.
+
+`--dump-outputs DIR` writes what the last timed step returned as .npy files (see `dump_outputs`).  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -198,6 +201,42 @@ def parity_and_cpu_baseline(sample, stage, out, sizes, pairs_total, world):
     return parity, cpu
 
 
+DUMP_CELLS = 1 << 21    # matrix cells sampled by --dump-outputs: the int32 tiles of C2 are ~1.2 GB, the sample ~32 MB
+
+
+def dump_outputs(d, stage, out, rank, world):
+    """Write the result of one `LocalStage.run` step as .npy files in `d`, every value finite:
+      ice_weights      float64, one weight per bin of every chromosome; 0 = filtered bin (NaN in the weights
+                       the step returns; the weight of a kept bin is positive)
+      ice_scale, ice_var, ice_iters, ice_converged   float64, one value per chromosome; the scale is 0 where
+                       every bin of the chromosome is filtered (NaN in the step's results; the library sets the
+                       variance of such a chromosome to 0, so a non-finite variance is a fault and is written as is)
+      cells_sampled    float32 (k, 3): chromosome index, row, column of the sampled matrix cells
+      counts_sampled   float32 (k,): the binned contact counts of those cells
+    The cells are drawn uniformly over all matrix cells with a fixed seed, so the same arguments give the same
+    cells.  With several ranks every rank writes the chromosomes it holds, with a `_rank<r>` suffix, and samples
+    DUMP_CELLS / ranks cells, so that the dump stays near 33 MB in all."""
+    import torch
+    os.makedirs(d, exist_ok=True)
+    b = stage.batch
+    n = np.array(b.sizes, np.int64)
+    start = np.concatenate([[0], np.cumsum(n * n)])
+    flat = np.unique(np.random.default_rng(20240601).integers(0, start[-1], size=min(DUMP_CELLS // world, int(start[-1]))))
+    ci = np.searchsorted(start, flat, side="right") - 1
+    row, col = np.divmod(flat - start[ci], n[ci])
+    at = np.array(b.offsets, np.int64)[ci] + row * np.array(b.lds, np.int64)[ci] + col
+    res = out["results"]
+    filtered_as_zero = lambda a: np.where(np.isnan(a), 0.0, a).astype(np.float64)
+    arrays = {"ice_weights": filtered_as_zero(out["bias"].cpu().numpy()),
+              "ice_scale": filtered_as_zero(res["scale"]), "ice_var": res["var"].astype(np.float64),
+              "ice_iters": res["iters"].astype(np.float64), "ice_converged": res["converged"].astype(np.float64),
+              "cells_sampled": np.stack([ci, row, col], axis=1).astype(np.float32),
+              "counts_sampled": b.buf[torch.from_numpy(at).to(b.device)].cpu().numpy().astype(np.float32)}
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + suffix + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------
 def run_ours(args):
     import torch
@@ -280,6 +319,8 @@ def run_ours(args):
         sampler.start()
     ms_step, out = timed(step, args.steps)
     launches = (_abi.launch_count() - launches0) // args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, stage, out, rank, world)
     # roofline of the dominant kernel (the fused ICE iteration), from the same timed steps
     iters = out["results"]["iters"].astype(np.int64)
     info = out["info"]
@@ -872,8 +913,13 @@ def run_c3(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of the C2 step (`value`), and of --impl reference unless steps + warmup full steps "
+                         "exceed HC_REF_BUDGET_S (then `steps` < `steps_requested` in its line); the e2e leg times "
+                         "min(steps, 3) steps; the other sections use fixed counts: C1 3 warm-up + 5 timed, C3 the last "
+                         "of 3, C4/C5 the faster of 2 after 1 warm-up")
+    ap.add_argument("--warmup", type=int, default=3,
+                    help="untimed steps before the timed ones; at least 3 for C2 (the line reports the number run)")
     ap.add_argument("--pairs", type=int, default=400_000_000)
     ap.add_argument("--c4-pairs", type=int, default=1_000_000_000)
     ap.add_argument("--c5-pairs", type=int, default=2_000_000_000)
@@ -883,7 +929,13 @@ def main():
     ap.add_argument("--skip-c4", action="store_true", help="leave the genome-wide 10 kb section out of the line")
     ap.add_argument("--skip-secondary", action="store_true")
     ap.add_argument("--config", default="C2", choices=["C2", "C3", "C4", "C5"], help="C2 = the driver's headline workload (its line carries C4 too)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed C2 step computed (weights, ICE results, a seeded sample of the matrices) as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "C2"):
+        ap.error("--dump-outputs writes the outputs of the C2 workload of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     if args.config == "C3":

@@ -210,6 +210,23 @@ def test_inter_chromosomal_imputation_matches_reference_golden(small_genome_file
     assert fired > 1000          # the fixtures do exercise the neighbourhood vote
 
 
+def test_imputation_error_behaviour_of_the_oracle(tmp_path):
+    """The oracle half of test_oracle_vs_reference's error test, which needs no reference: NameError when the P_P
+    loop needs `M_M_sub` and the M_M loop never set it, IndexError when the stale window belongs to a coarser
+    resolution (the reference's own behaviour on the same inputs, checked live where its source is present)."""
+    import pytest
+    from test_oracle_vs_reference import _live_imputation
+    (tmp_path / "a").mkdir()
+    (tmp_path / "b").mkdir()
+    _, oracle = _live_imputation(tmp_path / "a", 204, [500000], (1500000, 2, 0.7), drop_mm_onesided=True)
+    with pytest.raises(NameError):
+        oracle({"UnImputated_Whole": {500000: {"Matrix": np.zeros((82, 82), np.int64)}}})
+    _, oracle = _live_imputation(tmp_path / "b", 205, [250000, 500000], (1500000, 2, 0.7))
+    with pytest.raises(IndexError):
+        oracle({"UnImputated_Whole": {250000: {"Matrix": np.zeros((160, 160), np.int64)},
+                                      500000: {"Matrix": np.zeros((82, 82), np.int64)}}})
+
+
 def test_building_blocks_golden():
     """oracle restatements of the reference's helper functions vs outputs of the reference itself
     (Coverage_M :904, Gap_defined :915, Gap_definedLowRes :742, Trans2symmetry :945, Correct_VC :780)."""
