@@ -74,6 +74,9 @@ SIGNATURES = {
     "hc_twostep_batch": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I32, C.POINTER(_I32), C.POINTER(_I64),
                                    C.POINTER(_I32), C.POINTER(_I64), C.POINTER(_I64), _P, C.POINTER(_I64), _P, _P, _P, _P,
                                    _P, _P]),
+    "hc_twostep_csr_batch_work_bytes": (C.c_int64, [_I64, _I64, _I32]),
+    "hc_twostep_csr_batch": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I32, _I64, _I64, _P, _P, _P, _P, _P, _P,
+                                       C.POINTER(_I64), _P, _P]),
     "hc_rownnz_f64": (C.c_int, [_P, _I64, _I32, _I32, _P, _P]),
     "hc_gap_rows": (C.c_int, [_P, _I32, _I32, _I32, _P, _P, _P, _P, _P]),
     "hc_trans2symmetry_f64": (C.c_int, [_P, _I64, _I32, _P, _P, _I64, _P]),
@@ -91,6 +94,7 @@ SIGNATURES = {
     "hc_csr_count": (C.c_int, [_P, _I64, _P, _P, C.POINTER(_I64), _P]),
     "hc_csr_emit": (C.c_int, [_P, _I64, _P, _P, _I64, _I32, _I64, _I64, _P, _P, _P, _P, _P, _P]),
     "hc_pairs_to_entries": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _P, _P, _I32, _I32, _I32, _I32, _P, _P, _P, _P]),
+    "hc_pairs_to_directed_entries": (C.c_int, [_P, _P, _P, _P, _P, _I64, _I32, _P, _P, _I32, _I32, _I32, _I32, _P, _P, _P, _P]),
     "hc_entries_count": (C.c_int, [_P, _I64, _P, _I32, _P, C.POINTER(_I64), _P]),
     "hc_entries_reduce": (C.c_int, [_P, _I64, _P, _P, _I64, _I32, _I32, _P, _P, _P, C.POINTER(_I32), _P]),
     "hc_entries_emit": (C.c_int, [_P, _I64, _P, _P, _I64, _I32, _I32, _I32, _P, _P, _P, _P, C.POINTER(_I32), _P]),

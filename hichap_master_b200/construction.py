@@ -29,8 +29,9 @@ import torch
 from . import _abi, kernels
 from .device import DenseBatch, PairColumns, require_cuda
 from .matrixBuilding import (CisCsr, GenomeWideMatrixCorrection, IntraMatrixToSparseDict, Load_Genome, Sort_Chromosomes,
-                             WholeMatrixToSparseDict, _bins_from_genome, _start_table, bin_traditional,
-                             chrom_offsets_from_bins, ice_balance_sparse, impute_inter_chromosomal)
+                             WholeMatrixToSparseDict, _bins_from_genome, _dense_bytes, _start_table, bin_traditional,
+                             bin_traditional_sparse, chrom_offsets_from_bins, dense_budget_bytes, ice_balance_sparse,
+                             impute_inter_chromosomal)
 from .pairs import read_pair_files
 
 log = logging.getLogger(__name__)
@@ -275,21 +276,27 @@ def TraditionalMatrixConstruction(OutPath, RepPath, genomeSize, wholeRes, localR
 # allelic mode
 # ======================================================================================
 class HaplotypeData:
-    """Device-resident counterpart of the reference's ``DataSets`` dictionary (:1059-1500)."""
+    """Device-resident counterpart of the reference's ``DataSets`` dictionary (:1059-1500).  A local resolution in
+    ``sparse_res`` holds ``CisCsr`` matrices (T: the cis CSR of the traditional matrices; un / imp: CSRs over the
+    concatenated haplotype bins, the imputed one general with its transpose); ``cols`` then keeps the pair columns
+    they were binned from, so that merged replicates can be re-binned."""
 
     def __init__(self):
         self.tra_whole, self.tra_local = {}, {}
         self.un_whole, self.un_local = {}, {}
         self.imp_whole, self.imp_local = {}, {}
         self.hap_bins = {}
+        self.sparse_res, self.cols = [], None
 
     def add(self, other):
+        """dense replicate merge (+=); the sparse resolutions are re-binned from all replicates' pairs by the caller"""
         for a, b in ((self.tra_whole, other.tra_whole), (self.un_whole, other.un_whole), (self.imp_whole, other.imp_whole)):
             for res in a:
                 _add_into(a[res][1], b[res][1])
         for a, b in ((self.tra_local, other.tra_local), (self.un_local, other.un_local), (self.imp_local, other.imp_local)):
             for res in a:
-                _add_into(a[res], b[res])
+                if res not in self.sparse_res:
+                    _add_into(a[res], b[res])
 
     def to_datasets(self, order):
         """the reference's DataSets layout with NumPy matrices (for parity checks / callers)"""
@@ -299,7 +306,8 @@ class HaplotypeData:
                                          ("UnImputated", self.un_whole, self.un_local, hap_order),
                                          ("Imputated", self.imp_whole, self.imp_local, hap_order)):
             out[name + "_Whole"] = {res: {"Bins": b, "Matrix": W.to_numpy(0)} for res, (b, W) in whole.items()}
-            out[name + "_Local"] = {res: {k: L.to_numpy(i) for i, k in enumerate(keys)} for res, L in local.items()}
+            out[name + "_Local"] = {res: L.matrices() if isinstance(L, CisCsr) else {k: L.to_numpy(i) for i, k in enumerate(keys)}
+                                    for res, L in local.items()}
         return out
 
 
@@ -313,11 +321,19 @@ def _haplotype_counts(bed_files, genome, wholeRes, localRes, chroms, dev, imputa
         fs = [f for f in bed_files if (tag + ".bed") in f]
         c1, p1, c2, p2, mark = read_pair_files(fs, order, chroms, "allelic")
         cols[tag] = PairColumns(c1, p1, c2, p2, mark, dev)
-    # traditional matrices: all five classes together (:1081-1094)
-    allp = PairColumns(*(torch.cat([getattr(cols[t], a) for t in cols]) for a in ("c1", "p1", "c2", "p2")), device=dev)
-    data.tra_whole, data.tra_local = bin_traditional(allp, genome, wholeRes, localRes, dev, budget=1 << 62)   # the correction reads dense tiles
     sizes = lambda res: [genome[c] // res + 1 for c in order]
-    for res in localRes:
+    budget = dense_budget_bytes(dev)
+    data.sparse_res = [res for res in localRes if _allelic_dense_bytes(sizes(res)) > budget]
+    dense_res = [res for res in localRes if res not in data.sparse_res]
+    # traditional matrices: all five classes together (:1081-1094)
+    allp = _all_pairs(cols, dev)
+    data.tra_whole, data.tra_local = bin_traditional(allp, genome, wholeRes, dense_res, dev, budget=1 << 62)   # the correction reads dense tiles
+    del allp
+    if data.sparse_res:
+        data.cols = cols
+        for res in data.sparse_res:
+            _bin_haplotype_sparse(data, cols, genome, res, dev)
+    for res in dense_res:
         # haplotype local matrices live in one batch: M chromosomes then P chromosomes
         un = DenseBatch(sizes(res) + sizes(res), dev)
         for hap, tag in ((0, "M_M"), (1, "P_P")):
@@ -351,6 +367,34 @@ def _haplotype_counts(bed_files, genome, wholeRes, localRes, chroms, dev, imputa
     return data
 
 
+def _allelic_dense_bytes(sizes) -> int:
+    """Dense working set of one local resolution in allelic mode: the traditional tiles, the un-imputed and imputed
+    maternal and paternal tiles, and the float64 corrected maternal and paternal matrices."""
+    return 5 * _dense_bytes(sizes) + 16 * sum(n * n for n in sizes)
+
+
+def _all_pairs(cols, dev):
+    """the five allelic classes as one set of pairs (the traditional matrix, matrixBuilding.py:1081-1094)"""
+    return PairColumns(*(torch.cat([getattr(cols[t], a) for t in cols]) for a in ("c1", "p1", "c2", "p2")), device=dev)
+
+
+def _bin_haplotype_sparse(data: HaplotypeData, cols, genome, res, dev):
+    """One local resolution through the sort path, for a dense working set beyond ``dense_budget_bytes``: T as the
+    cis CSR of the traditional binning, the un-imputed (Both pairs, symmetric) and imputed (Both pairs plus the
+    one-sided ones, asymmetric, with its transpose) haplotype matrices as CSRs over the concatenated haplotype bins in
+    the order of the dense batch: all M chromosomes, then all P chromosomes."""
+    order = Sort_Chromosomes(genome)
+    bins, csr = bin_traditional_sparse(_all_pairs(cols, dev), genome, res, cis_only=True, device=dev)
+    data.tra_local[res] = CisCsr(csr, bins, order)
+    hap_order = ["M" + c for c in order] + ["P" + c for c in order]
+    hb, htot = _bins_from_genome(genome, res, [(h, h[1:]) for h in hap_order])
+    chrom_bins = torch.tensor([genome[c] // res + 1 for c in order], dtype=torch.int32, device=dev)
+    parts = [(cols["M_M"], _start_table(hb, hap_order[:len(order)], dev)),
+             (cols["P_P"], _start_table(hb, hap_order[len(order):], dev))]
+    data.un_local[res] = CisCsr(kernels.pairs_to_directed_csr(parts, res, chrom_bins, htot, False, False), hb, hap_order)
+    data.imp_local[res] = CisCsr(kernels.pairs_to_directed_csr(parts, res, chrom_bins, htot, True, True), hb, hap_order)
+
+
 def _sub_batch(batch: DenseBatch, first: int, count: int) -> DenseBatch:
     """A view of ``count`` consecutive matrices of a batch (shares the buffer)."""
     sub = DenseBatch.__new__(DenseBatch)
@@ -373,7 +417,8 @@ def _sub_batch(batch: DenseBatch, first: int, count: int) -> DenseBatch:
 
 
 def _haplotype_outputs(OutPath, prefix, genome, data: HaplotypeData, wholeRes, localRes):
-    """Correction + stores of HaplotypeMatrixBuilding (matrixBuilding.py:1502-1638)."""
+    """Correction + stores of HaplotypeMatrixBuilding (matrixBuilding.py:1502-1638).  ``nor_local[res]`` holds float64
+    device matrices for a dense resolution and the upper-triangle records for a sparse one."""
     order = Sort_Chromosomes(genome)
     nchrom = len(order)
     hap_order = ["M" + c for c in order] + ["P" + c for c in order]
@@ -393,7 +438,11 @@ def _haplotype_outputs(OutPath, prefix, genome, data: HaplotypeData, wholeRes, l
         hb, W = data.un_whole[res]
         un.add(res, WholeMatrixToSparseDict(hb, W), hb)
     for res in localRes:
-        recs, _ = kernels.dense_batch_triu_records(data.un_local[res])
+        L = data.un_local[res]
+        if isinstance(L, CisCsr):
+            un.add(res, L.records())
+            continue
+        recs, _ = kernels.dense_batch_triu_records(L)
         un.add(res, {k: recs[i].copy() for i, k in enumerate(hap_order)})
     un.save()
     _say("    Two-Step balancing for Imputated Matrix ...")
@@ -406,6 +455,12 @@ def _haplotype_outputs(OutPath, prefix, genome, data: HaplotypeData, wholeRes, l
         imp.add(res, WholeMatrixToSparseDict_float(hb, nor_whole[res]), hb)
     for res in localRes:
         T, H = data.tra_local[res], data.imp_local[res]
+        if isinstance(H, CisCsr):                   # sparse: the corrected matrices come out as their upper-triangle records
+            recs, gl = kernels.twostep_csr_batch(T.csr, T.off, H.csr, H.off)
+            nor_local[res] = dict(zip(hap_order, recs))
+            gap_local[str(res)] = dict(zip(hap_order, gl))
+            imp.add(res, nor_local[res])
+            continue
         mats, gl = kernels.twostep_batch(T, H)                                            # :1031-1039, one call
         nor = {("M" if k < nchrom else "P") + order[k % nchrom]: mats[k] for k in range(2 * nchrom)}
         gaps = {("M" if k < nchrom else "P") + order[k % nchrom]: gl[k] for k in range(2 * nchrom)}
@@ -469,10 +524,11 @@ def HaplotypeMatrixConstruction(OutPath, RepPath, genomeSize, wholeRes, localRes
     CoolerPath = os.path.join(OutPath, "Cooler")
     os.makedirs(CoolerPath, exist_ok=True)
     genome = Load_Genome(genomeSize, chroms)
-    total = None
+    total, rep_cols = None, []
     for rep_p in RepPath:
         _, data = HaplotypeMatrixBuilding(CoolerPath, rep_p, genomeSize, wholeRes, localRes, Imputation_region,
                                           Imputation_min, Imputation_ratio, chroms, _return_device=True)
+        rep_cols.append(data.cols)
         if total is None:
             total = data
         else:
@@ -482,5 +538,12 @@ def HaplotypeMatrixConstruction(OutPath, RepPath, genomeSize, wholeRes, localRes
         _say("All Done !!!")
         return
     _say("Merging the Replicates...")
+    if total.sparse_res:            # sparse matrices: the merged counts are those of all replicates' pairs binned at once
+        dev = require_cuda()
+        cols = {t: PairColumns(*(torch.cat([getattr(c[t], a) for c in rep_cols]) for a in ("c1", "p1", "c2", "p2", "mark")),
+                               device=dev) for t in rep_cols[0]}
+        del rep_cols
+        for res in total.sparse_res:
+            _bin_haplotype_sparse(total, cols, genome, res, dev)
     _haplotype_outputs(CoolerPath, "Merged_", genome, total, wholeRes, localRes)
     _say("All Done !!!")

@@ -10,6 +10,7 @@ void hc_count_launch(int n = 1);
 // synchronous small device->host read through a pinned mailbox (no copy engine; see hc_abi.cu)
 cudaError_t hc_read_small(void* dst, const void* src, size_t bytes, cudaStream_t s);
 cudaMemPool_t hc_big_pool(void);      // stream-ordered pool reserved for multi-GB scratch blocks (hc_abi.cu)
+int hc_exclusive_scan_i64(int64_t* v, long long n, cudaStream_t s);   // single-CTA, in place, total to v[n] (hc_csr.cu)
 
 #define HC_CUDA(call)                                                                       \
     do {                                                                                    \

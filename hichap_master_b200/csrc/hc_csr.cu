@@ -245,6 +245,50 @@ pairs_to_entries_kernel(const int32_t* __restrict__ c1, const int32_t* __restric
     }
 }
 
+// Directed entries of the allelic haplotype matrices (cis pairs of an M_M or P_P bed).  Same cells as the tile updates of
+// hc_bin.cu: a Both pair (mark 0) counts at (b1, b2) and, off the diagonal, at (b2, b1) -- HC_BIN_SYM_BOTH; with `onesided`, an
+// R1 pair (mark 1) counts at (b1, b2) and a pair with any other non-zero mark at (b2, b1) -- HC_BIN_ONESIDED.  Two entry slots
+// per pair; an unused slot holds the padding key.
+__device__ __forceinline__ void directed_entries(int a, int x, int b, int y, int mk, FastDiv res, const int64_t* __restrict__ start,
+                                                 const int32_t* __restrict__ chrom_bins, int nchrom, int onesided, int col_bits,
+                                                 int cnt_bits, unsigned long long& e0, unsigned long long& e1,
+                                                 unsigned long long& n_valid, unsigned long long& n_oob) {
+    e0 = e1 = PAD_KEY;
+    if (a < 0 || b < 0 || a >= nchrom || b >= nchrom) return;          // filtered chromosome
+    if (mk != 0 && !onesided) return;
+    if (a != b) return;                                                // cis only
+    if (x < 0 || y < 0) { ++n_oob; return; }
+    const long long ba = fast_div((uint32_t)x, res), bb = fast_div((uint32_t)y, res);
+    if (ba >= chrom_bins[a] || bb >= chrom_bins[a]) { ++n_oob; return; }
+    const unsigned long long r = (unsigned long long)(ba + start[a]), c = (unsigned long long)(bb + start[a]);
+    const unsigned long long rc = (((r << col_bits) | c) << cnt_bits) | 1ull, cr = (((c << col_bits) | r) << cnt_bits) | 1ull;
+    if (mk == 0) { e0 = rc; if (r != c) e1 = cr; }
+    else e0 = mk == 1 ? rc : cr;
+    n_valid += 1 + (e1 != PAD_KEY);
+}
+
+__global__ void __launch_bounds__(256)
+pairs_to_directed_entries_kernel(const int32_t* __restrict__ c1, const int32_t* __restrict__ p1, const int32_t* __restrict__ c2,
+                                 const int32_t* __restrict__ p2, const uint8_t* __restrict__ mark, long long npairs, FastDiv res,
+                                 const int64_t* __restrict__ start, const int32_t* __restrict__ chrom_bins, int nchrom,
+                                 int onesided, int col_bits, int cnt_bits, unsigned long long* __restrict__ entries,
+                                 unsigned long long* __restrict__ n_valid, unsigned long long* __restrict__ oob) {
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    unsigned long long local_valid = 0, local_oob = 0;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < npairs; i += stride) {
+        ulonglong2 e;
+        directed_entries(c1[i], p1[i], c2[i], p2[i], mark[i], res, start, chrom_bins, nchrom, onesided, col_bits, cnt_bits, e.x, e.y,
+                         local_valid, local_oob);
+        reinterpret_cast<ulonglong2*>(entries)[i] = e;
+    }
+    local_valid = (unsigned long long)warp_sum_ll((long long)local_valid);
+    local_oob = (unsigned long long)warp_sum_ll((long long)local_oob);
+    if ((threadIdx.x & 31) == 0) {
+        if (local_valid) atomicAdd(n_valid, local_valid);
+        if (local_oob && oob) atomicAdd(oob, local_oob);
+    }
+}
+
 // heads per tile on the cell bits (entry >> cnt_bits)
 __global__ void __launch_bounds__(RLE_THREADS)
 ent_count_kernel(const unsigned long long* __restrict__ ent, const unsigned long long* __restrict__ n_valid_p,
@@ -576,6 +620,35 @@ extern "C" int hc_pairs_to_entries(const int32_t* c1, const int32_t* p1, const i
         pairs_to_entries_kernel<false><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
             c1, p1, c2, p2, npairs, make_fast_div((uint32_t)res), start, chrom_bins, nchrom, cis_only, col_bits, cnt_bits,
             entries, n_valid, oob);
+    HC_LAUNCH_CHECK();
+    return HC_OK;
+}
+
+// Two entries per pair (entries: 2*npairs, 16-byte aligned); *n_valid and *oob are ADDED to, so that the M_M and P_P beds can
+// fill the two halves of one buffer.
+extern "C" int hc_pairs_to_directed_entries(const int32_t* c1, const int32_t* p1, const int32_t* c2, const int32_t* p2,
+                                            const uint8_t* mark, int64_t npairs, int32_t res, const int64_t* start,
+                                            const int32_t* chrom_bins, int32_t nchrom, int32_t onesided, int32_t col_bits,
+                                            int32_t cnt_bits, unsigned long long* entries, unsigned long long* n_valid,
+                                            unsigned long long* oob, void* stream) {
+    HC_REQUIRE(npairs >= 0 && res > 0 && nchrom > 0 && col_bits > 0 && cnt_bits > 0 && cnt_bits <= 31 &&
+               2 * col_bits + cnt_bits <= 63, "sizes");
+    HC_REQUIRE(n_valid != nullptr, "n_valid");
+    if (npairs == 0) return HC_OK;
+    HC_REQUIRE(mark != nullptr, "mark column required");
+    HC_REQUIRE((reinterpret_cast<uintptr_t>(entries) & 15) == 0, "entries must be 16-byte aligned");
+    long long blocks = (npairs + 255) / 256;
+    const long long cap = (long long)hc_num_sms() * 16;
+    if (blocks > cap) blocks = cap;
+    pairs_to_directed_entries_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        c1, p1, c2, p2, mark, npairs, make_fast_div((uint32_t)res), start, chrom_bins, nchrom, onesided ? 1 : 0, col_bits, cnt_bits,
+        entries, n_valid, oob);
+    HC_LAUNCH_CHECK();
+    return HC_OK;
+}
+
+int hc_exclusive_scan_i64(int64_t* v, long long n, cudaStream_t s) {
+    csr_exclusive_scan_kernel<<<1, 1024, 0, s>>>(v, n);
     HC_LAUNCH_CHECK();
     return HC_OK;
 }

@@ -13,6 +13,7 @@
 //   sym pass WRITE   : out = RF * Sym_ij / (s_j s_i), RF = mean(X)/mean(Cor)  (reads X, writes fp64)
 // The reference's 2*N^2 interpreted iterations in Trans2symmetry become the tile-pair passes.
 // Roofline: HBM-bound, (4+4+4+4+8) N^2 = 24 N^2 bytes per haplotype matrix (+4 N^2 for TM).
+#include <limits.h>
 #include <math.h>
 #include "hc_common.cuh"
 #include <algorithm>
@@ -678,6 +679,173 @@ extern "C" int hc_twostep_batch(const int32_t* tmats, const int64_t* t_off, cons
     }
     HC_CUDA(cudaFreeAsync(scratch, s));
     HC_CUDA(cudaGetLastError());
+    return HC_OK;
+}
+
+
+// =========================================================================================
+// The same correction on CSR matrices: local resolutions of allelic mode whose dense tiles would not fit (10 kb / 5 kb).
+// Every step needs only per-row vectors and a per-cell rule, so it runs on the non-zeros: memory O(nnz + n).
+//   T  : symmetric CSR of the nchrom traditional matrices over their concatenated bins (t_bin_off)
+//   X  : general CSR of the 2*nchrom imputed haplotype matrices (all maternal, then all paternal; h_bin_off), global
+//        column indices, rows column-sorted;  XT: its transpose, same layout (diagonal entries, if any, are not read)
+// Passes, each one launch over all matrices:
+//   csr_rowstats (T, X)  row sums (int64); non-zero counts of X -- coverage counts the non-zeros of the asymmetric matrix
+//   twostep_alpha        the dense path's kernel: coverage -> gaps, alpha, percentiles (gaps are bit-exact)
+//   sym ROWSUM           row i of Sym = merge of row i of X and row i of XT with S = X / alpha[:, None] and the rule of
+//                        Trans2symmetry; s_i = rowsum(Sym)_i^(2/3), 0 -> 1 (the row sum stands in for the column sum)
+//   sym TOTAL            per row: sum_j Sym_ij / (s_i s_j), and the number of non-zero upper-triangle cells (j >= i)
+//   scan, rescale        record offsets; RF = mean(X) / mean(Cor) per matrix (the n^2 cancels)
+//   sym EMIT             upper-triangle records (bin1, bin2, IF) in chromosome-local bins, row-major
+// One thread merges one row: haplotype rows hold tens of cells at 10 kb, so a row is a short serial merge.
+// =========================================================================================
+namespace {
+
+enum { CSR_ROWSUM = 0, CSR_TOTAL = 1, CSR_EMIT = 2 };
+
+struct Rec24 { long long bin1; long long bin2; double IF; };   // matrixBuilding.py:460-461 S_dtype
+
+struct SymCsrArgs {
+    const int64_t* x_ptr; const int32_t* x_col; const int32_t* x_cnt;
+    const int64_t* xt_ptr; const int32_t* xt_col; const int32_t* xt_cnt;
+    const int64_t* t_bin_off; const int64_t* h_bin_off; int nchrom; int64_t h_nbins;
+    const double* alpha; const uint8_t* gapflag; const int32_t* ngap;
+    double* rsinv;          // [h_nbins] 1 / s_i
+    double* rowtot;         // [h_nbins] per-row sum of Cor
+    const double* scalars;  // [2*nchrom][4]: RF, mean(X), mean(Cor)
+    int64_t* rec_ptr;       // [h_nbins + 1] upper-cell counts, then their exclusive scan
+    Rec24* rec;
+};
+
+// row sums (+ non-zero counts) of a CSR, one warp per row
+__global__ void __launch_bounds__(256)
+csr_rowstats_kernel(const int64_t* __restrict__ row_ptr, const int32_t* __restrict__ cnt, int64_t nrows,
+                    int64_t* __restrict__ rowsum, int32_t* __restrict__ rownnz) {
+    const int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (r >= nrows) return;
+    long long s = 0;
+    int c = 0;
+    for (int64_t e = row_ptr[r] + lane; e < row_ptr[r + 1]; e += 32) { const int x = cnt[e]; s += x; c += (x != 0); }
+    s = warp_sum_ll(s);
+    c = warp_sum_i(c);
+    if (lane == 0) { rowsum[r] = s; if (rownnz) rownnz[r] = c; }
+}
+
+template <int PASS>
+__global__ void __launch_bounds__(256) sym_csr_kernel(SymCsrArgs a) {
+    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= a.h_nbins) return;
+    int lo = 0, hi = 2 * a.nchrom - 1;                 // matrix of the row: largest k with h_bin_off[k] <= g
+    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (a.h_bin_off[mid] <= g) lo = mid; else hi = mid - 1; }
+    const int k = lo, c = k % a.nchrom, hap = k / a.nchrom;
+    const int64_t base = a.h_bin_off[k], tb = a.t_bin_off[c] - base;     // alpha of global bin j: alpha[tb + j]
+    const bool has_gap = a.ngap[2 * c + hap] > 0;
+    const double rai = 1.0 / a.alpha[tb + g];
+    const bool gi = has_gap && a.gapflag[g];
+    const double rsi = PASS != CSR_ROWSUM ? a.rsinv[g] : 0.0;
+    const double rf = PASS == CSR_EMIT ? a.scalars[4 * k] : 0.0;
+    int64_t pa = a.x_ptr[g], pb = a.xt_ptr[g], o = PASS == CSR_EMIT ? a.rec_ptr[g] : 0;
+    const int64_t ea = a.x_ptr[g + 1], eb = a.xt_ptr[g + 1];
+    double acc = 0.0;
+    long long upper = 0;
+    while (pa < ea || pb < eb) {
+        const int ja = pa < ea ? a.x_col[pa] : INT_MAX, jb = pb < eb ? a.xt_col[pb] : INT_MAX;
+        const int j = ja < jb ? ja : jb;
+        const int xij = ja == j ? a.x_cnt[pa++] : 0;
+        const int xji = jb == j ? a.xt_cnt[pb++] : 0;
+        const double sij = i32_to_f64(xij) * rai;
+        double sym;
+        if (j == g) sym = sij;                         // the diagonal is S_ii
+        else {
+            const double sji = i32_to_f64(xji) * (1.0 / a.alpha[tb + j]);
+            if (has_gap) sym = (gi && a.gapflag[j]) ? fmax(sij, sji) : (sij + sji) * 0.5;
+            else sym = sij + sji;
+        }
+        if (PASS == CSR_ROWSUM) { acc += sym; continue; }
+        const double cor = sym * (rsi * a.rsinv[j]);
+        const bool keep = j >= g && sym != 0.0;        // the non-zeros of the dense upper triangle
+        if (PASS == CSR_TOTAL) { acc += cor; upper += keep; }
+        else if (keep) {
+            Rec24 r; r.bin1 = g - base; r.bin2 = j - base; r.IF = rf * cor;
+            a.rec[o++] = r;
+        }
+    }
+    if (PASS == CSR_ROWSUM) {
+        double s = pow(acc, 2.0 / 3.0);
+        if (s == 0.0) s = 1.0;
+        a.rsinv[g] = 1.0 / s;
+    } else if (PASS == CSR_TOTAL) {
+        a.rowtot[g] = acc;
+        a.rec_ptr[g] = upper;
+    }
+}
+
+// RF of matrix blockIdx.x from its row totals of Cor and its row sums of X (one CTA per matrix)
+__global__ void __launch_bounds__(1024) csr_rescale_factor_kernel(SymCsrArgs a, const int64_t* __restrict__ rowsum_x) {
+    const int k = blockIdx.x;
+    const int64_t base = a.h_bin_off[k];
+    const int n = (int)(a.h_bin_off[k + 1] - base);
+    if (n == 0) return;
+    vc_rescale_factor_run(a.rowtot + base, n, rowsum_x + base, n, const_cast<double*>(a.scalars) + 4 * k);
+}
+
+}  // namespace
+
+extern "C" int64_t hc_twostep_csr_batch_work_bytes(int64_t t_nbins, int64_t h_nbins, int32_t nchrom) {
+    return (int64_t)sizeof(int64_t) * (t_nbins + h_nbins) + (int64_t)sizeof(double) * (2 * t_nbins + 2 * h_nbins + 8 * (int64_t)nchrom) +
+           (int64_t)sizeof(int32_t) * h_nbins + 256;
+}
+
+extern "C" int hc_twostep_csr_batch(const int64_t* t_row_ptr, const int32_t* t_cnt, const int64_t* x_row_ptr, const int32_t* x_col,
+                                    const int32_t* x_cnt, const int64_t* xt_row_ptr, const int32_t* xt_col, const int32_t* xt_cnt,
+                                    const int64_t* t_bin_off, const int64_t* h_bin_off, int32_t nchrom, int64_t t_nbins,
+                                    int64_t h_nbins, double* alpha, uint8_t* gapflag, int32_t* gapidx, int32_t* ngap,
+                                    int64_t* rec_ptr, void* records, int64_t* h_nrec, void* work, void* stream) {
+    HC_REQUIRE(nchrom > 0 && t_nbins >= 0 && h_nbins == 2 * t_nbins && h_nrec != nullptr, "sizes (h_nbins = 2 t_nbins)");
+    HC_REQUIRE(t_row_ptr && x_row_ptr && xt_row_ptr && t_bin_off && h_bin_off && alpha && gapflag && gapidx && ngap && rec_ptr &&
+               records && work, "null pointer");      // col / cnt arrays of an empty CSR may be NULL
+    HC_REQUIRE(h_nbins < (1ll << 31), "column indices are int32");
+    cudaStream_t s = (cudaStream_t)stream;
+    *h_nrec = 0;
+    if (t_nbins == 0) return HC_OK;
+    int64_t* rs_t = reinterpret_cast<int64_t*>(work);
+    int64_t* rs_h = rs_t + t_nbins;
+    double* awork = reinterpret_cast<double*>(rs_h + h_nbins);
+    double* rsinv = awork + 2 * t_nbins;
+    double* rowtot = rsinv + h_nbins;
+    double* scalars = rowtot + h_nbins;
+    int32_t* nz_h = reinterpret_cast<int32_t*>(scalars + 8 * (int64_t)nchrom);
+
+    csr_rowstats_kernel<<<(unsigned)((t_nbins * 32 + 255) / 256), 256, 0, s>>>(t_row_ptr, t_cnt, t_nbins, rs_t, nullptr);
+    HC_LAUNCH_CHECK();
+    csr_rowstats_kernel<<<(unsigned)((h_nbins * 32 + 255) / 256), 256, 0, s>>>(x_row_ptr, x_cnt, h_nbins, rs_h, nz_h);
+    HC_LAUNCH_CHECK();
+    AlphaArgs aa;
+    aa.rs_t = rs_t; aa.rs_m = rs_h; aa.rs_p = rs_h; aa.nnz_a = nz_h; aa.nnz_b = nz_h; aa.n = 0; aa.ncols = 0;
+    aa.gap_mode = HC_GAP_PERCENTILE; aa.alpha = alpha; aa.gf_a = gapflag; aa.gf_b = gapflag; aa.gi_a = gapidx; aa.gi_b = gapidx;
+    aa.ngap = ngap; aa.work = awork; aa.q25 = 25.0 / 100.0; aa.q20 = 20.0 / 100.0;
+    aa.t_bin_off = t_bin_off; aa.h_bin_off = h_bin_off; aa.nchrom = nchrom;
+    twostep_alpha_kernel<<<nchrom, 1024, 0, s>>>(aa);
+    HC_LAUNCH_CHECK();
+
+    SymCsrArgs a;
+    a.x_ptr = x_row_ptr; a.x_col = x_col; a.x_cnt = x_cnt; a.xt_ptr = xt_row_ptr; a.xt_col = xt_col; a.xt_cnt = xt_cnt;
+    a.t_bin_off = t_bin_off; a.h_bin_off = h_bin_off; a.nchrom = nchrom; a.h_nbins = h_nbins;
+    a.alpha = alpha; a.gapflag = gapflag; a.ngap = ngap; a.rsinv = rsinv; a.rowtot = rowtot; a.scalars = scalars;
+    a.rec_ptr = rec_ptr; a.rec = reinterpret_cast<Rec24*>(records);
+    const unsigned rows = (unsigned)((h_nbins + 255) / 256);
+    sym_csr_kernel<CSR_ROWSUM><<<rows, 256, 0, s>>>(a);
+    HC_LAUNCH_CHECK();
+    sym_csr_kernel<CSR_TOTAL><<<rows, 256, 0, s>>>(a);
+    HC_LAUNCH_CHECK();
+    if (hc_exclusive_scan_i64(rec_ptr, h_nbins, s) != HC_OK) return HC_ERR_CUDA;
+    csr_rescale_factor_kernel<<<(unsigned)(2 * nchrom), 1024, 0, s>>>(a, rs_h);
+    HC_LAUNCH_CHECK();
+    sym_csr_kernel<CSR_EMIT><<<rows, 256, 0, s>>>(a);
+    HC_LAUNCH_CHECK();
+    HC_CUDA(cudaMemcpyAsync(h_nrec, rec_ptr + h_nbins, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    HC_CUDA(cudaStreamSynchronize(s));
     return HC_OK;
 }
 

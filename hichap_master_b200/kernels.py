@@ -529,6 +529,80 @@ def pairs_to_csr(pairs: PairColumns, res: int, start, chrom_bins, nbins: int, ci
     return SymCsr(row_ptr, col, cnt, nbins)
 
 
+class GenCsr(SymCsr):
+    """General (asymmetric) CSR over ``nbins`` concatenated bins, rows column-sorted, nothing mirrored.  ``t``: its
+    transpose without the diagonal (a GenCsr), when it was built."""
+    t = None
+
+
+def pairs_to_directed_csr(parts, res: int, chrom_bins, nbins: int, onesided: bool, transpose: bool) -> GenCsr:
+    """Haplotype matrices of allelic mode through the sort path.  ``parts``: [(PairColumns of an M_M / P_P bed,
+    device start table of its chromosomes in the concatenated haplotype bins)].  Both pairs count symmetrically; with
+    ``onesided`` the R1 / R2 pairs are added at (b1, b2) / (b2, b1) -- the cells of ``bin_pairs_local`` with
+    HC_BIN_SYM_BOTH then HC_BIN_ONESIDED.  Directed entries -> radix sort -> reduce-by-cell -> CSR; with ``transpose``
+    the swapped list of the same reduction, re-sorted on its row bits, becomes ``.t``.  A cell count that does not fit
+    the entry count field raises ``CountFieldOverflow``."""
+    dev = chrom_bins.device
+    cb, cnt_bits = key_col_bits(nbins), entry_cnt_bits(nbins)
+    total = sum(p.n for p, _ in parts)
+    ent = torch.empty(2 * max(total, 1), dtype=torch.int64, device=dev)
+    n_valid = torch.zeros(1, dtype=torch.int64, device=dev)
+    oob = torch.zeros(1, dtype=torch.int64, device=dev)
+    done = 0
+    for pairs, start in parts:
+        check(lib().hc_pairs_to_directed_entries(ptr(pairs.c1), ptr(pairs.p1), ptr(pairs.c2), ptr(pairs.p2), ptr(pairs.mark),
+                                                 pairs.n, int(res), ptr(start), ptr(chrom_bins), int(start.numel()),
+                                                 int(bool(onesided)), cb, cnt_bits, C.c_void_p(ent.data_ptr() + 16 * done),
+                                                 ptr(n_valid), ptr(oob), stream_ptr()), "hc_pairs_to_directed_entries")
+        done += pairs.n
+    _raise_oob(oob, "intra-chromosomal")
+    sent, free = sort_entries(ent[:2 * total], nbins, cnt_bits, 2)
+    red = reduce_entries(sent, n_valid, nbins, unit=True, lower_into=free, want_lower=transpose)
+    up = red[0] if transpose else red
+    X = GenCsr(*entries_to_csr(up, None, None, nbins, nbins), nbins)
+    if transpose:
+        _, lo, n_lo = red
+        nuniq = int(up.numel())
+        slo, _ = sort_entries(lo, nbins, cnt_bits + cb, 1, tmp=sent[:nuniq] if sent.numel() >= nuniq else None)
+        X.t = GenCsr(*entries_to_csr(slo[:int(n_lo.item())], None, None, nbins, nbins), nbins)
+    return X
+
+
+def twostep_csr_batch(T: SymCsr, t_bin_off, X: GenCsr, h_bin_off):
+    """``twostep_batch`` on CSR matrices (``hc_twostep_csr_batch``): ``T`` the symmetric CSR of the nchrom traditional
+    matrices over their concatenated bins (host offsets ``t_bin_off``), ``X`` the imputed haplotype matrices (all
+    maternal, then all paternal; host offsets ``h_bin_off``) with its transpose in ``X.t``.  Returns (list of 2*nchrom
+    S_DTYPE arrays: the upper-triangle records of every corrected matrix in chromosome-local bins, row-major -- what
+    ``IntraMatrixToSparseDict`` takes from the dense corrected matrix --, list of 2*nchrom host gap-index arrays)."""
+    nchrom = len(t_bin_off) - 1
+    dev = T.device
+    t_off = torch.from_numpy(np.ascontiguousarray(t_bin_off, dtype=np.int64)).to(dev)
+    h_off = torch.from_numpy(np.ascontiguousarray(h_bin_off, dtype=np.int64)).to(dev)
+    alpha = torch.empty(max(T.nbins, 1), dtype=torch.float64, device=dev)
+    gapflag = torch.empty(max(X.nbins, 1), dtype=torch.uint8, device=dev)
+    gapidx = torch.empty(max(X.nbins, 1), dtype=torch.int32, device=dev)
+    ngap = torch.zeros(2 * nchrom, dtype=torch.int32, device=dev)
+    rec_ptr = torch.empty(X.nbins + 1, dtype=torch.int64, device=dev)
+    recs = torch.empty(24 * max(X.nnz + X.t.nnz, 1), dtype=torch.uint8, device=dev)   # the union has at most this many cells
+    work = torch.empty(int(lib().hc_twostep_csr_batch_work_bytes(T.nbins, X.nbins, nchrom)), dtype=torch.uint8, device=dev)
+    nrec = C.c_int64(0)
+    check(lib().hc_twostep_csr_batch(ptr(T.row_ptr), ptr(T.cnt), ptr(X.row_ptr), ptr(X.col), ptr(X.cnt), ptr(X.t.row_ptr),
+                                     ptr(X.t.col), ptr(X.t.cnt), ptr(t_off), ptr(h_off), nchrom, T.nbins, X.nbins, ptr(alpha),
+                                     ptr(gapflag), ptr(gapidx), ptr(ngap), ptr(rec_ptr), ptr(recs), C.byref(nrec), ptr(work),
+                                     stream_ptr()), "hc_twostep_csr_batch")
+    bounds = rec_ptr[h_off].cpu().numpy()
+    rec = recs[:24 * int(nrec.value)].cpu().numpy().view(S_DTYPE)
+    ng, gi = ngap.cpu().numpy(), gapidx.cpu().numpy()
+    recs_out, gaps = [], []
+    for k in range(2 * nchrom):
+        recs_out.append(rec[int(bounds[k]):int(bounds[k + 1])])
+        c, hap = k % nchrom, k // nchrom
+        cnt = int(ng[2 * c + hap])
+        lo = int(h_bin_off[k])
+        gaps.append(gi[lo:lo + cnt].astype(np.int64) if cnt else np.array([]))
+    return recs_out, gaps
+
+
 def csr_upper_records(csr: SymCsr):
     """Upper-triangular (bin1, bin2, count) int32 device tensors of the local rows, row-major
     (global bin indices)."""

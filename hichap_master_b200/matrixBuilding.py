@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from . import _abi, kernels
-from .device import DenseBatch, PairColumns, require_cuda
+from .device import DenseBatch, PairColumns, as_int32_counts, require_cuda
 from .pairs import chrom_passes, read_pairs
 
 log = logging.getLogger(__name__)
@@ -124,12 +124,22 @@ def _check_fits(nbytes, dev, what):
 
 
 class CisCsr:
-    """All intra-chromosomal matrices of one resolution as ONE symmetric CSR over the concatenated bins (keys built
-    cis-only): the sparse counterpart of the per-chromosome ``DenseBatch``."""
+    """All intra-chromosomal matrices of one resolution as ONE CSR over the concatenated bins (keys built cis-only):
+    the sparse counterpart of the per-chromosome ``DenseBatch``.  Symmetric for the traditional and un-imputed
+    matrices; the imputed haplotype matrices are a general ``kernels.GenCsr``.  ``order`` names the matrices in bin
+    order (chromosomes, or M chromosomes then P chromosomes)."""
 
     def __init__(self, csr, bins, order):
         self.csr, self.bins, self.order = csr, bins, list(order)
-        self.off = chrom_offsets_from_bins(bins)
+        self.off = np.array([bins[c][0] for c in self.order] + [bins[self.order[-1]][1] + 1], dtype=np.int64)
+
+    def matrices(self):
+        """{chrom: scipy.sparse.csr_matrix (int64 counts)}: the per-chromosome blocks of the CSR"""
+        import scipy.sparse as sp
+        c = self.csr
+        full = sp.csr_matrix((c.cnt.cpu().numpy().astype(np.int64), c.col.cpu().numpy(), c.row_ptr.cpu().numpy()),
+                             shape=(c.nbins, c.nbins))
+        return {name: full[a:b, a:b] for name, a, b in zip(self.order, self.off[:-1], self.off[1:])}
 
     def records(self):
         """{chrom: upper-triangular S_dtype records in chromosome-local coordinates} (matrixBuilding.py:508-524)"""
@@ -477,8 +487,53 @@ def two_step_device(T: DenseBatch, ti: int, M: DenseBatch, mi: int, P: DenseBatc
     return nor_m, nor_p, _gap_array(gi_m, int(ng[0])), _gap_array(gi_p, int(ng[1]))
 
 
+def _is_sparse(*mats):
+    import scipy.sparse as sp
+    return any(sp.issparse(m) for m in mats)
+
+
+def _device_csr(m, cls):
+    """host matrix of integer counts (scipy.sparse or dense) -> device CSR: duplicates summed, explicit zeros dropped
+    (coverage counts the stored entries), columns sorted"""
+    import scipy.sparse as sp
+    m = sp.csr_matrix(m, copy=True)
+    m.sum_duplicates()
+    m.eliminate_zeros()
+    m.sort_indices()
+    dev = require_cuda()
+    up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt)).to(dev)
+    return cls(up(m.indptr, np.int64), up(m.indices, np.int32), up(as_int32_counts(m.data), np.int32), m.shape[0])
+
+
+def _twostep_sparse(tra, hap):
+    """TwoStepCorrection of nchrom chromosomes on the CSR path: ``tra`` nchrom square count matrices, ``hap`` their
+    2*nchrom haplotype matrices (all M, then all P).  Returns (2*nchrom symmetric float64 scipy CSR matrices, both
+    triangles stored, and 2*nchrom gap arrays)."""
+    import scipy.sparse as sp
+    sizes = [m.shape[0] for m in tra]
+    if any(m.shape != (n, n) for m, n in zip(list(tra) + list(hap), sizes * 3)) or len(hap) != 2 * len(tra):
+        raise ValueError("square traditional and haplotype matrices of matching sides expected")
+    t_off = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+    h_off = np.concatenate([[0], np.cumsum(sizes + sizes)]).astype(np.int64)
+    H = sp.block_diag(hap, format="csr")
+    X = _device_csr(H, kernels.GenCsr)
+    X.t = _device_csr(H.T, kernels.GenCsr)
+    recs, gaps = kernels.twostep_csr_batch(_device_csr(sp.block_diag(tra, format="csr"), kernels.SymCsr), t_off, X, h_off)
+    mats = []
+    for r, n in zip(recs, sizes + sizes):
+        b1, b2, v = r["bin1"], r["bin2"], r["IF"]
+        off = b1 != b2
+        mats.append(sp.csr_matrix((np.concatenate([v, v[off]]), (np.concatenate([b1, b2[off]]), np.concatenate([b2, b1[off]]))),
+                                  shape=(n, n)))
+    return mats, gaps
+
+
 def TwoStepCorrection(TM, MM, PM):
-    """matrixBuilding.py:984-1023 -> (Nor_MM, Nor_PM, Gap_M, Gap_P)."""
+    """matrixBuilding.py:984-1023 -> (Nor_MM, Nor_PM, Gap_M, Gap_P).  With ``scipy.sparse`` inputs the correction runs
+    on the non-zeros (``hc_twostep_csr_batch``) and Nor_MM / Nor_PM are symmetric ``scipy.sparse`` CSR matrices."""
+    if _is_sparse(TM, MM, PM):
+        mats, gaps = _twostep_sparse([TM], [MM, PM])
+        return mats[0], mats[1], gaps[0], gaps[1]
     b = DenseBatch.from_numpy([np.asarray(TM), np.asarray(MM), np.asarray(PM)])
     nor_m, nor_p, gap_m, gap_p = two_step_device(b, 0, b, 1, b, 2)
     return nor_m.cpu().numpy(), nor_p.cpu().numpy(), gap_m, gap_p
@@ -486,8 +541,13 @@ def TwoStepCorrection(TM, MM, PM):
 
 def IntraChromMatrixCorrection(Tra_Lib, Hap_Lib):
     """matrixBuilding.py:1026-1041 -> (Nor_Lib, Gap_Lib) keyed 'M'+chrom / 'P'+chrom.  All
-    chromosomes are corrected by one batched library call (``kernels.twostep_batch``)."""
+    chromosomes are corrected by one batched library call (``kernels.twostep_batch``; with ``scipy.sparse``
+    inputs ``kernels.twostep_csr_batch``, and the corrected matrices are symmetric ``scipy.sparse`` CSR)."""
     chros = list(Tra_Lib.keys())
+    if _is_sparse(*Tra_Lib.values(), *Hap_Lib.values()):
+        mats, gaps = _twostep_sparse([Tra_Lib[c] for c in chros], [Hap_Lib["M" + c] for c in chros] + [Hap_Lib["P" + c] for c in chros])
+        keys = ["M" + c for c in chros] + ["P" + c for c in chros]
+        return dict(zip(keys, mats)), dict(zip(keys, gaps))
     T = DenseBatch.from_numpy([np.asarray(Tra_Lib[c]) for c in chros])
     H = DenseBatch.from_numpy([np.asarray(Hap_Lib["M" + c]) for c in chros] +
                               [np.asarray(Hap_Lib["P" + c]) for c in chros])

@@ -290,6 +290,19 @@ int hc_entries_emit(const unsigned long long* sorted, int64_t n, const unsigned 
                     unsigned long long* lo, unsigned long long* n_lo, int32_t* d_overflow, int32_t* h_overflow, void* stream);
 int hc_entries_transpose(const unsigned long long* up, int64_t n, int32_t col_bits, int32_t cnt_bits,
                          unsigned long long* lo, unsigned long long* n_lo, void* stream);
+/* Directed entries of the allelic haplotype matrices: two slots per pair (entries[2*npairs], 16-byte aligned), cis pairs
+ * of an M_M or P_P bed routed through `start` (the M or P offsets of the concatenated haplotype bins).  A Both pair
+ * (mark 0) gives (b1, b2) and, off the diagonal, (b2, b1) -- the cells of HC_BIN_SYM_BOTH; with `onesided`, an R1 pair
+ * (mark 1) gives (b1, b2) and a pair with any other non-zero mark (b2, b1) -- the cells of HC_BIN_ONESIDED
+ * (matrixBuilding.py:1153-1161, :1295-1301).  Unused slots hold the padding key.  *n_valid and *oob are ADDED to (not
+ * reset), so the two beds can fill the two halves of one buffer.  Sorted on 2*col_bits bits and reduced with
+ * hc_entries_count / hc_entries_emit, the entries give the rows of a general (asymmetric) CSR; the swapped list of
+ * hc_entries_emit, re-sorted on its row bits, gives its transpose without the diagonal. */
+int hc_pairs_to_directed_entries(const int32_t* c1, const int32_t* p1, const int32_t* c2, const int32_t* p2,
+                                 const uint8_t* mark, int64_t npairs, int32_t res, const int64_t* start,
+                                 const int32_t* chrom_bins, int32_t nchrom, int32_t onesided, int32_t col_bits,
+                                 int32_t cnt_bits, unsigned long long* entries, unsigned long long* n_valid,
+                                 unsigned long long* oob, void* stream);
 int64_t hc_entries_csr_work_bytes(int64_t nrows);
 int hc_entries_to_csr(const unsigned long long* up, int64_t n_up, const unsigned long long* lo,
                       const unsigned long long* n_lo, int32_t col_bits, int32_t cnt_bits, int64_t row0,
@@ -382,6 +395,25 @@ int hc_twostep_batch(const int32_t* tmats, const int64_t* t_off, const int32_t* 
                      const int64_t* h_hoff, const int32_t* h_hld, const int64_t* h_tbin, const int64_t* h_hbin,
                      double* out, const int64_t* h_out_off, double* alpha, uint8_t* gapflag, int32_t* gapidx,
                      int32_t* ngap, void* work, void* stream);
+
+/* hc_twostep_batch on CSR matrices, for local resolutions whose dense tiles would not fit: memory O(nnz + n).
+ * T: symmetric CSR (row_ptr, cnt) of the nchrom traditional matrices over t_nbins concatenated bins (t_bin_off,
+ * device, nchrom+1).  X: general CSR (row_ptr int64, col int32 = global bin, cnt int32; rows column-sorted) of the
+ * 2*nchrom imputed haplotype matrices (all maternal, then all paternal; h_bin_off, device, 2*nchrom+1; h_nbins =
+ * 2*t_nbins).  XT: the transpose of X in the same layout (its diagonal is not read).  Same arithmetic as the dense
+ * batch: row sums and coverage (non-zeros of the asymmetric X), gaps / alpha by the same kernel (bit-exact gaps),
+ * Trans2symmetry on the union pattern of X and XT, Correct_VC(2/3) with the row sum for the column sum, RF =
+ * sum(X) / sum(Cor).  Outputs: alpha, gapflag, gapidx, ngap as hc_twostep_batch; rec_ptr[h_nbins+1] the offsets of
+ * every row's records; records: 24-byte (int64 bin1, int64 bin2, float64 IF) upper-triangle records of every matrix,
+ * chromosome-local bins, row-major, matrix k starting at rec_ptr[h_bin_off[k]] -- room for nnz(X) + nnz(XT) records;
+ * *h_nrec the number written (synchronises; the only host round trip).
+ * work: hc_twostep_csr_batch_work_bytes(t_nbins, h_nbins, nchrom). */
+int64_t hc_twostep_csr_batch_work_bytes(int64_t t_nbins, int64_t h_nbins, int32_t nchrom);
+int hc_twostep_csr_batch(const int64_t* t_row_ptr, const int32_t* t_cnt, const int64_t* x_row_ptr, const int32_t* x_col,
+                         const int32_t* x_cnt, const int64_t* xt_row_ptr, const int32_t* xt_col, const int32_t* xt_cnt,
+                         const int64_t* t_bin_off, const int64_t* h_bin_off, int32_t nchrom, int64_t t_nbins,
+                         int64_t h_nbins, double* alpha, uint8_t* gapflag, int32_t* gapidx, int32_t* ngap,
+                         int64_t* rec_ptr, void* records, int64_t* h_nrec, void* work, void* stream);
 
 /* The reference's own building blocks, separately callable (SURVEY.md section 8b keeps Correct_VC(X, alpha)
  * among the signatures; hc_twostep_correct fuses all of them for the int32 tiles).  Float64 matrices,
