@@ -7,7 +7,6 @@
 // Roofline: HBM-bound streaming read of the columnar pairs (16 B/pair, +1 B mark) with 128-bit
 // loads; the += 1 updates are 32-bit RED atomics resolved in L2 (not HBM traffic).
 #include <algorithm>
-#include <cooperative_groups.h>
 #include <stdlib.h>
 #include "hc_common.cuh"
 
@@ -232,29 +231,25 @@ __global__ void __launch_bounds__(BIN_THREADS) bin_pairs_band_kernel(BandArgs a)
     }
 }
 
-// ---- cluster variant: the hottest diagonals are counted in DISTRIBUTED SHARED MEMORY ---------------------------
+// ---- hot-diagonal variant: the hottest diagonals are counted in SHARED MEMORY ----------------------------------
 // The banded kernel above is bound by the L2 atomic rate (~80 G RED/s measured: 400 M pairs = 5 ms).  Half of all
-// Hi-C pairs fall on the first few diagonals (P(s) ~ 1/s), so a thread-block cluster keeps 16-bit counters for the
-// diagonals d < d_hot of EVERY bin in the shared memory of its CTAs (cluster of 8 x 200 KB = 800 K counters = 10
-// diagonals of the 75 918 bins of hg19 at 40 kb): a pair on a hot diagonal becomes one shared-memory atomic on the
-// CTA that owns the counter (distributed shared memory), and only the other pairs go to L2 (band) / DRAM (far
-// pairs).  At the end of the launch every CTA adds its non-zero counters into the band.  A counter that reaches
-// 0x8000 is drained into the band by the thread that saw it cross (at most 8 x 1024 threads can add in between, so the
-// 16-bit field never carries into its neighbour).
+// Hi-C pairs fall on the first few diagonals (P(s) ~ 1/s), so every CTA keeps 16-bit counters for the diagonals
+// d < d_hot of EVERY bin in its own 200 KB of shared memory (100 K counters: the main diagonal of the 75 918 bins of
+// hg19 at 40 kb): a pair on a hot diagonal becomes one shared-memory atomic, and only the other pairs go to L2 (band)
+// / DRAM (far pairs).  At the end of the launch every CTA adds its non-zero counters into the band.  A counter that
+// reaches 0x8000 is drained into the band by the thread that saw it cross (only the 1024 threads of the CTA can add in
+// between, so the 16-bit field never carries into its neighbour).
 constexpr int HOT_THREADS = 1024;
 constexpr int HOT_PER_CTA = 100 * 1024;          // 16-bit counters per CTA (200 KB of shared memory)
 constexpr int HOT_MAX_D = 16;
 
 template <bool U8>
-__global__ void __launch_bounds__(HOT_THREADS, 1) bin_pairs_band_cluster_kernel(BandArgs a) {
-    namespace cg = cooperative_groups;
+__global__ void __launch_bounds__(HOT_THREADS, 1) bin_pairs_band_hot_kernel(BandArgs a) {
     extern __shared__ __align__(16) uint32_t hot[];          // HOT_PER_CTA / 2 words
-    cg::cluster_group cluster = cg::this_cluster();
-    const unsigned csize = cluster.num_blocks(), crank = cluster.block_rank();
     const long long nbins = a.bin_off[a.nchrom];
-    const int d_hot = (int)min((long long)HOT_MAX_D, nbins > 0 ? (long long)csize * HOT_PER_CTA / nbins : 0ll);
+    const int d_hot = (int)min((long long)HOT_MAX_D, nbins > 0 ? (long long)HOT_PER_CTA / nbins : 0ll);
     for (int i = threadIdx.x; i < HOT_PER_CTA / 2; i += blockDim.x) hot[i] = 0u;
-    cluster.sync();
+    __syncthreads();
     const int64_t nvec = a.npairs / PAIRS_PER_THREAD;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     unsigned long long my_oob = 0;
@@ -271,9 +266,8 @@ __global__ void __launch_bounds__(HOT_THREADS, 1) bin_pairs_band_cluster_kernel(
         const long long grow = a.bin_off[c1] + lo;
         if ((int)d < d_hot) {
             const unsigned idx = (unsigned)(grow * d_hot + d);
-            const unsigned owner = idx / HOT_PER_CTA, local = idx - owner * HOT_PER_CTA;
-            uint32_t* w = (csize == 1u ? hot : cluster.map_shared_rank(hot, owner)) + (local >> 1);   // csize 1: plain shared-memory atomic
-            const unsigned sh = (local & 1u) * 16u;
+            uint32_t* w = hot + (idx >> 1);
+            const unsigned sh = (idx & 1u) * 16u;
             const uint32_t old = atomicAdd(w, 1u << sh);
             if (((old >> sh) & 0xffffu) == 0x7fffu) {          // this add made it 0x8000: drain that much into the band
                 atomicSub(w, 0x8000u << sh);
@@ -305,7 +299,7 @@ __global__ void __launch_bounds__(HOT_THREADS, 1) bin_pairs_band_cluster_kernel(
         const int x = U8 ? (int)c1b[i] : a.in.c1[i], y = U8 ? (int)c2b[i] : a.in.c2[i];
         apply(x, a.in.p1[i], y, a.in.p2[i], a.in.mark ? a.in.mark[i] : 0);
     }
-    cluster.sync();            // every remote add has landed; nobody touches this CTA's counters any more
+    __syncthreads();           // every add has landed; nobody touches the counters any more
     if (d_hot > 0) {
         for (int i = threadIdx.x; i < HOT_PER_CTA / 2; i += blockDim.x) {
             const uint32_t w = hot[i];
@@ -314,7 +308,7 @@ __global__ void __launch_bounds__(HOT_THREADS, 1) bin_pairs_band_cluster_kernel(
             for (int h = 0; h < 2; ++h) {
                 const int v = (int)((w >> (16 * h)) & 0xffffu);
                 if (v) {
-                    const unsigned idx = crank * HOT_PER_CTA + 2u * i + h;
+                    const unsigned idx = 2u * i + h;
                     const long long grow = idx / d_hot;
                     const int d = (int)(idx - grow * d_hot);
                     if (grow < nbins) red_add_s32_hint(a.band + ((grow << a.bw_shift) + d), v, keep);
@@ -516,27 +510,13 @@ extern "C" int hc_bin_band_accumulate(const void* c1, const int32_t* p1, const v
     a.nchrom = nchrom; a.mats = mats; a.mat_off = mat_off; a.mat_n = mat_n; a.mat_ld = mat_ld; a.bin_off = bin_off;
     a.band = reinterpret_cast<int32_t*>(work); a.oob = oob;
     a.bw_shift = band_shift(band_width);
-    // HC_BIN_CLUSTER=N: 1 (default) = every CTA counts the main diagonal in 16-bit shared-memory counters of its own and
-    // drains them into the band at the end (measured on C2: binning 5.50 -> 5.39 ms, step 12.92 -> 12.76 ms, twice in a row);
-    // N = 2, 4, 8 or 16: the hottest diagonals spread over the distributed shared memory of clusters of N CTAs (measured
-    // slower: 7.2-8.1 ms); 0 = every near-diagonal update is an L2 RED
-    int csize = 1;
-    if (const char* e = getenv("HC_BIN_CLUSTER")) csize = atoi(e);
-    if (csize >= 1 && csize <= 16 && (csize & (csize - 1)) == 0 && npairs >= (1 << 20)) {
-        auto kern = chrom_is_u8 ? bin_pairs_band_cluster_kernel<true> : bin_pairs_band_cluster_kernel<false>;
+    // large inputs: every CTA counts the hottest diagonals in 16-bit shared-memory counters of its own and drains them
+    // into the band at the end (measured on C2: binning 5.50 -> 5.39 ms, step 12.92 -> 12.76 ms, twice in a row)
+    if (npairs >= (1 << 20)) {
+        auto kern = chrom_is_u8 ? bin_pairs_band_hot_kernel<true> : bin_pairs_band_hot_kernel<false>;
         const size_t smem = (size_t)HOT_PER_CTA * 2;
         HC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        if (csize > 8) HC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(hc_num_sms() / csize * csize));      // one CTA per SM, whole clusters
-        cfg.blockDim = dim3(HOT_THREADS);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = s;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)csize; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        HC_CUDA(cudaLaunchKernelEx(&cfg, kern, a));
+        kern<<<hc_num_sms(), HOT_THREADS, smem, s>>>(a);      // one CTA per SM
         HC_LAUNCH_CHECK();
         return HC_OK;
     }

@@ -28,18 +28,11 @@
 //     instructions so that the kernel is a pure HBM stream.
 #include <cooperative_groups.h>
 #include <vector>
-#include <thread>
-#include <string>
 #include <algorithm>
 #include <math.h>
 #include <stdlib.h>
 #include "hc_common.cuh"
 #include "hc_select.cuh"
-
-// hc_ice_sym.cu
-int hc_ice_dense_balance_sym(const int32_t* mats, const int64_t* mat_off, const int32_t* mat_n, const int32_t* mat_ld,
-                             const int64_t* bin_off, int32_t nprob, const int32_t* h_mat_n, const hc_ice_params* P,
-                             double* bias, hc_ice_result* results, hc_ice_run_info* h_info, cudaStream_t s);
 
 namespace {
 
@@ -1157,78 +1150,10 @@ extern "C" int hc_ice_filter_bins(const double* nnz_marg, double* marg, int64_t 
     return HC_OK;
 }
 
-static int ice_dense_balance_impl(const int32_t* mats, const int64_t* mat_off, const int32_t* mat_n,
-                                  const int32_t* mat_ld, const int64_t* bin_off, int32_t nprob,
-                                  const int32_t* h_mat_n, const hc_ice_params* P, double* bias,
-                                  hc_ice_result* results, hc_ice_run_info* h_info, void* stream);
-
-// The chromosomes of a batch are independent problems, and one iteration of a batch is a bandwidth-bound stream kernel
-// followed by a short latency-bound update kernel (cluster syncs, ~8 us) plus two launch gaps: ~30 % of the loop is not
-// streaming.  With the batch cut into two halves of ~equal bytes, each iterated by its own host thread / stream / graph, the
-// update kernel and the gaps of one half could hide under the stream kernel of the other.  MEASURED SLOWER on C2 (loop 6.47 vs
-// 5.52 ms, step 15.7 vs 12.8 ms: the two persistent stream kernels are each sized to fill the GPU and take turns instead of
-// overlapping, and each half pays its own update latency), so it stays opt-in: HC_ICE_SPLIT=2.
 extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off, const int32_t* mat_n,
                                     const int32_t* mat_ld, const int64_t* bin_off, int32_t nprob,
                                     const int32_t* h_mat_n, const hc_ice_params* P, double* bias,
                                     hc_ice_result* results, hc_ice_run_info* h_info, void* stream) {
-    HC_REQUIRE(nprob > 0 && h_mat_n != nullptr && P != nullptr, "nprob>0, h_mat_n, params");
-    int split = 1, mode = 1;
-    if (const char* e = getenv("HC_ICE_SPLIT")) split = atoi(e);
-    if (const char* e = getenv("HC_ICE_PACKED")) mode = atoi(e);
-    double cells = 0.0;
-    for (int p = 0; p < nprob; ++p) { if (h_mat_n[p] < 0) { split = 1; break; } cells += (double)h_mat_n[p] * h_mat_n[p]; }
-    // worth it only when each half still fills the GPU: >= 4 problems and >= 64 M cells in total
-    if (split < 2 || mode >= 2 || nprob < 4 || cells < 64e6)
-        return ice_dense_balance_impl(mats, mat_off, mat_n, mat_ld, bin_off, nprob, h_mat_n, P, bias, results, h_info, stream);
-    int p0 = 1;
-    { double acc = 0.0; for (p0 = 0; p0 < nprob - 1 && acc < 0.5 * cells; ++p0) acc += (double)h_mat_n[p0] * h_mat_n[p0]; }
-    if (p0 < 1) p0 = 1;
-    // 0-based bin offsets of each half (the kernels index their bias slice with them)
-    std::vector<int64_t> h_off((size_t)nprob + 2, 0);
-    int64_t base2 = 0;
-    for (int p = 0; p < p0; ++p) { h_off[p + 1] = h_off[p] + h_mat_n[p]; base2 += h_mat_n[p]; }
-    int64_t* h_off2 = h_off.data() + p0 + 1;
-    h_off2[0] = 0;
-    for (int p = p0; p < nprob; ++p) h_off2[p - p0 + 1] = h_off2[p - p0] + h_mat_n[p];
-    cudaStream_t cs = (cudaStream_t)stream;
-    int dev = 0;
-    HC_CUDA(cudaGetDevice(&dev));
-    int64_t* d_off = nullptr;
-    HC_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d_off), sizeof(int64_t) * h_off.size(), cs));
-    HC_CUDA(cudaMemcpyAsync(d_off, h_off.data(), sizeof(int64_t) * h_off.size(), cudaMemcpyHostToDevice, cs));
-    hc_ice_run_info info1 = {}, info2 = {};
-    int rc2 = HC_OK;
-    std::string err2;
-    std::thread second([&]() {
-        if (cudaSetDevice(dev) != cudaSuccess) { rc2 = HC_ERR_CUDA; err2 = "cudaSetDevice failed in the second ICE group"; return; }
-        rc2 = ice_dense_balance_impl(mats, mat_off + p0, mat_n + p0, mat_ld + p0, d_off + p0 + 1, nprob - p0, h_mat_n + p0, P,
-                                     bias + base2, results + p0, h_info ? &info2 : nullptr, stream);
-        if (rc2 != HC_OK) err2 = hc_last_error();
-    });
-    const int rc1 = ice_dense_balance_impl(mats, mat_off, mat_n, mat_ld, d_off, p0, h_mat_n, P, bias, results,
-                                           h_info ? &info1 : nullptr, stream);
-    second.join();
-    cudaFreeAsync(d_off, cs);
-    if (h_info) {
-        *h_info = info1;
-        h_info->launches = info1.launches + info2.launches;
-        h_info->loop_ms = info1.loop_ms > info2.loop_ms ? info1.loop_ms : info2.loop_ms;
-        h_info->pack_ms = info1.pack_ms > info2.pack_ms ? info1.pack_ms : info2.pack_ms;
-        h_info->overflow_cells = info1.overflow_cells + info2.overflow_cells;
-        // stream_full_ms: the two stream kernels share the GPU, so a launch bracket does not time a kernel alone
-        h_info->stream_full_ms = 0.f;
-        h_info->stream_full_launches = 0;
-    }
-    if (rc1 != HC_OK) return rc1;
-    if (rc2 != HC_OK) { hc_set_error("%s", err2.c_str()); return rc2; }
-    return HC_OK;
-}
-
-static int ice_dense_balance_impl(const int32_t* mats, const int64_t* mat_off, const int32_t* mat_n,
-                                  const int32_t* mat_ld, const int64_t* bin_off, int32_t nprob,
-                                  const int32_t* h_mat_n, const hc_ice_params* P, double* bias,
-                                  hc_ice_result* results, hc_ice_run_info* h_info, void* stream) {
     HC_REQUIRE(nprob > 0 && h_mat_n != nullptr && P != nullptr, "nprob>0, h_mat_n, params");
     HC_REQUIRE(P->max_iters >= 1 && P->ignore_diags >= 0, "max_iters>=1, ignore_diags>=0");
     int64_t nbins = 0;
@@ -1258,15 +1183,9 @@ static int ice_dense_balance_impl(const int32_t* mats, const int64_t* mat_off, c
     // variant: 4 rows per warp step is the fastest per byte, but a warp item is at least RG rows; when the
     // batch is small (one large chromosome per GPU in the 8-way sharded run) fewer rows per item keep
     // every resident warp busy.  HC_ICE_VARIANT overrides (tuning).
-    // HC_ICE_PACKED: 2 (default) = symmetric packed blocks + persistent dataflow kernel (hc_ice_sym.cu); 1 = full-matrix
-    // uint8 + overflow encoding streamed once per iteration by the kernels below; 0 = stream the int32 tiles
-    int mode = 1;   // TODO(validate on hardware, then default 2)
-    if (const char* e = getenv("HC_ICE_PACKED")) mode = atoi(e);
-    if (mode >= 2) {
-        const int r = hc_ice_dense_balance_sym(mats, mat_off, mat_n, mat_ld, bin_off, nprob, h_mat_n, P, bias, results, h_info, s);
-        if (r <= 0) return r;       // +1: not applicable (a chromosome beyond 8192 bins): full-matrix packed kernel
-    }
-    bool packed = mode != 0;
+    // HC_ICE_PACKED=0: stream the int32 tiles instead of the uint8 + overflow encoding
+    bool packed = true;
+    if (const char* e = getenv("HC_ICE_PACKED")) packed = atoi(e) != 0;
     int64_t total_rows = 0;
     for (int p = 0; p < nprob; ++p) total_rows += h_mat_n[p];
     StreamVariant V;

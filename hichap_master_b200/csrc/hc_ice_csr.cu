@@ -110,98 +110,6 @@ ice_csr_stream_kernel(CsrView A, const double* __restrict__ bias, int kd, const 
     }
 }
 
-// ---- iteration kernel with a TMA-staged bias window ------------------------------------------
-// Contacts concentrate near the diagonal, so most gathers bias[col] of a block of consecutive rows
-// fall into a window of the bias vector around those rows.  Each CTA takes a block of ROWS_PER_CTA
-// rows (drawn from a global counter), stages bias[w0, w0 + WIN) in shared memory with ONE bulk
-// asynchronous copy (cp.async.bulk global -> shared, completion on an mbarrier: the TMA engine
-// moves the 64 KB while the warps fetch their row pointers), and serves in-window columns from
-// shared memory; only the far / trans columns still gather 32-byte sectors from L2.
-#ifndef HC_CSR_WIN
-#define HC_CSR_WIN 2048
-#endif
-constexpr int WIN = HC_CSR_WIN;      // doubles: 16 KB window (20 Mb of 10 kb bins), 8 CTAs per SM
-constexpr int ROWS_PER_CTA = 64;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__global__ void __launch_bounds__(256)
-ice_csr_window_kernel(CsrView A, const double* __restrict__ bias, long long nbins, int kd,
-                      const int64_t* __restrict__ bin_off, int nprob, const int32_t* __restrict__ done_at, int k,
-                      double* __restrict__ marg, unsigned int* block_counter) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    double* sbias = reinterpret_cast<double*>(smem_raw);
-    __shared__ __align__(8) unsigned long long mbar;
-    __shared__ unsigned int blk_s;
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const long long nblocks = (A.nloc + ROWS_PER_CTA - 1) / ROWS_PER_CTA;
-    const long long win = nbins < WIN ? (nbins & ~1ll) : WIN;       // whole (even) window
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(&mbar)), "r"(1) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    uint32_t phase = 0;
-    for (;;) {
-        if (threadIdx.x == 0) blk_s = atomicAdd(block_counter, 1u);
-        __syncthreads();                       // also: every warp is done reading the previous window
-        const long long blk = blk_s;
-        __syncthreads();                       // blk_s is rewritten by thread 0 at the top of the next round
-        if (blk >= nblocks) break;
-        const long long rl0 = blk * ROWS_PER_CTA, rl1 = min(rl0 + ROWS_PER_CTA, A.nloc);
-        long long w0 = (A.row0 + (rl0 + rl1) / 2 - win / 2) & ~1ll;  // 16-byte aligned source
-        if (w0 < 0) w0 = 0;
-        if (w0 + win > nbins) w0 = (nbins - win) & ~1ll;
-        if (threadIdx.x == 0 && win > 0) {
-            const uint32_t bytes = (uint32_t)(win * sizeof(double));
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(&mbar)), "r"(bytes) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         :: "r"(smem_u32(sbias)), "l"(bias + w0), "r"(bytes), "r"(smem_u32(&mbar)) : "memory");
-        }
-        if (win > 0) {                         // all threads wait for the bytes to land
-            uint32_t done = 0;
-            while (!done) {
-                asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                             : "=r"(done) : "r"(smem_u32(&mbar)), "r"(phase) : "memory");
-            }
-            phase ^= 1;
-        }
-        for (long long rl = rl0 + wid; rl < rl1; rl += 8) {
-            const long long r = A.row0 + rl;
-            const int p = nprob > 1 ? find_problem(bin_off, nprob, r) : 0;
-            const int d = done_at[p];
-            if (d != 0 && d < k) continue;     // this chromosome converged in an earlier iteration
-            const long long e0 = A.row_ptr[rl], e1 = A.row_ptr[rl + 1];
-            double acc0 = 0.0, acc1 = 0.0;
-            auto one = [&](int c, int v, double& acc) {
-                const double w = csr_band_weight(c, r, kd);
-                const unsigned long long off = (unsigned long long)((long long)c - w0);
-                const double b = off < (unsigned long long)win ? sbias[off] : __ldg(bias + c);
-                acc = fma(w * (double)v, b, acc);
-            };
-            const long long head = min((long long)((4 - (e0 & 3)) & 3), e1 - e0);
-            if (lane < head) one(__ldg(A.col + e0 + lane), __ldg(A.cnt + e0 + lane), acc0);
-            const long long eb = e0 + head;
-            const long long nvec = (e1 - eb) >> 2;
-            long long v = lane;
-            for (; v + 32 < nvec; v += 64) {
-                const int4 c0 = ld_stream_v4(A.col + eb + 4 * v), k0 = ld_stream_v4(A.cnt + eb + 4 * v);
-                const int4 c1 = ld_stream_v4(A.col + eb + 4 * (v + 32)), k1 = ld_stream_v4(A.cnt + eb + 4 * (v + 32));
-                one(c0.x, k0.x, acc0); one(c0.y, k0.y, acc1); one(c0.z, k0.z, acc0); one(c0.w, k0.w, acc1);
-                one(c1.x, k1.x, acc0); one(c1.y, k1.y, acc1); one(c1.z, k1.z, acc0); one(c1.w, k1.w, acc1);
-            }
-            for (; v < nvec; v += 32) {
-                const int4 c0 = ld_stream_v4(A.col + eb + 4 * v), k0 = ld_stream_v4(A.cnt + eb + 4 * v);
-                one(c0.x, k0.x, acc0); one(c0.y, k0.y, acc1); one(c0.z, k0.z, acc0); one(c0.w, k0.w, acc1);
-            }
-            const long long et = eb + (nvec << 2);
-            if (et + lane < e1) one(__ldg(A.col + et + lane), __ldg(A.cnt + et + lane), acc1);
-            const double acc = warp_sum(acc0 + acc1);
-            if (lane == 0) marg[r] = __ldg(bias + r) * acc;
-        }
-    }
-}
-
 // ---- per-iteration statistics and update (grid = (STAT_SLICES, nprob)) ---------------------
 struct StatArgs {
     const int64_t* bin_off; int nprob;
@@ -371,15 +279,6 @@ extern "C" int hc_ice_csr_balance(const int64_t* row_ptr, const int32_t* col, co
     long long* part_cnt = reinterpret_cast<long long*>(part_var + (size_t)nprob * STAT_SLICES);
     int32_t* done_at = reinterpret_cast<int32_t*>(part_cnt + (size_t)nprob * STAT_SLICES);
     int32_t* n_done = done_at + nprob;
-    unsigned int* block_counter = reinterpret_cast<unsigned int*>(n_done + 1);
-    // TMA-staged bias window: measured slower than the pipelined gather kernel on C4-like data
-    // (0.91 vs 0.68 ms per iteration, profiles/README.md) because 42 % of the stored entries are trans
-    // contacts outside any window and the 64 KB windows cut occupancy to 24 warps/SM; opt-in only.
-    bool use_window = false;
-    if (const char* e = getenv("HC_CSR_WINDOW")) use_window = atoi(e) != 0;
-    const int window_grid = hc_num_sms() * 8;     // 8 x 16 KB windows per SM
-    if (use_window)
-        HC_CUDA(cudaFuncSetAttribute(ice_csr_window_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(WIN * sizeof(double))));
     HC_CUDA(cudaMemsetAsync(marg, 0, sizeof(double) * 2 * nbins, s));
     HC_CUDA(cudaMemsetAsync(done_at, 0, sizeof(int32_t) * (nprob + 1), s));
 
@@ -423,14 +322,8 @@ extern "C" int hc_ice_csr_balance(const int64_t* row_ptr, const int32_t* col, co
     int launches = 0, h_done = 0, rc = HC_OK;
     for (int k = 1; k <= P->max_iters; ++k) {
         if (nloc > 0) {
-            if (use_window) {
-                cudaMemsetAsync(block_counter, 0, sizeof(unsigned int), s);
-                ice_csr_window_kernel<<<window_grid, 256, WIN * sizeof(double), s>>>(A, bias, nbins, P->ignore_diags, bin_off,
-                                                                                    nprob, done_at, k, marg_local, block_counter);
-            } else {
-                ice_csr_stream_kernel<false><<<stream_grid(), 256, 0, s>>>(A, bias, P->ignore_diags, bin_off, nprob, done_at,
-                                                                         k, marg_local, nullptr);
-            }
+            ice_csr_stream_kernel<false><<<stream_grid(), 256, 0, s>>>(A, bias, P->ignore_diags, bin_off, nprob, done_at,
+                                                                     k, marg_local, nullptr);
             hc_count_launch(); ++launches;
         }
         if (nccl_comm) {

@@ -325,209 +325,6 @@ csrb_stream_kernel(CsrbArgs A) {
     }
 }
 
-// ---------------------------------------------------------------------------------------
-// TMA-fed variant (opt-in, HC_CSRB_TMA=1): the entries themselves are staged in shared memory by bulk copies
-// ---------------------------------------------------------------------------------------
-// ncu on the kernel above (profiles/r2e_ncu_csrb_stream_v2.json): long-scoreboard stalls on the entry / bounds loads
-// dominate at 50 % issue activity and 3.0 TB/s.  An item's entries are one contiguous byte range, so here the producer
-// thread hands whole items to the TMA engine -- entries (<= 48 KB) and segment bounds -- three items ahead, and the warps
-// only ever read shared memory: LDS.128 for the entries, LDS.64 for the bias gathers.  Items are capped at TMA_ROWS rows
-// and assigned to the CTAs statically (item i -> CTA i mod grid; they are of near-equal size), so the loop has no queue
-// and no CTA-wide barrier except when the column block (the staged bias) changes.
-// MEASURED (profiles/r2j_ncu_csrb_tma_v1.json, C4 on one B200): 2.68 ms per launch against 1.30 ms for the kernel above.
-// A stage must hold the largest possible item (target + one full segment = 48 KB) but holds 17 KB on average, and only
-// three stages fit beside the 64 KB bias block, so ~32 KB are in flight per SM -- half of what the DRAM latency needs;
-// 43 % of the stall samples are the wait for the bulk copy.  Kept opt-in for the record.
-constexpr int TMA_ROWS = 512;                       // rows per super-chunk: an item never spans more
-constexpr int TMA_TARGET = 4096;                    // entries per item; < TMA_TARGET + CB with the last segment's overshoot
-constexpr int TMA_ENT_BYTES = (TMA_TARGET + CB) * 4;            // 48 KB
-constexpr int TMA_BND_BYTES = ((TMA_ROWS + 4) * 8 + 127) / 128 * 128;
-constexpr int TMA_STAGE_BYTES = TMA_ENT_BYTES + TMA_BND_BYTES;
-constexpr int TMA_NST = 3;
-constexpr int TMA_THREADS = 768;
-constexpr int TMA_WARPS = TMA_THREADS / 32;
-
-// items per (column block, super-chunk of TMA_ROWS rows)
-__global__ void __launch_bounds__(256)
-csrb_chunk_count_kernel(const int64_t* __restrict__ seg_ptr, long long nloc, int nb, int nrc, int32_t* __restrict__ cnt) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (long long)nb * nrc) return;
-    const long long cb = i / nrc, rc = i - cb * nrc;
-    const long long lo = rc * TMA_ROWS, hi = min(nloc, lo + TMA_ROWS);
-    const int64_t* sp = seg_ptr + cb * nloc;
-    const long long e = sp[hi] - sp[lo];
-    cnt[i] = (int32_t)((e + TMA_TARGET - 1) / TMA_TARGET);
-}
-// exclusive scan of int32 counts (single CTA), total -> v[n]
-__global__ void __launch_bounds__(1024) csrb_scan32_kernel(int32_t* __restrict__ v, int n) {
-    __shared__ int sh[1024];
-    __shared__ int carry;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    for (int b0 = 0; b0 < n; b0 += 1024) {
-        const int i = b0 + threadIdx.x;
-        const int x = i < n ? v[i] : 0;
-        sh[threadIdx.x] = x;
-        __syncthreads();
-        for (int o = 1; o < 1024; o <<= 1) {
-            const int t = threadIdx.x >= o ? sh[threadIdx.x - o] : 0;
-            __syncthreads();
-            sh[threadIdx.x] += t;
-            __syncthreads();
-        }
-        if (i < n) v[i] = carry + sh[threadIdx.x] - x;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry += sh[1023];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) v[n] = carry;
-}
-// item -> two descriptors: {cb, first row, end row, log2 lanes per segment}, {first 16-byte vector of its entries, vectors, 0, 0}
-__global__ void __launch_bounds__(256)
-csrb_tma_items_kernel(const int64_t* __restrict__ seg_ptr, long long nloc, int nb, int nrc, const int32_t* __restrict__ first,
-                      int nitems, int4 gthr, int4* __restrict__ desc) {
-    const int it = blockIdx.x * blockDim.x + threadIdx.x;
-    if (it >= nitems) return;
-    int lo = 0, hi = nb * nrc - 1;
-    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (first[mid] <= it) lo = mid; else hi = mid - 1; }
-    const int sc = lo, k = it - first[sc];
-    const int cb = sc / nrc, rc = sc - cb * nrc;
-    const long long rlo = (long long)rc * TMA_ROWS, rhi = min(nloc, rlo + TMA_ROWS);
-    const int64_t* sp = seg_ptr + (long long)cb * nloc;
-    const long long base = sp[rlo];
-    auto first_row_at = [&](long long off) {
-        long long a = rlo, b = rhi;
-        while (a < b) { const long long m = (a + b) >> 1; if (sp[m] < off) a = m + 1; else b = m; }
-        return a;
-    };
-    const long long r0 = k == 0 ? rlo : first_row_at(base + (long long)k * TMA_TARGET);
-    const long long r1 = it + 1 == first[sc + 1] ? rhi : first_row_at(base + (long long)(k + 1) * TMA_TARGET);
-    const long long entries = sp[r1] - sp[r0];
-    const long long rows = r1 > r0 ? r1 - r0 : 1;
-    const long long avg = entries / rows;
-    const int glog = avg >= gthr.w ? 5 : (avg >= gthr.z ? 4 : (avg >= gthr.y ? 3 : (avg >= gthr.x ? 2 : 1)));
-    desc[2 * (long long)it] = make_int4(cb, (int)r0, (int)r1, glog);
-    desc[2 * (long long)it + 1] = make_int4((int)(sp[r0] >> 2), (int)(entries >> 2), 0, 0);
-}
-
-template <int G>
-__device__ __forceinline__ void csrb_tma_process(const CsrbArgs& A, const double* __restrict__ sb, const int4* __restrict__ e4,
-                                                 const long long* __restrict__ bnd, long long base4, int cb, int r0, int r1) {
-    const int lane = threadIdx.x & 31, gl = lane & (G - 1);
-    const int gid = (threadIdx.x >> 5) * (32 / G) + lane / G, ng = TMA_WARPS * (32 / G);
-    const unsigned gmask = G == 32 ? 0xffffffffu : (((1u << G) - 1u) << (lane & ~(G - 1)));
-    double* __restrict__ pout = A.part + (long long)cb * A.nloc;
-    for (int row = r0 + gid; row < r1; row += ng) {
-        if (A.nprob > 1 && A.done_at[find_problem(A.bin_off, A.nprob, A.row0 + row)] != 0) continue;   // group-uniform
-        const int v0 = (int)((bnd[row - r0] >> 2) - base4), v1 = (int)((bnd[row - r0 + 1] >> 2) - base4);
-        double a0 = 0.0, a1 = 0.0;
-        int v = v0 + gl;
-        for (; v + G < v1; v += 2 * G) {
-            const int4 q = e4[v], u = e4[v + G];
-            csrb_fma4(q, sb, a0, a1);
-            csrb_fma4(u, sb, a0, a1);
-        }
-        if (v < v1) csrb_fma4(e4[v], sb, a0, a1);
-        double acc = a0 + a1;
-#pragma unroll
-        for (int o = G / 2; o > 0; o >>= 1) acc += __shfl_xor_sync(gmask, acc, o);
-        if (gl == 0) pout[row] = acc;
-    }
-}
-
-struct TmaItems { const int4* desc; int nitems; };
-
-__global__ void __launch_bounds__(TMA_THREADS, 1)
-csrb_tma_kernel(CsrbArgs A, TmaItems Q) {
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    double* sb = reinterpret_cast<double*>(smem_raw);                    // 64 KB: bias of the staged column block
-    unsigned char* stages = smem_raw + CB * sizeof(double);
-    __shared__ __align__(8) unsigned long long full[TMA_NST], empty[TMA_NST], biasbar;
-    if (*A.n_done >= A.nonempty) return;             // every problem converged: the rest of the replayed graph is idle
-    const int tid = threadIdx.x, lane = tid & 31;
-    if (tid == 0) {
-        for (int x = 0; x < TMA_NST; ++x) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(&full[x])), "r"(1) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(&empty[x])), "r"(TMA_WARPS) : "memory");
-        }
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(&biasbar)), "r"(1) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    const int G = gridDim.x;
-    // thread 0: hand item j (global index blockIdx.x + j * G) to the TMA engine: its entries and its segment bounds
-    auto issue = [&](int j) {
-        const long long it = (long long)blockIdx.x + (long long)j * G;
-        if (it >= Q.nitems) return;
-        const int x = j % TMA_NST;
-        const int4 d0 = __ldg(Q.desc + 2 * it), d1 = __ldg(Q.desc + 2 * it + 1);
-        unsigned char* st = stages + (size_t)x * TMA_STAGE_BYTES;
-        const long long s0 = (long long)d0.x * A.nloc + d0.y;            // index of the item's first bound in seg_ptr
-        const long long a0 = s0 & ~1ll;                                  // 16-byte aligned start
-        const uint32_t nb_b = (uint32_t)((((s0 - a0) + (d0.z - d0.y) + 1 + 1) & ~1ll) * 8);
-        const uint32_t ne_b = (uint32_t)d1.y * 16u;
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(&full[x])), "r"(nb_b + ne_b) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     :: "r"(smem_u32(st + TMA_ENT_BYTES)), "l"(A.seg_ptr + a0), "r"(nb_b), "r"(smem_u32(&full[x])) : "memory");
-        if (ne_b)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         :: "r"(smem_u32(st)), "l"(reinterpret_cast<const int4*>(A.ent) + d1.x), "r"(ne_b), "r"(smem_u32(&full[x])) : "memory");
-    };
-    if (tid == 0) for (int j = 0; j < TMA_NST; ++j) issue(j);
-    int staged = -1;
-    uint32_t bias_phase = 0;
-    for (int j = 0;; ++j) {
-        const long long it = (long long)blockIdx.x + (long long)j * G;
-        if (it >= Q.nitems) break;
-        const int x = j % TMA_NST;
-        const uint32_t par = (uint32_t)(j / TMA_NST) & 1u;
-        const int4 d0 = __ldg(Q.desc + 2 * it), d1 = __ldg(Q.desc + 2 * it + 1);
-        if (d0.x != staged) {           // new column block: everybody is done with the old bias, then stage the new one
-            __syncthreads();
-            if (tid == 0) {
-                const uint32_t bytes = CB * (uint32_t)sizeof(double);
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(smem_u32(&biasbar)), "r"(bytes) : "memory");
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                             :: "r"(smem_u32(sb)), "l"(A.bias_pad + (long long)d0.x * CB), "r"(bytes), "r"(smem_u32(&biasbar)) : "memory");
-            }
-            uint32_t done = 0;
-            while (!done)
-                asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                             : "=r"(done) : "r"(smem_u32(&biasbar)), "r"(bias_phase) : "memory");
-            bias_phase ^= 1u;
-            staged = d0.x;
-        }
-        {                               // the item's entries and bounds have landed
-            uint32_t done = 0;
-            while (!done)
-                asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                             : "=r"(done) : "r"(smem_u32(&full[x])), "r"(par) : "memory");
-        }
-        const unsigned char* st = stages + (size_t)x * TMA_STAGE_BYTES;
-        const long long s0 = (long long)d0.x * A.nloc + d0.y;
-        const long long* bnd = reinterpret_cast<const long long*>(st + TMA_ENT_BYTES) + (s0 & 1ll);
-        const int4* e4 = reinterpret_cast<const int4*>(st);
-        if (d0.w == 5) csrb_tma_process<32>(A, sb, e4, bnd, d1.x, d0.x, d0.y, d0.z);
-        else if (d0.w == 4) csrb_tma_process<16>(A, sb, e4, bnd, d1.x, d0.x, d0.y, d0.z);
-        else if (d0.w == 3) csrb_tma_process<8>(A, sb, e4, bnd, d1.x, d0.x, d0.y, d0.z);
-        else if (d0.w == 2) csrb_tma_process<4>(A, sb, e4, bnd, d1.x, d0.x, d0.y, d0.z);
-        else csrb_tma_process<2>(A, sb, e4, bnd, d1.x, d0.x, d0.y, d0.z);
-        // this warp is done with stage x; thread 0 refills it once every warp is
-        __syncwarp();
-        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(smem_u32(&empty[x])) : "memory");
-        if (tid == 0) {
-            uint32_t done = 0;
-            while (!done)
-                asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                             : "=r"(done) : "r"(smem_u32(&empty[x])), "r"(par) : "memory");
-            issue(j + TMA_NST);
-        }
-        __syncwarp();
-    }
-}
-
 struct VecArgs {
     const int64_t* bin_off; int nprob;
     long long nloc, row0, nbins; int nb;
@@ -711,7 +508,7 @@ int hc_ice_csr_balance_blocked(const int64_t* row_ptr, const int32_t* col, const
         HC_CUDA(scratch.alloc_big((void**)&d_ent, sizeof(uint32_t) * (size_t)ent_cap));
         tick("alloc entries");
         HC_CUDA(scratch.alloc((void**)&d_start, sizeof(int64_t) * nseg));
-        HC_CUDA(scratch.alloc((void**)&d_seg, sizeof(int64_t) * (nseg + 4)));      // + slack: the bulk copies of the bounds are 16-byte granular
+        HC_CUDA(scratch.alloc((void**)&d_seg, sizeof(int64_t) * (nseg + 1)));      // + the total
         HC_CUDA(scratch.alloc((void**)&d_bsum, sizeof(int64_t) * (nsb + 1 + nb + 1) + 16));
         d_tot = d_bsum + nsb + 1;
         d_flag = reinterpret_cast<int32_t*>(d_tot + nb + 1);
@@ -765,30 +562,12 @@ int hc_ice_csr_balance_blocked(const int64_t* row_ptr, const int32_t* col, const
         const long long e = h_tot[b + 1] - h_tot[b];
         h_first[b + 1] = h_first[b] + (int32_t)(e > 0 ? (e + target - 1) / target : 0);
     }
-    int nitems = h_first[nb];
-    // default: the register-staged stream kernel with its global queue; HC_CSRB_TMA=1: the TMA-fed kernel, whose items
-    // are also capped at TMA_ROWS rows and are assigned to the CTAs statically
-    bool tma = false;       // measured slower (C4, 1 GPU: 2.68 vs 1.30 ms per launch): see DESIGN.md section 4
-    if (const char* e = getenv("HC_CSRB_TMA")) tma = atoi(e) != 0;
+    const int nitems = h_first[nb];
     int4* d_items = nullptr;
     int32_t* d_first = nullptr;
-    const int nrc = (int)((nloc + TMA_ROWS - 1) / TMA_ROWS);
-    if (!tma || nloc == 0) {
-        tma = false;
-        HC_CUDA(scratch.alloc((void**)&d_items, sizeof(int4) * (size_t)std::max(nitems, 1)));
-        HC_CUDA(scratch.alloc((void**)&d_first, sizeof(int32_t) * (nb + 1)));
-        HC_CUDA(cudaMemcpyAsync(d_first, h_first.data(), sizeof(int32_t) * (nb + 1), cudaMemcpyHostToDevice, s));
-    } else {
-        const long long nsc = (long long)nb * nrc;
-        HC_REQUIRE(nsc < (1ll << 30), "too many (column block, row chunk) pairs");
-        HC_CUDA(scratch.alloc((void**)&d_first, sizeof(int32_t) * (size_t)(nsc + 1)));
-        csrb_chunk_count_kernel<<<(unsigned)((nsc + 255) / 256), 256, 0, s>>>(d_seg, nloc, nb, nrc, d_first);
-        HC_LAUNCH_CHECK();
-        csrb_scan32_kernel<<<1, 1024, 0, s>>>(d_first, (int)nsc);
-        HC_LAUNCH_CHECK();
-        HC_CUDA(hc_read_small(&nitems, d_first + nsc, sizeof(int32_t), s));
-        HC_CUDA(scratch.alloc((void**)&d_items, 2 * sizeof(int4) * (size_t)std::max(nitems, 1)));
-    }
+    HC_CUDA(scratch.alloc((void**)&d_items, sizeof(int4) * (size_t)std::max(nitems, 1)));
+    HC_CUDA(scratch.alloc((void**)&d_first, sizeof(int32_t) * (nb + 1)));
+    HC_CUDA(cudaMemcpyAsync(d_first, h_first.data(), sizeof(int32_t) * (nb + 1), cudaMemcpyHostToDevice, s));
     // average segment length from which a segment gets 4 / 8 / 16 / 32 lanes (HC_CSRB_GTHR="a,b,c,d" overrides)
     int4 gthr = make_int4(8, 32, 128, 512);      // measured on C4 (profiles/README.md): flat between these and (20, 20, 192, 192)
     if (const char* e = getenv("HC_CSRB_GTHR")) {
@@ -796,8 +575,7 @@ int hc_ice_csr_balance_blocked(const int64_t* row_ptr, const int32_t* col, const
         if (sscanf(e, "%d,%d,%d,%d", &a, &b, &c, &d) == 4) gthr = make_int4(a, b, c, d);
     }
     if (nitems > 0) {
-        if (tma) csrb_tma_items_kernel<<<(nitems + 255) / 256, 256, 0, s>>>(d_seg, nloc, nb, nrc, d_first, nitems, gthr, d_items);
-        else csrb_items_kernel<<<(nitems + 255) / 256, 256, 0, s>>>(d_seg, nloc, nb, d_first, nitems, target, gthr, d_items);
+        csrb_items_kernel<<<(nitems + 255) / 256, 256, 0, s>>>(d_seg, nloc, nb, d_first, nitems, target, gthr, d_items);
         HC_LAUNCH_CHECK();
     }
     HC_CUDA(cudaStreamSynchronize(s));             // h_first goes out of use
@@ -840,18 +618,13 @@ int hc_ice_csr_balance_blocked(const int64_t* row_ptr, const int32_t* col, const
     V.done_at = d_book; V.n_done = d_book + nprob; V.nonempty = nonempty; V.results = results; V.tol = P->tol; V.max_iters = P->max_iters;
 
     const size_t smem = (size_t)CB * sizeof(double);
-    const size_t smem_tma = smem + (size_t)TMA_NST * TMA_STAGE_BYTES;
     HC_CUDA(cudaFuncSetAttribute(csrb_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaFuncSetAttribute(csrb_stream_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    HC_CUDA(cudaFuncSetAttribute(csrb_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tma));
-    TmaItems Q{d_items, nitems};
-    const int grid_tma = std::max(1, std::min(hc_num_sms(), nitems));
     int rc = HC_OK;
     auto one_iteration = [&](cudaEvent_t t0, cudaEvent_t t1, unsigned flags) -> int {
         if (nloc > 0 && nitems > 0) {
             if (t0) cudaEventRecordWithFlags(t0, s, flags);
-            if (tma) csrb_tma_kernel<<<grid_tma, TMA_THREADS, smem_tma, s>>>(A, Q);
-            else csrb_stream_kernel<<<grid, ST_THREADS, smem, s>>>(A);
+            csrb_stream_kernel<<<grid, ST_THREADS, smem, s>>>(A);
             if (t1) cudaEventRecordWithFlags(t1, s, flags);
             csrb_marg_kernel<<<(unsigned)((nloc + 255) / 256), 256, 0, s>>>(V);
         } else {

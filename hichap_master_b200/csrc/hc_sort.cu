@@ -6,23 +6,17 @@
 //
 // Roofline: HBM-bound, 8*P (histogram) + passes*16*P bytes for P keys.
 #include "hc_common.cuh"
-#include <stdlib.h>
 
 namespace {
 
 constexpr int RADIX_BITS = 8;
 constexpr int RADIX = 1 << RADIX_BITS;
-#ifndef HC_SORT_DEFAULT_THREADS
-#define HC_SORT_DEFAULT_THREADS 512
-#endif
-constexpr int SORT_DEFAULT_THREADS = HC_SORT_DEFAULT_THREADS;
-constexpr int SORT_MIN_TILE = 256 * 16;               // smallest tile of any variant (sizes the status array)
 constexpr int MAX_PASSES = 8;
-#ifndef HC_SORT_MIN_BLOCKS
-#define HC_SORT_MIN_BLOCKS 4
-#endif
-constexpr int SORT_MIN_BLOCKS = HC_SORT_MIN_BLOCKS;   // 64 registers/thread -> 4 CTAs (32 warps) per SM
-
+constexpr int SORT_THREADS = 512;
+constexpr int SORT_ITEMS = 16;                        // keys per thread
+constexpr int SORT_TILE = SORT_THREADS * SORT_ITEMS;
+constexpr int SORT_MIN_BLOCKS = 2;                    // 64 registers/thread -> 2 CTAs (32 warps) per SM
+constexpr int SORT_LOOKBACK = 8;                      // status words fetched per look-back step
 
 __device__ __forceinline__ unsigned long long ld_relaxed_u64(const unsigned long long* p) {
     unsigned long long v;
@@ -74,13 +68,13 @@ __global__ void __launch_bounds__(RADIX) radix_scan_kernel(unsigned long long* _
 }
 
 // ---- one digit pass -------------------------------------------------------------------
-// THREADS x 16 keys per tile.  The tile size sets the length of the digit runs a tile writes (tile / 256 keys on a
+// 512 threads x 16 keys per tile.  The tile size sets the length of the digit runs a tile writes (tile / 256 keys on a
 // uniform digit): 128 B runs at 4096 keys, 256 B at 8192 -- the low-digit passes are bound by those scattered writes
-// (measured 2.1 TB/s at 4096 against 3.3 TB/s for the top digit, whose 64 occupied bins give 512 B runs).
-template <int THREADS, int SORT_ITEMS>
-struct SortSmemT {
-    unsigned long long keys[THREADS * SORT_ITEMS];
-    unsigned int warp_hist[THREADS / 32][RADIX];
+// (measured 2.1 TB/s at 4096 against 3.3 TB/s for the top digit, whose 64 occupied bins give 512 B runs).  12 keys per
+// thread at five CTAs of 256 threads per SM was measured too: 19.9 against 17.3 ms per 500 M keys.
+struct SortSmem {
+    unsigned long long keys[SORT_TILE];
+    unsigned int warp_hist[SORT_THREADS / 32][RADIX];
     unsigned int tile_off[RADIX];       // exclusive scan of the tile's digit totals
     unsigned long long gbase[RADIX];    // global position of the tile's first key of each digit, minus tile_off
     unsigned int scan_tmp[RADIX / 32];
@@ -90,9 +84,7 @@ struct SortSmemT {
 // Lanes of the warp that hold the same 8-bit digit.  MATCH.ANY does it in one instruction, but it runs on the address
 // divergence unit at about one warp instruction per 60 cycles and SM: with 16 of them per thread the pass sat at 81 % ADU
 // utilisation and 2.1 TB/s (profiles/r2r_ncu_onesweep_v2.json).  Eight ballots (ALU pipe) narrow the mask bit by bit.
-template <bool BALLOT>
 __device__ __forceinline__ unsigned match_digit(unsigned d, bool ok) {
-    if (!BALLOT) return __match_any_sync(0xffffffffu, ok ? d : (unsigned)(RADIX + (threadIdx.x & 31)));   // padding lanes match nobody
     unsigned m = __ballot_sync(0xffffffffu, ok);
 #pragma unroll
     for (int b = 0; b < RADIX_BITS; ++b) {
@@ -103,21 +95,20 @@ __device__ __forceinline__ unsigned match_digit(unsigned d, bool ok) {
     return m;
 }
 
-template <int SORT_LOOKBACK, int THREADS, int MINB, bool BALLOT, int SORT_ITEMS>
-__global__ void __launch_bounds__(THREADS, MINB)
+__global__ void __launch_bounds__(SORT_THREADS, SORT_MIN_BLOCKS)
 radix_onesweep_kernel(const unsigned long long* __restrict__ in, unsigned long long* __restrict__ out, long long n,
                       int shift, const unsigned long long* __restrict__ digit_base /*[256]*/,
                       unsigned long long* status /*[num_tiles][256]*/, unsigned int* tile_counter) {
-    constexpr int WARPS = THREADS / 32, TILE = THREADS * SORT_ITEMS;
+    constexpr int WARPS = SORT_THREADS / 32;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    SortSmemT<THREADS, SORT_ITEMS>& sm = *reinterpret_cast<SortSmemT<THREADS, SORT_ITEMS>*>(smem_raw);
+    SortSmem& sm = *reinterpret_cast<SortSmem*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
     if (tid == 0) sm.tile_id = atomicAdd(tile_counter, 1u);   // tiles are claimed in launch order
-    for (int i = tid; i < WARPS * RADIX; i += THREADS) (&sm.warp_hist[0][0])[i] = 0;
+    for (int i = tid; i < WARPS * RADIX; i += SORT_THREADS) (&sm.warp_hist[0][0])[i] = 0;
     __syncthreads();
     const long long tile = sm.tile_id;
-    const long long base = tile * TILE;
-    const int valid = (int)min((long long)TILE, n - base);
+    const long long base = tile * SORT_TILE;
+    const int valid = (int)min((long long)SORT_TILE, n - base);
 
     // warp-striped load keeps memory order == (warp, item, lane) order -> stable ranking
     unsigned long long key[SORT_ITEMS];
@@ -135,7 +126,7 @@ radix_onesweep_kernel(const unsigned long long* __restrict__ in, unsigned long l
         const int j = w * (32 * SORT_ITEMS) + i * 32 + lane;
         const bool ok = j < valid;
         const unsigned d = (unsigned)((key[i] >> shift) & (RADIX - 1));
-        const unsigned m = match_digit<BALLOT>(d, ok);          // padding lanes match nobody and count nowhere
+        const unsigned m = match_digit(d, ok);          // padding lanes match nobody and count nowhere
         const int leader = __ffs(m) - 1;
         unsigned prev = 0;
         if (ok && lane == leader) {
@@ -221,7 +212,7 @@ radix_onesweep_kernel(const unsigned long long* __restrict__ in, unsigned long l
         sm.gbase[tid] = digit_base[tid] + excl - sm.tile_off[tid];
     }
     __syncthreads();
-    for (int j = tid; j < valid; j += THREADS) {
+    for (int j = tid; j < valid; j += SORT_THREADS) {
         const unsigned long long k = sm.keys[j];
         const unsigned d = (unsigned)((k >> shift) & (RADIX - 1));
         out[sm.gbase[d] + (unsigned)j] = k;
@@ -230,10 +221,10 @@ radix_onesweep_kernel(const unsigned long long* __restrict__ in, unsigned long l
 
 }  // namespace
 
-// Workspace layout (bytes): [passes*256 u64 histogram][16 B counters][num_tiles*256 u64 status]; sized for the
-// smallest tile (4096 keys)
+// Workspace layout (bytes): [passes*256 u64 histogram][16 B counters][num_tiles*256 u64 status]; the status array has
+// room for one row per 4096 keys, twice the tiles of SORT_TILE keys
 extern "C" int64_t hc_sort_work_bytes(int64_t n) {
-    const int64_t tiles = (n + SORT_MIN_TILE - 1) / SORT_MIN_TILE;
+    const int64_t tiles = (n + 4095) / 4096;
     return (int64_t)sizeof(unsigned long long) * (MAX_PASSES * RADIX + (tiles > 0 ? tiles : 1) * RADIX) + 64;
 }
 
@@ -265,30 +256,14 @@ extern "C" int hc_sort_keys_u64(unsigned long long* keys, unsigned long long* tm
     radix_scan_kernel<<<passes, RADIX, 0, s>>>(ghist);
     HC_LAUNCH_CHECK();
 
-    // variants: HC_SORT_LOOKBACK = 1 | 8 status words fetched per look-back step; HC_SORT_THREADS = 256 | 512 threads per tile
-    // (4096 / 8192 keys); HC_SORT_MATCH = any | ballot.  (12 keys per thread at five CTAs of 256 threads per SM was measured
-    // too: 19.9 against 17.3 ms per 500 M keys.)
-    static const int lookback = [] { const char* e = getenv("HC_SORT_LOOKBACK"); return (e && atoi(e) == 1) ? 1 : 8; }();
-    static const int threads = [] { const char* e = getenv("HC_SORT_THREADS"); const int v = e ? atoi(e) : SORT_DEFAULT_THREADS;
-                                    return (v == 256 || v == 512) ? v : SORT_DEFAULT_THREADS; }();
-    static const bool ballot = [] { const char* e = getenv("HC_SORT_MATCH"); return !(e && e[0] == 'a'); }();
-    using Kern = void (*)(const unsigned long long*, unsigned long long*, long long, int, const unsigned long long*,
-                          unsigned long long*, unsigned int*);
-    static const Kern table[2][2][2] = {
-        {{radix_onesweep_kernel<1, 256, 4, false, 16>, radix_onesweep_kernel<1, 256, 4, true, 16>},
-         {radix_onesweep_kernel<8, 256, 4, false, 16>, radix_onesweep_kernel<8, 256, 4, true, 16>}},
-        {{radix_onesweep_kernel<1, 512, 2, false, 16>, radix_onesweep_kernel<1, 512, 2, true, 16>},
-         {radix_onesweep_kernel<8, 512, 2, false, 16>, radix_onesweep_kernel<8, 512, 2, true, 16>}}};
-    const Kern kern = table[threads == 256 ? 0 : 1][lookback == 1 ? 0 : 1][ballot ? 1 : 0];
-    const size_t smem = threads == 256 ? sizeof(SortSmemT<256, 16>) : sizeof(SortSmemT<512, 16>);
-    const long long tile_keys = (long long)threads * 16;
-    const long long tiles = (n + tile_keys - 1) / tile_keys;
-    HC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const size_t smem = sizeof(SortSmem);
+    const long long tiles = (n + SORT_TILE - 1) / SORT_TILE;
+    HC_CUDA(cudaFuncSetAttribute(radix_onesweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     unsigned long long* src = keys;
     unsigned long long* dst = tmp;
     for (int p = 0; p < passes; ++p) {
         HC_CUDA(cudaMemsetAsync(counter, 0, 16 + sizeof(unsigned long long) * tiles * RADIX, s));
-        kern<<<(unsigned)tiles, threads, smem, s>>>(
+        radix_onesweep_kernel<<<(unsigned)tiles, SORT_THREADS, smem, s>>>(
             src, dst, n, begin_bit + RADIX_BITS * p, ghist + p * RADIX, status, counter);
         HC_LAUNCH_CHECK();
         unsigned long long* t = src; src = dst; dst = t;

@@ -293,12 +293,12 @@ def _ice_vs_oracle(mb, mats, what, **kw):
     ({"HC_ICE_CLUSTER_UPDATE": "0"}, (700, 333), dict()),            # single-CTA update kernel on the packed encoding
     ({"HC_ICE_PACKED": "0"}, (700, 333), dict()),                    # int32 tiles, fp64 FMA kernel
     ({"HC_ICE_PACKED": "1"}, (700, 333), dict()),                    # full-matrix packed encoding, one launch pair per iteration
-    ({"HC_ICE_PACKED": "2"}, (700, 333), dict()),                    # symmetric blocks, persistent dataflow kernel (3 + 2 blocks per side)
-    ({"HC_ICE_PACKED": "2"}, (700, 333), dict(ignore_diags=0)),      # ... kept diagonal: half weights on the stored diagonal
-    ({"HC_ICE_PACKED": "2"}, (700, 333), dict(ignore_diags=3)),
-    ({"HC_ICE_PACKED": "2"}, (256, 257, 40, 1), dict()),             # block edges, a single-block and a 1-bin chromosome
-    ({"HC_ICE_PACKED": "2"}, (2100,), dict(max_iters=7)),            # 9 blocks per side, stops at max_iters
-    ({"HC_ICE_PACKED": "2"}, (1500, 900, 333, 90, 64), dict(mad_max=0, min_nnz=0)),   # five chromosomes in flight at once
+    ({}, (700, 333), dict(ignore_diags=3)),
+    ({}, (256, 257, 40, 1), dict()),                                 # on and one past a tile edge, a 1-bin chromosome
+    ({}, (2100,), dict(max_iters=7)),                                # stops at max_iters
+    ({}, (1500, 900, 333, 90, 64), dict(mad_max=0, min_nnz=0)),      # five chromosomes in flight at once
+    ({"HC_ICE_PACKED": "0"}, (256, 257, 40, 1), dict()),             # the same shapes on the int32 tiles
+    ({"HC_ICE_PACKED": "0"}, (1500, 900, 333, 90, 64), dict(mad_max=0, min_nnz=0)),
 ])
 def test_ice_encodings_and_kernel_variants(mb, monkeypatch, env, sizes, kw):
     """Every stream / update kernel variant of hc_ice_dense_balance against the oracle, with counts far above 255
@@ -323,8 +323,6 @@ def test_ice_packed_wide_bias_range_matches_int32_path(mb, monkeypatch):
     M = rng.poisson(np.minimum(lam, 2.0e9 / n)).astype(np.int64)
     M = np.triu(M) + np.triu(M, 1).T
     kw = dict(mad_max=0, min_nnz=1, max_iters=300)
-    monkeypatch.setenv("HC_ICE_PACKED", "2")
-    w_sym, st_sym = mb.ice_balance_dense([M], **kw)
     monkeypatch.setenv("HC_ICE_PACKED", "1")
     w_packed, st_packed = mb.ice_balance_dense([M], **kw)
     monkeypatch.setenv("HC_ICE_PACKED", "0")
@@ -336,10 +334,48 @@ def test_ice_packed_wide_bias_range_matches_int32_path(mb, monkeypatch):
     assert np.nanmax(ref) / np.nanmin(ref) > 2.0 ** 20
     assert np.array_equal(np.isnan(w_packed), np.isnan(w_i32)) and np.array_equal(np.isnan(w_packed), np.isnan(ref))
     assert st_packed["iters"] == st_i32["iters"] == rst["iters"]
-    assert st_sym["iters"] == rst["iters"] and np.array_equal(np.isnan(w_sym), np.isnan(ref))
-    check_weights(w_sym, ref, "symmetric packed, wide bias range")
     check_weights(w_packed, ref, "packed, wide bias range")
     check_weights(w_i32, ref, "int32, wide bias range")
+
+
+def test_ice_chr21_and_chr22_sized_packed_and_int32_vs_oracle(mb, monkeypatch):
+    """chr21- and chr22-sized matrices at 40 kb (1.5 M contacts each): the packed encoding (default) and the int32
+    tiles against the oracle."""
+    mats = []
+    for c, seed in (("21", 1), ("22", 2)):
+        L = synth.HG19[c]
+        p1, p2 = synth.cis_pairs(c, L, 1_500_000, seed=seed)
+        n = L // 40000 + 1
+        z = np.zeros(p1.size, np.int32)
+        mats.append(ho.bin_local_dense(z, p1, z, p2, [n], 40000)[0])
+    out = {}
+    for mode in ("1", "0"):
+        monkeypatch.setenv("HC_ICE_PACKED", mode)
+        out[mode] = mb.ice_balance_dense(mats)
+    off = np.concatenate([[0], np.cumsum([m.shape[0] for m in mats])])
+    b1, b2, cnt = [], [], []
+    for m, lo in zip(mats, off[:-1]):
+        x, y = np.nonzero(np.triu(m)); b1.append(x + lo); b2.append(y + lo); cnt.append(m[x, y])
+    ref, rst = cooler_ice.balance(np.concatenate(b1), np.concatenate(b2), np.concatenate(cnt), int(off[-1]), off, cis_only=True)
+    for mode, (w, st) in out.items():
+        check_weights(w, ref, "HC_ICE_PACKED=%s" % mode)
+        assert st["iters"] == rst["iters"], mode
+        np.testing.assert_allclose(st["scale"], rst["scale"], rtol=RTOL)
+
+
+def test_ice_degenerate_chromosomes(mb):
+    """A 300 x 300 chromosome batched with an all-zero one (nothing to balance: NaN weights, converged after one
+    pass) and a 1 x 1 one."""
+    rng = np.random.default_rng(4)
+    A = rng.poisson(5.0, size=(300, 300)); A = np.triu(A) + np.triu(A, 1).T
+    Z = np.zeros((33, 33), np.int64)
+    one = np.array([[7]])
+    w, st = mb.ice_balance_dense([A, Z, one])
+    x, y = np.nonzero(np.triu(A))
+    ref, rst = cooler_ice.balance(x, y, A[x, y], 334, [0, 300, 333, 334], cis_only=True)
+    check_weights(w, ref, "degenerate chromosomes")
+    assert np.isnan(w[300:]).all()
+    assert st["iters"] == rst["iters"]
 
 
 def test_ice_more_than_8192_columns(mb):
@@ -496,11 +532,10 @@ def test_banded_binning_equals_direct_and_oracle(mb, cuda_device, n, res, mode):
         kernels.bin_pairs_local_banded(bad, res, DenseBatch(sizes, cuda_device))
 
 
-@pytest.mark.parametrize("csize,pile", [("8", False), ("4", True), ("16", False), ("2", True), ("1", True), ("1", False), ("0", True)])
-def test_cluster_binning_equals_direct(mb, cuda_device, monkeypatch, csize, pile):
-    """HC_BIN_CLUSTER=N: the hottest diagonals are counted in the distributed shared memory of N-CTA clusters
-    (16-bit counters, drained into the band when they reach 0x8000).  `pile`: 200 000 pairs in ONE cell, several
-    times the 16-bit drain threshold."""
+@pytest.mark.parametrize("pile", [True, False])
+def test_hot_diagonal_binning_equals_direct(mb, cuda_device, pile):
+    """1.4 M pairs (>= 2^20): every CTA counts the hottest diagonals in 16-bit shared-memory counters, drained into the
+    band when they reach 0x8000.  `pile`: 200 000 pairs in ONE cell, several times the 16-bit drain threshold."""
     import torch
     from hichap_master_b200 import kernels
     from hichap_master_b200.device import DenseBatch, PairColumns
@@ -515,7 +550,6 @@ def test_cluster_binning_equals_direct(mb, cuda_device, monkeypatch, csize, pile
     pc = PairColumns(c1, p1, c2, p2)
     A = DenseBatch(sizes, cuda_device); B = DenseBatch(sizes, cuda_device)
     kernels.bin_pairs_local(pc, res, A)
-    monkeypatch.setenv("HC_BIN_CLUSTER", csize)
     kernels.bin_pairs_local_banded(pc, res, B)
     assert torch.equal(A.buf, B.buf)
     # uint8 chromosome columns, fed in two chunks (the PCIe-overlapped path)
