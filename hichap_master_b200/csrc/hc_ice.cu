@@ -629,13 +629,14 @@ __device__ __forceinline__ void mma_u8(int (&c)[4], const int4& a, const uint2& 
 }
 
 // Streaming half of an iteration on the packed encoding.  Same work distribution as the int32 kernel (persistent
-// warps, global queue of row-group items; a row group is RS strips of 16 rows).  Per k-tile a lane issues RS
-// 128-bit streaming loads (its A fragments), one 64-bit load of the bias planes (B fragment, through L1) and RS
-// MMAs; U k-tiles are in flight.  C fragment: lane l holds, for rows g and g + 8 (g = l / 4), the int32 sums of
+// warps, global queue of items; a row group is one strip of 16 rows).  Per k-tile a lane issues one 128-bit
+// streaming load (its A fragment), one 64-bit load of the bias planes (B fragment, through L1) and one MMA;
+// Q8_U k-tiles are in flight.  C fragment: lane l holds, for rows g and g + 8 (g = l / 4), the int32 sums of
 // planes 2 * (l % 4) and 2 * (l % 4) + 1 -- folded into fp64 with the planes' weights, reduced over the 4 lanes
 // of the group, scaled by 2^(E - 64), plus the row's overflow cells in fp64.
-template <int RS, int U, int MINB>
-__global__ void __launch_bounds__(256, MINB)
+// 16 k-tiles in flight per lane at 2 CTAs/SM (16 warps/SM): the fastest of the variants measured on B200.
+constexpr int Q8_U = 16, Q8_MINB = 2;
+__global__ void __launch_bounds__(256, Q8_MINB)
 ice_q8_mma_kernel(IceDenseArgs A) {
     const int lane = threadIdx.x & 31;
     const int g = lane >> 2, t4 = lane & 3;
@@ -643,11 +644,11 @@ ice_q8_mma_kernel(IceDenseArgs A) {
     const double w_even = __longlong_as_double((long long)(1023 + 8 * (7 - 2 * t4)) << 52);
     const double w_odd = __longlong_as_double((long long)(1023 + 8 * (6 - 2 * t4)) << 52);
     const unsigned nitems = *A.nitems;
-    // An item = one row group (RS strips) x one K segment, described by 4 x int4 the host precomputed:
+    // An item = one strip x one K segment, described by 4 x int4 the host precomputed:
     //   d0 = tile byte offset (int64) | index of the item's first partial sum (int64)
     //   d1 = byte offset of the segment's bias planes (int64) | global row of the first row (int64)
     //   d2 = chromosome, offset of the chromosome in the padded vectors, (unused), rows
-    //   d3 = k-tiles in the segment, segment index, k-tiles per strip, (unused)
+    //   d3 = k-tiles in the segment, segment index, (k-tiles per strip, unused), (unused)
     // Items 0..W-1 are pre-assigned to the W warps; the rest are drawn from the global queue.  The descriptor
     // of the NEXT item is fetched while the current one is processed, and the draw after that is in flight too,
     // so no item starts with a chain of dependent L2 reads.
@@ -678,58 +679,43 @@ ice_q8_mma_kernel(IceDenseArgs A) {
             const int64_t part_base = ((int64_t)(uint32_t)d0.z) | ((int64_t)d0.w << 32);
             const int64_t dig_off = ((int64_t)(uint32_t)d1.x) | ((int64_t)d1.y << 32);
             const int64_t grow = ((int64_t)(uint32_t)d1.z) | ((int64_t)d1.w << 32);
-            const int nrows = d2.w, nk = d3.x, seg = d3.y, KT = d3.z;
+            const int nrows = d2.w, nk = d3.x, seg = d3.y;
             const uint8_t* qp = A.q8 + tile_off + 16 * lane;
             const uint8_t* dig = A.digits + dig_off + 8 * lane;
             const double* __restrict__ b = A.bias + d2.y;
             const double scale = __longlong_as_double((long long)(1023 + A.dig_exp[p] - 64) << 52);   // 2^(E - 64)
             double* pout = A.part + part_base;
-            const int ns = min(RS, (nrows + 15) >> 4);      // strips that exist
-            const uint8_t* sp[RS];
+            int c[4] = {0, 0, 0, 0};
+            for (int t = 0; t < nk; t += Q8_U) {       // nk <= 1024: the int32 plane sums cannot overflow
+                int4 a[Q8_U];
+                uint2 bf[Q8_U];
 #pragma unroll
-            for (int s = 0; s < RS; ++s) sp[s] = qp + (int64_t)min(s, ns - 1) * KT * 512;
-            int c[RS][4];
-#pragma unroll
-            for (int s = 0; s < RS; ++s) { c[s][0] = 0; c[s][1] = 0; c[s][2] = 0; c[s][3] = 0; }
-            for (int t = 0; t < nk; t += U) {       // nk <= 1024: the int32 plane sums cannot overflow
-                int4 a[U][RS];
-                uint2 bf[U];
-#pragma unroll
-                for (int u = 0; u < U; ++u) {
+                for (int u = 0; u < Q8_U; ++u) {
                     const int tt = min(t + u, nk - 1);
-#pragma unroll
-                    for (int s = 0; s < RS; ++s)
-                        a[u][s] = ld_stream_v4(reinterpret_cast<const int32_t*>(sp[s] + (int64_t)tt * 512));
+                    a[u] = ld_stream_v4(reinterpret_cast<const int32_t*>(qp + (int64_t)tt * 512));
                     bf[u] = t + u < nk ? *reinterpret_cast<const uint2*>(dig + (int64_t)tt * 256) : make_uint2(0u, 0u);
                 }
 #pragma unroll
-                for (int u = 0; u < U; ++u)
-#pragma unroll
-                    for (int s = 0; s < RS; ++s) mma_u8(c[s], a[u][s], bf[u]);
+                for (int u = 0; u < Q8_U; ++u) mma_u8(c, a[u], bf[u]);
             }
-#pragma unroll
-            for (int s = 0; s < RS; ++s) {
-                if (s < ns) {       // warp-uniform
-                    const int ra = 16 * s + g, rb = ra + 8;
-                    double va = ((double)c[s][0] * w_even + (double)c[s][1] * w_odd) * scale;
-                    double vb = ((double)c[s][2] * w_even + (double)c[s][3] * w_odd) * scale;
-                    if (seg == 0) {      // the first segment of a row also carries its overflow cells
-                        if (ra < nrows) {
-                            const int64_t x0 = A.ovf_ptr[grow + ra], x1 = A.ovf_ptr[grow + ra + 1];
-                            for (int64_t e = x0 + t4; e < x1; e += 4) va = fma((double)A.ovf_val[e], b[A.ovf_col[e]], va);
-                        }
-                        if (rb < nrows) {
-                            const int64_t x0 = A.ovf_ptr[grow + rb], x1 = A.ovf_ptr[grow + rb + 1];
-                            for (int64_t e = x0 + t4; e < x1; e += 4) vb = fma((double)A.ovf_val[e], b[A.ovf_col[e]], vb);
-                        }
-                    }
-                    va += __shfl_xor_sync(0xffffffffu, va, 1); va += __shfl_xor_sync(0xffffffffu, va, 2);
-                    vb += __shfl_xor_sync(0xffffffffu, vb, 1); vb += __shfl_xor_sync(0xffffffffu, vb, 2);
-                    if (t4 == 0) {
-                        if (ra < nrows) pout[ra] = va;
-                        if (rb < nrows) pout[rb] = vb;
-                    }
+            const int ra = g, rb = g + 8;
+            double va = ((double)c[0] * w_even + (double)c[1] * w_odd) * scale;
+            double vb = ((double)c[2] * w_even + (double)c[3] * w_odd) * scale;
+            if (seg == 0) {      // the first segment of a row also carries its overflow cells
+                if (ra < nrows) {
+                    const int64_t x0 = A.ovf_ptr[grow + ra], x1 = A.ovf_ptr[grow + ra + 1];
+                    for (int64_t e = x0 + t4; e < x1; e += 4) va = fma((double)A.ovf_val[e], b[A.ovf_col[e]], va);
                 }
+                if (rb < nrows) {
+                    const int64_t x0 = A.ovf_ptr[grow + rb], x1 = A.ovf_ptr[grow + rb + 1];
+                    for (int64_t e = x0 + t4; e < x1; e += 4) vb = fma((double)A.ovf_val[e], b[A.ovf_col[e]], vb);
+                }
+            }
+            va += __shfl_xor_sync(0xffffffffu, va, 1); va += __shfl_xor_sync(0xffffffffu, va, 2);
+            vb += __shfl_xor_sync(0xffffffffu, vb, 1); vb += __shfl_xor_sync(0xffffffffu, vb, 2);
+            if (t4 == 0) {
+                if (ra < nrows) pout[ra] = va;
+                if (rb < nrows) pout[rb] = vb;
             }
         }
         cur = nxt; d0 = e0; d1 = e1; d2 = e2; d3 = e3;
@@ -1059,28 +1045,17 @@ struct EventPair {
 };
 
 typedef void (*StreamKernel)(IceDenseArgs);
-struct StreamVariant { StreamKernel fn; int rg, u, minb; };
-// tuned on B200 (profiles/): RG rows share the bias loads; RG*U 128-bit loads in flight per lane
+struct StreamVariant { StreamKernel fn; int rg, minb; };
+// int32 kernel, tuned on B200 (profiles/): RG rows share the bias loads; RG*U 128-bit loads in flight per lane.
+// <4,2,4> is the fastest per byte (5.5 TB/s on C2, profiles/r1c_ice_variants_v3.log); the others keep every
+// resident warp busy when the batch has few rows.
 const StreamVariant kVariants[] = {
-    {ice_dense_stream_kernel<4, 2, 4>, 4, 2, 4},   // default: 5.5 TB/s on C2 (profiles/r1c_ice_variants_v3.log)
-    {ice_dense_stream_kernel<4, 2, 3>, 4, 2, 3},
-    {ice_dense_stream_kernel<2, 2, 4>, 2, 2, 4},
-    {ice_dense_stream_kernel<2, 4, 3>, 2, 4, 3},
-    {ice_dense_stream_kernel<4, 4, 2>, 4, 4, 2},
-    {ice_dense_stream_kernel<1, 4, 4>, 1, 4, 4},
+    {ice_dense_stream_kernel<4, 2, 4>, 4, 4},
+    {ice_dense_stream_kernel<2, 2, 4>, 2, 4},
+    {ice_dense_stream_kernel<1, 4, 4>, 1, 4},
 };
-
-// packed kernel: <RS strips of 16 rows per step, U k-tiles in flight, CTAs per SM>; .rg = rows per step
-const StreamVariant kQ8Variants[] = {
-    {ice_q8_mma_kernel<2, 4, 4>, 32, 4, 4},
-    {ice_q8_mma_kernel<1, 4, 4>, 16, 4, 4},
-    {ice_q8_mma_kernel<1, 8, 3>, 16, 8, 3},
-    {ice_q8_mma_kernel<2, 4, 3>, 32, 4, 3},
-    {ice_q8_mma_kernel<1, 8, 4>, 16, 8, 4},
-    {ice_q8_mma_kernel<2, 8, 2>, 32, 8, 2},
-    {ice_q8_mma_kernel<1, 16, 2>, 16, 16, 2},
-    {ice_q8_mma_kernel<1, 12, 3>, 16, 12, 3},
-};
+// packed kernel: an item is one strip of 16 rows
+const StreamVariant kQ8 = {ice_q8_mma_kernel, 16, Q8_MINB};
 
 }  // namespace
 
@@ -1180,36 +1155,23 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
         cudaEventDestroy(e_in);
     }
 
-    // variant: 4 rows per warp step is the fastest per byte, but a warp item is at least RG rows; when the
-    // batch is small (one large chromosome per GPU in the 8-way sharded run) fewer rows per item keep
-    // every resident warp busy.  HC_ICE_VARIANT overrides (tuning).
-    // HC_ICE_PACKED=0: stream the int32 tiles instead of the uint8 + overflow encoding
+    // HC_ICE_PACKED=0: stream the int32 tiles instead of the uint8 + overflow encoding (the reference path that the
+    // tests compare the packed kernel against)
     bool packed = true;
     if (const char* e = getenv("HC_ICE_PACKED")) packed = atoi(e) != 0;
-    int64_t total_rows = 0;
-    for (int p = 0; p < nprob; ++p) total_rows += h_mat_n[p];
-    StreamVariant V;
-    if (packed) {
-        int vi = -1;
-        if (const char* e = getenv("HC_ICE_Q8_VARIANT")) vi = atoi(e);
-        if (vi < 0 || vi >= (int)(sizeof(kQ8Variants) / sizeof(kQ8Variants[0]))) vi = 6;   // <1,16,2>: 16 warps/SM, 16 tiles in flight per lane
-        V = kQ8Variants[vi];
-    } else {
-        int vi = -1;
-        if (const char* e = getenv("HC_ICE_VARIANT")) vi = atoi(e);
-        if (vi < 0 || vi >= (int)(sizeof(kVariants) / sizeof(kVariants[0]))) {
-            const int64_t warps = (int64_t)hc_num_sms() * 4 * 8;
-            vi = total_rows / 4 >= warps + warps / 4 ? 0 : (total_rows / 2 >= warps + warps / 4 ? 2 : 5);   // <4,2,4> | <2,2,4> | <1,4,4>
-        }
-        V = kVariants[vi];
+    // int32 kernel: 4 rows per warp step is the fastest per byte, but a warp item is at least RG rows; when the
+    // batch is small (one large chromosome per GPU in the 8-way sharded run) fewer rows per item keep
+    // every resident warp busy
+    StreamVariant V = kQ8;
+    if (!packed) {
+        const int64_t warps = (int64_t)hc_num_sms() * 4 * 8;
+        V = kVariants[nbins / 4 >= warps + warps / 4 ? 0 : (nbins / 2 >= warps + warps / 4 ? 1 : 2)];   // <4,2,4> | <2,2,4> | <1,4,4>
     }
-    int item_kb = 32;   // int32 kernel: bytes of matrix per work item, small enough that the last item is a short tail
-    if (const char* e = getenv("HC_ICE_ITEM_KB")) item_kb = std::max(1, atoi(e));
-    // packed kernel: an item is V.rg rows x kseg k-tiles (of 32 columns): rows are split along K so that items stay
+    const int item_kb = 32;   // int32 kernel: bytes of matrix per work item, small enough that the last item is a short tail
+    // packed kernel: an item is one strip x kseg k-tiles (of 32 columns): rows are split along K so that items stay
     // small (16 rows of chr1 are 100 KB) -- the per-segment partial row sums are added up by the update kernel
     int kseg = 48;
-    if (const char* e = getenv("HC_ICE_KSEG")) kseg = std::min(1024, std::max(4, atoi(e) / 4 * 4));
-    else if (packed) {       // small batches (one chromosome per GPU): shorter segments keep every resident warp busy
+    if (packed) {       // small batches (one chromosome per GPU): shorter segments keep every resident warp busy
         const int64_t warps = (int64_t)hc_num_sms() * V.minb * 8;
         for (;;) {
             int64_t items = 0;
@@ -1234,51 +1196,54 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
         h_pad[p + 1] = h_pad[p] + h_ld[p];
     }
     const int64_t npad = h_pad[nprob];
+    int nseg_max = 1;
+    for (int p = 0; p < nprob; ++p) nseg_max = std::max(nseg_max, ((h_ld[p] >> 5) + kseg - 1) / kseg);
 
-    // ---- work items: RG-aligned row groups of ~item_kb KB, largest chromosomes first -----------
-    std::vector<int32_t> h_done(nprob, 0);
-    std::vector<int32_t> item_prob, item_row0, item_nrows;
-    std::vector<int4> item_desc;       // packed kernel: 4 per item, built once
-    bool desc_built = false;
+    // ---- work items, largest chromosomes first ---------------------------------------------------
+    std::vector<int> order(nprob);
+    for (int p = 0; p < nprob; ++p) order[p] = p;
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return h_mat_n[a] > h_mat_n[b]; });
+    // packed kernel: the descriptors of every item (4 x int4 each, see ice_q8_mma_kernel) are built once; the items
+    // of chromosome p are the ids [desc_lo[p], desc_hi[p])
+    std::vector<int4> item_desc;
     std::vector<int> desc_lo(nprob, 0), desc_hi(nprob, 0);
-    std::vector<int64_t> h_qoff(nprob, 0), h_binoff(nprob + 1, 0);
     if (packed) {
+        auto lohi = [](int64_t v, int& a, int& b) { a = (int)(uint32_t)(v & 0xffffffffll); b = (int)(v >> 32); };
+        std::vector<int64_t> h_qoff(nprob, 0), h_binoff(nprob + 1, 0);
         int64_t qb = 0;
         for (int p = 0; p < nprob; ++p) {
             h_qoff[p] = qb;
             qb += (int64_t)((h_mat_n[p] + 15) / 16) * 16 * h_ld[p];
             h_binoff[p + 1] = h_binoff[p] + h_mat_n[p];
         }
+        for (int p : order) {
+            const int n = h_mat_n[p], KT = h_ld[p] >> 5;
+            desc_lo[p] = (int)(item_desc.size() / 4);
+            for (int r0 = 0; r0 < n; r0 += V.rg)
+                for (int k0 = 0; k0 < KT; k0 += kseg) {
+                    int4 d0, d1, d2, d3;
+                    lohi(h_qoff[p] + ((int64_t)(r0 / 16) * KT + k0) * 512, d0.x, d0.y);
+                    lohi((int64_t)(k0 / kseg) * npad + h_pad[p] + r0, d0.z, d0.w);
+                    lohi(8 * h_pad[p] + (int64_t)k0 * 256, d1.x, d1.y);
+                    lohi(h_binoff[p] + r0, d1.z, d1.w);
+                    d2 = make_int4(p, (int)h_pad[p], r0, std::min(V.rg, n - r0));
+                    d3 = make_int4(std::min(kseg, KT - k0), k0 / kseg, KT, 0);
+                    item_desc.push_back(d0); item_desc.push_back(d1); item_desc.push_back(d2); item_desc.push_back(d3);
+                }
+            desc_hi[p] = (int)(item_desc.size() / 4);
+        }
     }
-    int nseg_max = 1;
-    for (int p = 0; p < nprob; ++p) nseg_max = std::max(nseg_max, ((h_ld[p] >> 5) + kseg - 1) / kseg);
+    // the live work list of the unconverged chromosomes: packed, their descriptor ids (item_prob); int32, row groups of
+    // ~item_kb KB, a multiple of RG rows each (chromosome, first row, rows)
+    std::vector<int32_t> h_done(nprob, 0);
+    std::vector<int32_t> item_prob, item_row0, item_nrows;
     auto build_items = [&]() {
         item_prob.clear(); item_row0.clear(); item_nrows.clear();
-        std::vector<int> order(nprob);
-        for (int p = 0; p < nprob; ++p) order[p] = p;
-        std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return h_mat_n[a] > h_mat_n[b]; });
         for (int p : order) {
             const int n = h_mat_n[p];
             if (n == 0 || h_done[p]) continue;
             if (packed) {
-                const int KT = h_ld[p] >> 5;
-                auto lohi = [](int64_t v, int& a, int& b) { a = (int)(uint32_t)(v & 0xffffffffll); b = (int)(v >> 32); };
-                if (desc_built) {      // later builds: only the list of live item ids changes
-                    for (int id = desc_lo[p]; id < desc_hi[p]; ++id) { item_prob.push_back(id); item_row0.push_back(0); item_nrows.push_back(0); }
-                    continue;
-                }
-                for (int r0 = 0; r0 < n; r0 += V.rg)
-                    for (int k0 = 0; k0 < KT; k0 += kseg) {
-                        item_prob.push_back((int)(item_desc.size() / 4)); item_row0.push_back(r0); item_nrows.push_back(std::min(V.rg, n - r0));
-                        int4 d0, d1, d2, d3;
-                        lohi(h_qoff[p] + ((int64_t)(r0 / 16) * KT + k0) * 512, d0.x, d0.y);
-                        lohi((int64_t)(k0 / kseg) * npad + h_pad[p] + r0, d0.z, d0.w);
-                        lohi(8 * h_pad[p] + (int64_t)k0 * 256, d1.x, d1.y);
-                        lohi(h_binoff[p] + r0, d1.z, d1.w);
-                        d2 = make_int4(p, (int)h_pad[p], r0, std::min(V.rg, n - r0));
-                        d3 = make_int4(std::min(kseg, KT - k0), k0 / kseg, KT, 0);
-                        item_desc.push_back(d0); item_desc.push_back(d1); item_desc.push_back(d2); item_desc.push_back(d3);
-                    }
+                for (int id = desc_lo[p]; id < desc_hi[p]; ++id) item_prob.push_back(id);
                 continue;
             }
             int rows = (int)((int64_t)item_kb * 1024 / ((int64_t)h_ld[p] * 4));
@@ -1290,17 +1255,6 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
     };
     build_items();
     const size_t max_items = item_prob.size();
-    if (packed) {       // descriptor ids are positions in build order: remember each chromosome's id range
-        desc_built = true;
-        std::vector<int> cnt(nprob, 0);
-        for (size_t i = 0; i < item_desc.size(); i += 4) cnt[item_desc[i + 2].x]++;
-        // build order = chromosomes by decreasing size; ids are contiguous per chromosome in that order
-        std::vector<int> order(nprob);
-        for (int p = 0; p < nprob; ++p) order[p] = p;
-        std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return h_mat_n[a] > h_mat_n[b]; });
-        int run = 0;
-        for (int p : order) { desc_lo[p] = run; run += cnt[p]; desc_hi[p] = run; }
-    }
 
     Scratch scratch(s);
     double* d_vec = nullptr;     // [npad] bias | [npad] marg | [nprob+1] pad_off (as int64)
@@ -1380,22 +1334,19 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
     const size_t desc_at = (3 * max_items + (size_t)nprob + 4 + 3) & ~(size_t)3;
     const size_t tab_ints = desc_at + (packed ? 16 * max_items : 0);
     HC_CUDA(scratch.alloc((void**)&d_tab, tab_ints * sizeof(int32_t)));
-    bool desc_uploaded = false;
     auto upload_items = [&]() -> cudaError_t {
         const size_t n = item_prob.size();
         const int32_t n32 = (int32_t)n;
         cudaError_t e = cudaMemcpyAsync(d_tab + 3 * max_items + nprob + 3, &n32, sizeof(int32_t), cudaMemcpyHostToDevice, s);
         if (e == cudaSuccess) e = cudaMemcpyAsync(d_tab, item_prob.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, s);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d_tab + max_items, item_row0.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, s);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d_tab + 2 * max_items, item_nrows.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, s);
-        if (e == cudaSuccess && packed && !desc_uploaded) {
-            e = cudaMemcpyAsync(d_tab + desc_at, item_desc.data(), item_desc.size() * sizeof(int4), cudaMemcpyHostToDevice, s);
-            desc_uploaded = true;
-        }
+        // the packed kernel reads only the id list; its descriptors are uploaded once, below
+        if (e == cudaSuccess && !packed) e = cudaMemcpyAsync(d_tab + max_items, item_row0.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, s);
+        if (e == cudaSuccess && !packed) e = cudaMemcpyAsync(d_tab + 2 * max_items, item_nrows.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, s);
         if (e == cudaSuccess) e = cudaStreamSynchronize(s);   // the host vectors may be rebuilt afterwards
         return e;
     };
     HC_CUDA(cudaMemsetAsync(d_tab + 3 * max_items, 0, ((size_t)nprob + 3) * sizeof(int32_t), s));
+    if (packed) HC_CUDA(cudaMemcpyAsync(d_tab + desc_at, item_desc.data(), item_desc.size() * sizeof(int4), cudaMemcpyHostToDevice, s));
     HC_CUDA(upload_items());
     const int grid = hc_num_sms() * V.minb;    // persistent: every resident slot filled exactly once
     const unsigned int queue_start = (unsigned)grid * 8u;
@@ -1434,7 +1385,6 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
     // update kernel: the 8-CTA cluster version needs every chromosome to fit 8 x 256 x 4 padded columns
     bool cluster_update = packed;
     for (int p = 0; p < nprob; ++p) cluster_update = cluster_update && h_ld[p] <= UPD_CLUSTER * 256 * 4;
-    if (const char* e = getenv("HC_ICE_CLUSTER_UPDATE")) cluster_update = cluster_update && atoi(e) != 0;
     auto launch_update = [&]() {
         if (cluster_update) ice_q8_update_cluster_kernel<<<nprob * UPD_CLUSTER, 256, 0, s>>>(A);
         else ice_dense_update_kernel<<<nprob, 1024, 0, s>>>(A);
@@ -1444,12 +1394,8 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
     int rc = HC_OK;
     // `poll` iterations (stream + update kernel each) captured once and replayed: the iteration index,
     // the work-list length and every convergence decision live in device memory, so the graph is static
+    // (plain launches only when capture or instantiation fails).
     cudaGraphExec_t gexec = nullptr;
-    bool use_graph = true;
-    if (const char* e = getenv("HC_ICE_GRAPH")) use_graph = atoi(e) != 0;
-    // HC_ICE_TIME_KERNEL=1 (set by bench.py): the first stream-kernel launch of every graph replay is bracketed by a pair
-    // of events, so that its duration can be read back separately from the update kernel and the launch gaps (external
-    // event-record nodes inside the graph; bracketing all 8 launches of a replay cost ~11 us per iteration)
     // The captured graph is kept between calls (per host thread): the next call with the same launch shape only
     // rewrites the kernel parameters of its nodes (cudaGraphExecKernelNodeSetParams) instead of capturing and
     // instantiating again -- ~0.4 ms of host time per call on C2.
@@ -1460,7 +1406,7 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
         cudaGraphExec_t exec = nullptr;
         cudaGraph_t graph = nullptr;
         std::vector<cudaGraphNode_t> knodes;
-        void* fn = nullptr;
+        StreamKernel fn = nullptr;     // the packed kernel or one of the int32 kernels
         int grid = 0, poll = 0, nprob = 0, cluster = 0, timed = 0, dev = -1;
         cudaEvent_t ev[2] = {nullptr, nullptr};
         void drop() {
@@ -1478,8 +1424,8 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
     }
     double stream_ms_sum = 0.0;
     int stream_ms_n = 0;
-    if (use_graph) {
-        const bool hit = gc.exec != nullptr && gc.fn == (void*)V.fn && gc.grid == grid && gc.poll == poll && gc.nprob == nprob &&
+    {
+        const bool hit = gc.exec != nullptr && gc.fn == V.fn && gc.grid == grid && gc.poll == poll && gc.nprob == nprob &&
                          gc.cluster == (int)cluster_update && gc.timed == (int)!sev.ev.empty() && gc.dev == dev;
         cudaError_t e = cudaSuccess;
         if (hit) {
@@ -1517,7 +1463,7 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
                 }
             }
             if (e != cudaSuccess) { gc.drop(); (void)cudaGetLastError(); }   // plain launches below
-            else { gc.fn = (void*)V.fn; gc.grid = grid; gc.poll = poll; gc.nprob = nprob; gc.cluster = (int)cluster_update;
+            else { gc.fn = V.fn; gc.grid = grid; gc.poll = poll; gc.nprob = nprob; gc.cluster = (int)cluster_update;
                    gc.timed = (int)!sev.ev.empty(); gc.dev = dev; }
         }
         gexec = gc.exec;

@@ -554,7 +554,6 @@ int hc_ice_csr_balance_blocked(const int64_t* row_ptr, const int32_t* col, const
     }
     // ---- items: ~target entries each, never across a column block ------------------------------------------
     long long target = 64 * 1024;
-    if (const char* e = getenv("HC_CSRB_ITEM_ENTRIES")) target = std::max(1024ll, atoll(e));
     const int grid = hc_num_sms() * ST_MINB;
     while (target > 4096 && total_ent / target < 8ll * grid) target >>= 1;     // small problems: enough items for every CTA
     std::vector<int32_t> h_first(nb + 1, 0);
@@ -568,12 +567,8 @@ int hc_ice_csr_balance_blocked(const int64_t* row_ptr, const int32_t* col, const
     HC_CUDA(scratch.alloc((void**)&d_items, sizeof(int4) * (size_t)std::max(nitems, 1)));
     HC_CUDA(scratch.alloc((void**)&d_first, sizeof(int32_t) * (nb + 1)));
     HC_CUDA(cudaMemcpyAsync(d_first, h_first.data(), sizeof(int32_t) * (nb + 1), cudaMemcpyHostToDevice, s));
-    // average segment length from which a segment gets 4 / 8 / 16 / 32 lanes (HC_CSRB_GTHR="a,b,c,d" overrides)
-    int4 gthr = make_int4(8, 32, 128, 512);      // measured on C4 (profiles/README.md): flat between these and (20, 20, 192, 192)
-    if (const char* e = getenv("HC_CSRB_GTHR")) {
-        int a = 0, b = 0, c = 0, d = 0;
-        if (sscanf(e, "%d,%d,%d,%d", &a, &b, &c, &d) == 4) gthr = make_int4(a, b, c, d);
-    }
+    // average segment length from which a segment gets 4 / 8 / 16 / 32 lanes
+    const int4 gthr = make_int4(8, 32, 128, 512);      // measured on C4 (profiles/README.md): flat between these and (20, 20, 192, 192)
     if (nitems > 0) {
         csrb_items_kernel<<<(nitems + 255) / 256, 256, 0, s>>>(d_seg, nloc, nb, d_first, nitems, target, gthr, d_items);
         HC_LAUNCH_CHECK();
@@ -644,10 +639,8 @@ int hc_ice_csr_balance_blocked(const int64_t* row_ptr, const int32_t* col, const
     if (h_info != nullptr && getenv("HC_ICE_TIME_KERNEL") != nullptr && atoi(getenv("HC_ICE_TIME_KERNEL")) != 0) {
         if (cudaEventCreate(&tk0) != cudaSuccess || cudaEventCreate(&tk1) != cudaSuccess) { tk0 = nullptr; tk1 = nullptr; (void)cudaGetLastError(); }
     }
-    bool use_graph = true;
-    if (const char* e = getenv("HC_ICE_GRAPH")) use_graph = atoi(e) != 0;
-    cudaGraphExec_t gexec = nullptr;
-    if (use_graph) {
+    cudaGraphExec_t gexec = nullptr;      // plain launches below only when capture or instantiation fails
+    {
         cudaGraph_t graph = nullptr;
         cudaError_t e = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal);
         if (e == cudaSuccess) {

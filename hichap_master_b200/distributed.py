@@ -75,7 +75,7 @@ def exchange_entry_lists(up, lo, nbins: int):
 
 
 def _build_row_block_csr_two_keys(pairs: PairColumns, res: int, start, chrom_bins, nbins: int, cis_only=False):
-    """First version (two keys per pair, keys exchanged unreduced); HC_SORT_KEYS_PER_PAIR=2 or count-field overflow."""
+    """First version (two keys per pair, keys exchanged unreduced); the fallback on count-field overflow."""
     rank, world = dist.get_rank(), dist.get_world_size()
     dev = pairs.device
     col_bits = kernels.key_col_bits(nbins)
@@ -132,13 +132,10 @@ def build_row_block_csr(pairs: PairColumns, res: int, start, chrom_bins, nbins: 
     mark("start")
     flag = torch.zeros(1, dtype=torch.int32, device=dev)
     lists = None
-    if os.environ.get("HC_SORT_KEYS_PER_PAIR", "1") == "2":
+    try:
+        lists = kernels.pairs_to_entry_lists(pairs, res, start, chrom_bins, nbins, cis_only)
+    except kernels.CountFieldOverflow:
         flag += 1
-    else:
-        try:
-            lists = kernels.pairs_to_entry_lists(pairs, res, start, chrom_bins, nbins, cis_only)
-        except kernels.CountFieldOverflow:
-            flag += 1
     dist.all_reduce(flag)                      # all ranks take the same path
     if int(flag.item()):
         del lists

@@ -47,7 +47,7 @@ def bin_pairs_local(pairs: PairColumns, res: int, batch: DenseBatch, mode=_abi.H
 
 
 def bin_pairs_local_banded(pairs: PairColumns, res: int, batch: DenseBatch, mode=_abi.HC_BIN_SYM_ALL,
-                           check_bounds=True, work=None, band_width=None, oob=None):
+                           check_bounds=True, work=None, band_width=128, oob=None):
     """``bin_pairs_local`` for the symmetric modes on matrices that are symmetric on entry
     (freshly zeroed tiles): upper-triangle-only updates with an L2-resident near-diagonal band
     accumulator, band merge, mirror.  Falls back to the direct kernel outside its limits.
@@ -55,8 +55,6 @@ def bin_pairs_local_banded(pairs: PairColumns, res: int, batch: DenseBatch, mode
     if len(batch) > 256 or mode == _abi.HC_BIN_ONESIDED or batch.nbins == 0:
         bin_pairs_local(pairs, res, batch, mode, check_bounds, oob=oob)
         return work
-    if band_width is None:
-        band_width = int(os.environ.get("HC_BIN_BAND", "128"))
     oob = _oob_counter(batch.device) if oob is None else oob
     nbytes = int(lib().hc_bin_band_work_bytes(batch.nbins, band_width))
     if work is None or work.numel() < nbytes:
@@ -75,11 +73,11 @@ class BandedBinning:
     """begin -> accumulate(chunk) x N -> finish: banded binning fed chunk by chunk (e.g. while later
     chunks are still in flight over PCIe).  Chromosome columns may be int32 or uint8 (255 = filtered)."""
 
-    def __init__(self, batch: DenseBatch, res: int, mode=_abi.HC_BIN_SYM_ALL, work=None, band_width=None, oob=None):
+    def __init__(self, batch: DenseBatch, res: int, mode=_abi.HC_BIN_SYM_ALL, work=None, band_width=128, oob=None):
         if len(batch) > 256 or mode == _abi.HC_BIN_ONESIDED:
             raise ValueError("banded binning: symmetric modes, at most 256 matrices")
         self.batch, self.res, self.mode = batch, int(res), int(mode)
-        self.bw = int(os.environ.get("HC_BIN_BAND", "128")) if band_width is None else int(band_width)
+        self.bw = int(band_width)
         self.oob = _oob_counter(batch.device) if oob is None else oob
         nbytes = int(lib().hc_bin_band_work_bytes(batch.nbins, self.bw))
         if work is None or work.numel() < nbytes:
@@ -475,42 +473,12 @@ def entries_to_csr(up, lo, n_lo, nbins: int, nrows: int, row0: int = 0, total=No
     return row_ptr, col, cnt
 
 
-def transpose_entries(up, nbins: int, lo=None, tmp=None):
-    """Lower-triangle list of an upper list: swapped entries, sorted by (row, col).  Returns (lo_sorted, n_lo device
-    scalar); the diagonal cells end up as padding keys behind the first n_lo entries."""
-    dev, n = up.device, int(up.numel())
-    cb, cnt_bits = key_col_bits(nbins), entry_cnt_bits(nbins)
-    if lo is None or lo.numel() < n:
-        lo = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
-    lo = lo[:n]
-    n_lo = torch.zeros(1, dtype=torch.int64, device=dev)
-    check(lib().hc_entries_transpose(ptr(up), n, cb, cnt_bits, ptr(lo), ptr(n_lo), stream_ptr()), "hc_entries_transpose")
-    if tmp is not None:
-        tmp = tmp[:n] if tmp.numel() >= n else None
-    slo, _ = sort_entries(lo, nbins, cnt_bits + cb, 1, tmp=tmp)
-    return slo, n_lo
-
-
 def _pairs_to_csr_two_keys(pairs: PairColumns, res: int, start, chrom_bins, nbins: int, cis_only: bool,
                            check_bounds=True) -> SymCsr:
     """The first version of the sort path: two keys per off-diagonal pair, five digit passes over all of them.
-    Kept as the fallback for counts that overflow the entry count field and for A/B measurements
-    (HC_SORT_KEYS_PER_PAIR=2)."""
-    dev = pairs.device
-    col_bits = key_col_bits(nbins)
-    keys = torch.empty(2 * max(pairs.n, 1), dtype=torch.int64, device=dev)
-    n_valid = torch.zeros(1, dtype=torch.int64, device=dev)
-    oob = torch.zeros(1, dtype=torch.int64, device=dev)
-    check(lib().hc_pairs_to_keys(ptr(pairs.c1), ptr(pairs.p1), ptr(pairs.c2), ptr(pairs.p2), pairs.n, int(res),
-                                 ptr(start), ptr(chrom_bins), int(start.numel()), int(bool(cis_only)), col_bits,
-                                 ptr(keys), ptr(n_valid), ptr(oob), stream_ptr()), "hc_pairs_to_keys")
-    if check_bounds:
-        _raise_oob(oob, "genome-wide")
-    keys = keys[:2 * pairs.n]
-    # padding keys are ~0: they sort last on every digit, so sorting the low key_sort_bits(nbins) bits
-    # (rounded up to whole 8-bit digits) leaves the real keys first and in order
-    skeys, free = sort_keys_u64(keys, key_sort_bits(nbins)) if pairs.n else (keys, None)
-    row_ptr, col, cnt = keys_to_csr(skeys, n_valid, col_bits, nbins, scratch=free)
+    Kept as the fallback for counts that overflow the entry count field."""
+    skeys, free, n_valid = pairs_to_sorted_keys(pairs, res, start, chrom_bins, nbins, cis_only, check_bounds)
+    row_ptr, col, cnt = keys_to_csr(skeys, n_valid, key_col_bits(nbins), nbins, scratch=free)
     return SymCsr(row_ptr, col, cnt, nbins)
 
 
@@ -519,7 +487,7 @@ def pairs_to_csr(pairs: PairColumns, res: int, start, chrom_bins, nbins: int, ci
     """Binning through the sort path (north_star kernel (a)): every pair becomes ONE 64-bit entry of its
     upper-triangle cell; the entries are radix-sorted and reduced by cell; the lower triangle is the swapped list
     re-sorted on its row bits only; the symmetric CSR is the row-wise concatenation of the two lists."""
-    if os.environ.get("HC_SORT_KEYS_PER_PAIR", "1") == "2" or pairs.n == 0:
+    if pairs.n == 0:
         return _pairs_to_csr_two_keys(pairs, res, start, chrom_bins, nbins, cis_only, check_bounds)
     try:
         up, slo, n_lo = pairs_to_entry_lists(pairs, res, start, chrom_bins, nbins, cis_only, check_bounds)

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """C4 on one GPU: sort path once, then the CSR ICE (filters + column-blocked encoding + iteration graph) twice; prints
 the event times.  Under `ncu --metrics gpu__time_duration.sum ... -k regex:'csrb|ice_|mad_|nccl'` it gives the launch
-list of the set-up kernels (HC_ICE_GRAPH=0 makes the iteration kernels visible to ncu one by one)."""
+list of the set-up kernels."""
 import argparse
 import json
 import os

@@ -1,4 +1,4 @@
-"""C4-shaped genome-wide 10 kb CSR (hg19, 25 % trans) + a few ICE iterations with plain launches (no graph), for
+"""C4-shaped genome-wide 10 kb CSR (hg19, 25 % trans) + a few ICE iterations, for
 `ncu -k regex:csrb_stream`:  python profiles/ncu_csr_ice.py [pairs] [iters]"""
 import os
 import sys
@@ -7,7 +7,6 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-os.environ.setdefault("HC_ICE_GRAPH", "0")
 from hichap_master_b200 import kernels, matrixBuilding as mb, synth  # noqa: E402
 from hichap_master_b200.device import PairColumns  # noqa: E402
 

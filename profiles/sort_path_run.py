@@ -39,5 +39,4 @@ for rep in range(a.reps):
     ms.append(e0.elapsed_time(e1))
     nnz = csr.nnz
     del csr
-print(json.dumps({"pairs": a.pairs, "bins": total, "nnz_stored": nnz, "ms": ms,
-                  "keys_per_pair": os.environ.get("HC_SORT_KEYS_PER_PAIR", "1")}))
+print(json.dumps({"pairs": a.pairs, "bins": total, "nnz_stored": nnz, "ms": ms}))

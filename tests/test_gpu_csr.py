@@ -52,10 +52,10 @@ def small_case(seed, n_pairs, trans):
 @pytest.mark.parametrize("keys_per_pair", ["1", "2"])
 @pytest.mark.parametrize("res,cis_only,npairs", [(40000, False, 60_000), (40000, True, 60_000), (500000, False, 5_000),
                                                  (10000, False, 7), (40000, False, 0)])
-def test_pairs_to_csr_matches_oracle(K, cuda_device, monkeypatch, res, cis_only, npairs, keys_per_pair):
+def test_pairs_to_csr_matches_oracle(K, cuda_device, res, cis_only, npairs, keys_per_pair):
     """keys_per_pair=1: the default (one upper-triangle entry per pair, lower list by a row-bits re-sort);
-    2: the first version (both orientations sorted)."""
-    monkeypatch.setenv("HC_SORT_KEYS_PER_PAIR", keys_per_pair)
+    2: the first version (both orientations sorted), the fallback on count-field overflow."""
+    import torch
     from hichap_master_b200 import matrixBuilding as mb
     from hichap_master_b200.device import PairColumns
     genome, order, c1, p1, c2, p2 = small_case(5, max(npairs, 1), 0.2)
@@ -64,6 +64,11 @@ def test_pairs_to_csr_matches_oracle(K, cuda_device, monkeypatch, res, cis_only,
     table, total = ho.chro_bins(genome, res)
     assert bins == table and csr.nbins == total
     start = np.array([table[c][0] for c in order], np.int64)
+    if keys_per_pair == "2":
+        chrom_bins = torch.tensor([genome[c] // res + 1 for c in order], dtype=torch.int32, device=cuda_device)
+        csr = K._pairs_to_csr_two_keys(PairColumns(c1, p1, c2, p2, device=cuda_device), res,
+                                       torch.from_numpy(start).to(cuda_device), chrom_bins, total, cis_only)
+        assert csr.nbins == total
     keep = (c1 == c2) if cis_only else np.ones(c1.size, bool)
     M = ho.bin_whole_dense(c1[keep], p1[keep], c2[keep], p2[keep], start, start, total, res)
     # full symmetric CSR
@@ -235,7 +240,7 @@ def _random_pairs_one_chrom(nb, res, npairs, seed, hot=0.0):
 
 
 @pytest.mark.parametrize("nb", [1024, 777, 1])
-def test_entry_path_equals_two_key_path(K, cuda_device, monkeypatch, nb):
+def test_entry_path_equals_two_key_path(K, cuda_device, nb):
     """Same symmetric CSR from both versions of the sort path, incl. a power-of-two bin count (padding-bit case)
     and dropped pairs (padding keys in the middle of the list)."""
     import torch
@@ -247,9 +252,8 @@ def test_entry_path_equals_two_key_path(K, cuda_device, monkeypatch, nb):
     start = torch.zeros(1, dtype=torch.int64, device=cuda_device)
     chrom_bins = torch.tensor([nb], dtype=torch.int32, device=cuda_device)
     out = {}
-    for mode in ("1", "2"):
-        monkeypatch.setenv("HC_SORT_KEYS_PER_PAIR", mode)
-        csr = K.pairs_to_csr(PairColumns(c1, p1, c1, p2, device=cuda_device), res, start, chrom_bins, nb, False)
+    for mode, build in (("1", K.pairs_to_csr), ("2", K._pairs_to_csr_two_keys)):
+        csr = build(PairColumns(c1, p1, c1, p2, device=cuda_device), res, start, chrom_bins, nb, False)
         out[mode] = [t.cpu().numpy() for t in (csr.row_ptr, csr.col, csr.cnt)]
     for a, b in zip(out["1"], out["2"]):
         assert np.array_equal(a, b)

@@ -288,9 +288,15 @@ def _ice_vs_oracle(mb, mats, what, **kw):
 @pytest.mark.parametrize("env,sizes,kw", [
     ({}, (700, 333), dict()),                                        # packed encoding, cluster update kernel
     ({}, (700, 333), dict(ignore_diags=0)),                          # kept diagonal counts twice: values up to 2 x count
-    ({"HC_ICE_KSEG": "4"}, (1500,), dict()),                         # 12 K-segments per row: more than the unrolled 8
-    ({"HC_ICE_KSEG": "8", "HC_ICE_Q8_VARIANT": "0"}, (900, 40), dict()),   # two strips per work item
-    ({"HC_ICE_CLUSTER_UPDATE": "0"}, (700, 333), dict()),            # single-CTA update kernel on the packed encoding
+    # K segments of the packed kernel: kseg starts at 48 k-tiles and drops by 16 (floor 16) while the batch has fewer
+    # than 4 x SMs x 2 x 8 items (9472 on 148 SMs); items = ceil(n / 16) x ceil(KT / kseg), KT = ceil(n / 128) x 4.
+    # 5000 bins: KT = 160; 313 x 4 = 1252 items at kseg 48, 1565 at 32 -> kseg 16, 10 segments per row: more than
+    # the unrolled 8 of the cluster update kernel
+    ({}, (5000,), dict()),
+    # 8200 bins have 8320 padded columns, more than the 8 x 256 x 4 of the cluster update: the single-CTA update
+    # kernel runs for the whole batch (kseg 16), its general packed branch for 8200 and, for 5000, its
+    # register-resident branch with 10 segments, so that branch's loop over segments beyond 8 runs too
+    ({}, (8200, 5000), dict()),
     ({"HC_ICE_PACKED": "0"}, (700, 333), dict()),                    # int32 tiles, fp64 FMA kernel
     ({"HC_ICE_PACKED": "1"}, (700, 333), dict()),                    # full-matrix packed encoding, one launch pair per iteration
     ({}, (700, 333), dict(ignore_diags=3)),
