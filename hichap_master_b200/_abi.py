@@ -87,6 +87,12 @@ SIGNATURES = {
     "hc_distance_sums_f64": (C.c_int, [_P, _I64, _I32, _P, _P, _P]),
     "hc_observed_expected_f64": (C.c_int, [_P, _I64, _I32, _P, _P, _I64, _P]),
     "hc_directionality_index_f64": (C.c_int, [_P, _I64, _I32, _P, _P, _I32, _P, _P]),
+    "hc_balance_apply_csr_i32": (C.c_int, [_P, _P, _P, _I32, _P, _P, _P]),
+    "hc_colnnz_csr": (C.c_int, [_P, _I64, _I32, _P, _P]),
+    "hc_distance_sums_csr_work_bytes": (C.c_int64, [_I64]),
+    "hc_distance_sums_csr_f64": (C.c_int, [_P, _P, _P, _I64, _I32, _P, _P, _P, _P]),
+    "hc_observed_expected_csr_f64": (C.c_int, [_P, _P, _P, _I32, _P, _P, _P]),
+    "hc_directionality_index_csc_f64": (C.c_int, [_P, _P, _P, _I32, _P, _P, _I32, _P, _P]),
     "hc_pairs_to_keys": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _P, _P, _I32, _I32, _I32, _P, _P, _P, _P]),
     "hc_sort_work_bytes": (C.c_int64, [_I64]),
     "hc_sort_keys_u64": (C.c_int, [_P, _P, _I64, _I32, _I32, _P, C.POINTER(_I32), _P]),

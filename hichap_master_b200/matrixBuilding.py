@@ -492,9 +492,10 @@ def _is_sparse(*mats):
     return any(sp.issparse(m) for m in mats)
 
 
-def _device_csr(m, cls):
-    """host matrix of integer counts (scipy.sparse or dense) -> device CSR: duplicates summed, explicit zeros dropped
-    (coverage counts the stored entries), columns sorted"""
+def _device_csr(m, cls, dtype=np.int32):
+    """host matrix (scipy.sparse or dense) -> device CSR: duplicates summed, explicit zeros dropped (coverage counts the
+    stored entries), columns sorted.  ``dtype`` int32: integer counts (``as_int32_counts``); float64: values as they
+    are.  The input is not modified; the canonical host copy is kept as ``.host``."""
     import scipy.sparse as sp
     m = sp.csr_matrix(m, copy=True)
     m.sum_duplicates()
@@ -502,7 +503,10 @@ def _device_csr(m, cls):
     m.sort_indices()
     dev = require_cuda()
     up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt)).to(dev)
-    return cls(up(m.indptr, np.int64), up(m.indices, np.int32), up(as_int32_counts(m.data), np.int32), m.shape[0])
+    vals = as_int32_counts(m.data) if dtype == np.int32 else m.data
+    X = cls(up(m.indptr, np.int64), up(m.indices, np.int32), up(vals, dtype), m.shape[0])
+    X.host = m
+    return X
 
 
 def _twostep_sparse(tra, hap):

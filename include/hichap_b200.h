@@ -457,6 +457,30 @@ int hc_observed_expected_f64(const double* M, int64_t ld, int32_t n, const doubl
 int hc_directionality_index_f64(const double* M, int64_t ld, int32_t n, const uint8_t* gapflag, const int32_t* window_bin,
                                 int32_t chitest, double* di, void* stream);
 
+/* The same consumers on a canonical CSR of an n x n matrix, for resolutions whose dense matrix does not fit (memory
+ * O(nnz + n)): row_ptr int64[n+1], col int32[nnz], rows sorted by column, no duplicate cells, no explicit zeros.
+ * Per-entry outputs (out[nnz]) have the pattern of the input.
+ *   hc_balance_apply_csr_i32         out[e] = nan_to_num(cnt[e] * w_i * w_j), bit-identical to hc_balance_apply_i32
+ *   hc_colnnz_csr                    stored entries per column (colnnz[n] is zeroed by the call)
+ *   hc_distance_sums_csr_f64         dsum[n] as hc_distance_sums_f64: entries keyed (|i-j| << idx_bits) | entry, stable
+ *                                    radix sort on the distance bits, one warp per distance; a fixed order, so repeated
+ *                                    calls are bit-identical (the order differs from the dense kernel's).
+ *                                    work: hc_distance_sums_csr_work_bytes(nnz)
+ *   hc_observed_expected_csr_f64     out[e] = val[e] / decline[|i-j|], bit-identical to hc_observed_expected_f64
+ *   hc_directionality_index_csc_f64  Get_DI on the column-compressed matrix (col_ptr[n+1], row[nnz]: the CSR of the
+ *                                    transpose), missing cells read as 0.0: bit-identical to hc_directionality_index_f64 */
+int hc_balance_apply_csr_i32(const int64_t* row_ptr, const int32_t* col, const int32_t* cnt, int32_t n, const double* weight,
+                             double* out, void* stream);
+int hc_colnnz_csr(const int32_t* col, int64_t nnz, int32_t n, int32_t* colnnz, void* stream);
+int64_t hc_distance_sums_csr_work_bytes(int64_t nnz);
+int hc_distance_sums_csr_f64(const int64_t* row_ptr, const int32_t* col, const double* val, int64_t nnz, int32_t n,
+                             const uint8_t* gapflag, double* dsum, void* work, void* stream);
+int hc_observed_expected_csr_f64(const int64_t* row_ptr, const int32_t* col, const double* val, int32_t n,
+                                 const double* decline, double* out, void* stream);
+int hc_directionality_index_csc_f64(const int64_t* col_ptr, const int32_t* row, const double* val, int32_t n,
+                                    const uint8_t* gapflag, const int32_t* window_bin, int32_t chitest, double* di,
+                                    void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Valid-pair text ingest (host, multithreaded; SURVEY.md section 8f row 1): parses the 23-column
  * *_Valid.bed (layout 0: chromosomes in columns 1 and 8, fragment mid-points in columns 6 and 13;
