@@ -7,8 +7,8 @@
 //       marg[r] = b[r] * sum_j w(r,j) A[r][j] b[j]   (fp64, warp-shuffle reduction, one store per row);
 //   update kernel (one CTA per chromosome): mean / variance of the fresh marginals over the non-zero bins,
 //       b <- b / (marg / mean), convergence test var < tol, bookkeeping -- all on the device.
-// `poll` iterations are captured once as a CUDA graph and replayed; nothing goes back to the host inside
-// the loop except a done-counter poll through a pinned mailbox.
+// The whole loop is one launch of a CUDA graph (a WHILE node that the last update CTA of an iteration ends), and the
+// update kernel also drops converged chromosomes from the work list: nothing goes back to the host inside the loop.
 //
 // Two encodings of the matrix for the stream kernel:
 //   * int32 tiles as they are (ice_dense_stream_kernel): 4*N^2 bytes per iteration per chromosome, fp64 FMAs;
@@ -47,38 +47,40 @@ __device__ __forceinline__ double band_weight(int j, int r, int kd) {
 // ---------------------------------------------------------------------------------------
 // filter marginals: per bin, count and sum of kept pixels
 // ---------------------------------------------------------------------------------------
+// one warp per global bin, grid-stride: the number of bins is read here, so the host launches without waiting for it
 __global__ void __launch_bounds__(256)
 ice_dense_marginals_kernel(const int32_t* __restrict__ mats, const int64_t* __restrict__ mat_off,
                            const int32_t* __restrict__ mat_n, const int32_t* __restrict__ mat_ld,
                            const int64_t* __restrict__ bin_off, int nprob, int kd,
                            double* __restrict__ nnz_marg, double* __restrict__ marg) {
-    const int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;  // global bin == one warp
     const int lane = threadIdx.x & 31;
-    if (g >= bin_off[nprob]) return;
-    int p = 0;
-    while (p + 1 < nprob && bin_off[p + 1] <= g) ++p;
-    const int r = (int)(g - bin_off[p]), n = mat_n[p];
-    const int64_t ld = mat_ld[p];
-    const int32_t* row = mats + mat_off[p] + (int64_t)r * ld;
-    const int nvec = (int)(ld >> 2);
-    long long s = 0;
-    int c = 0;
-    for (int v = lane; v < nvec; v += 32) {
-        const int4 a = ld_stream_v4(row + 4 * v);
-        const int j = 4 * v;
-        const int x[4] = {a.x, a.y, a.z, a.w};
+    const int64_t nbins = bin_off[nprob], nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; g < nbins; g += nwarps) {
+        int p = 0;
+        while (p + 1 < nprob && bin_off[p + 1] <= g) ++p;
+        const int r = (int)(g - bin_off[p]), n = mat_n[p];
+        const int64_t ld = mat_ld[p];
+        const int32_t* row = mats + mat_off[p] + (int64_t)r * ld;
+        const int nvec = (int)(ld >> 2);
+        long long s = 0;
+        int c = 0;
+        for (int v = lane; v < nvec; v += 32) {
+            const int4 a = ld_stream_v4(row + 4 * v);
+            const int j = 4 * v;
+            const int x[4] = {a.x, a.y, a.z, a.w};
 #pragma unroll
-        for (int e = 0; e < 4; ++e) {
-            if (j + e < n) {
-                const double w = band_weight(j + e, r, kd);
-                s += (long long)(w * x[e]);
-                c += (x[e] != 0) ? (int)w : 0;
+            for (int e = 0; e < 4; ++e) {
+                if (j + e < n) {
+                    const double w = band_weight(j + e, r, kd);
+                    s += (long long)(w * x[e]);
+                    c += (x[e] != 0) ? (int)w : 0;
+                }
             }
         }
+        s = warp_sum_ll(s);
+        c = warp_sum_i(c);
+        if (lane == 0) { marg[g] = (double)s; nnz_marg[g] = (double)c; }
     }
-    s = warp_sum_ll(s);
-    c = warp_sum_i(c);
-    if (lane == 0) { marg[g] = (double)s; nnz_marg[g] = (double)c; }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -327,9 +329,18 @@ struct IceDenseArgs {
     const int4* desc; int kseg;                 // packed items: 4 x int4 descriptors (see ice_q8_mma_kernel); a row group is split
                                                 // along K into segments of kseg k-tiles
     double* part; int nseg_max; long long npad; // partial row sums part[(k0 / kseg) * npad + pad_off + row], summed by the update kernel
-    const int64_t* bin_off;
     const int64_t* ovf_ptr; const int32_t* ovf_col; const int32_t* ovf_val;   // per global row: cells with w*count > 255
     int packed;
+    // loop control on the device (ice_iteration_end): the last update CTA of an iteration rewrites the live work list when
+    // a chromosome has converged, and sets the condition of the graph's WHILE node
+    int nonempty;               // chromosomes with at least one bin: the loop ends when n_done reaches it
+    unsigned int* upd_cnt;      // update CTAs that finished the current launch
+    int32_t* changed;           // a chromosome converged in the current iteration
+    const int32_t* rng;         // chromosomes, largest first: [nprob] chromosome | [nprob] first item | [nprob] item end
+    int32_t* rng_off;           // [nprob] their offsets in the live work list
+    const int32_t* full_row0; const int32_t* full_nrows;   // int32 kernel: the full list of items that the live list filters
+    cudaGraphConditionalHandle cond; int has_cond;         // has_cond == 0: plain launches, the host polls n_done
+    int loop_end;               // this update launch ends a graph body (or a plain-launch iteration): runs ice_iteration_end
 };
 
 // one column chunk (128 columns, 4 per lane) of RG rows: acc[q] += sum_j w * A[rq][j] * b[j]
@@ -598,9 +609,20 @@ ice_pack_ovf_kernel(const int32_t* __restrict__ mats, const int64_t* __restrict_
                     const int32_t* __restrict__ mat_n, const int32_t* __restrict__ mat_ld,
                     const int64_t* __restrict__ bin_off, int nprob, int kd, const int64_t* __restrict__ ovf_ptr,
                     const int32_t* __restrict__ ovf_lo, const int32_t* __restrict__ ovf_hi,
-                    int32_t* __restrict__ ovf_col, int32_t* __restrict__ ovf_val) {
+                    int32_t* __restrict__ ovf_col, int32_t* __restrict__ ovf_val, long long cap, IceDenseArgs A,
+                    int32_t* __restrict__ abort_flag) {
     const int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
+    if (ovf_ptr[bin_off[nprob]] > cap) {
+        // more overflow cells than the arrays hold: write none, mark every chromosome done so that the loop streams
+        // nothing, and leave the caller's bias alone (ice_finalize_kernel); the host grows the arrays and runs again
+        if (g == 0 && lane == 0) {
+            *abort_flag = 1;
+            for (int p = 0; p < nprob; ++p) A.done[p] = 1;
+            *A.n_done = A.nonempty;
+        }
+        return;
+    }
     if (g >= bin_off[nprob]) return;
     int64_t out = ovf_ptr[g];
     if (ovf_ptr[g + 1] == out) return;
@@ -723,11 +745,77 @@ ice_q8_mma_kernel(IceDenseArgs A) {
     }
 }
 
+__device__ __forceinline__ void ice_mark_done(const IceDenseArgs& A, int p) {
+    A.done[p] = 1;
+    atomicAdd(A.n_done, 1);
+    *A.changed = 1;
+}
+
+// The live work list after a convergence: the items of the chromosomes still running, in the order of A.rng (largest
+// first), and their number.  Run by the whole last CTA of an update launch, when every other CTA has finished.
+__device__ void ice_compact_items(const IceDenseArgs& A) {
+    __shared__ int wsum[32];
+    __shared__ int total_s;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5, nprob = A.nprob;
+    if (threadIdx.x == 0) total_s = 0;
+    __syncthreads();
+    for (int i0 = 0; i0 < nprob; i0 += blockDim.x) {      // exclusive scan of the live item counts
+        const int i = i0 + threadIdx.x;
+        const int cnt = i < nprob && !__ldcg(A.done + A.rng[i]) ? A.rng[2 * nprob + i] - A.rng[nprob + i] : 0;
+        int inc = cnt;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += t; }
+        if (lane == 31) wsum[wid] = inc;
+        __syncthreads();
+        int off = total_s;
+        for (int w = 0; w < wid; ++w) off += wsum[w];
+        if (i < nprob) A.rng_off[i] = off + inc - cnt;
+        __syncthreads();
+        if (threadIdx.x == blockDim.x - 1) total_s = off + inc;
+        __syncthreads();
+    }
+    int32_t* prob = const_cast<int32_t*>(A.item_prob);
+    int32_t* row0 = const_cast<int32_t*>(A.item_row0);
+    int32_t* nrows = const_cast<int32_t*>(A.item_nrows);
+    for (int i = wid; i < nprob; i += nw) {                // one warp per chromosome
+        const int p = A.rng[i];
+        if (__ldcg(A.done + p)) continue;
+        const int lo = A.rng[nprob + i], m = A.rng[2 * nprob + i] - lo, off = A.rng_off[i];
+        for (int j = lane; j < m; j += 32) {
+            if (A.packed) { prob[off + j] = lo + j; continue; }      // packed: descriptor ids
+            prob[off + j] = p; row0[off + j] = A.full_row0[lo + j]; nrows[off + j] = A.full_nrows[lo + j];
+        }
+    }
+    if (threadIdx.x == 0) { *const_cast<unsigned int*>(A.nitems) = (unsigned)total_s; *A.changed = 0; }
+}
+
+// Tail of the update launch that ends a graph body: the last CTA to finish compacts the work list if a chromosome
+// converged, and decides whether the graph's WHILE node runs another body -- so the loop needs no host round trip.
+__device__ void ice_iteration_end(const IceDenseArgs& A) {
+    __shared__ int last_s;
+    if (!A.loop_end) return;    // within a graph body the stream kernel skips the items of converged chromosomes
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const unsigned t = atomicAdd(A.upd_cnt, 1u);
+        last_s = t == gridDim.x - 1;
+        if (last_s) *A.upd_cnt = 0;
+    }
+    __syncthreads();
+    if (!last_s) return;
+    __threadfence();
+    if (*reinterpret_cast<volatile int32_t*>(A.changed)) ice_compact_items(A);
+    if (threadIdx.x == 0 && A.has_cond) {
+        const int k = *reinterpret_cast<volatile int32_t*>(A.iter);
+        const int nd = *reinterpret_cast<volatile int32_t*>(A.n_done);
+        cudaGraphSetConditional(A.cond, nd < A.nonempty && k < A.max_iters ? 1u : 0u);
+    }
+}
+
 // Vector half of an iteration (grid = one CTA per chromosome): mean / variance of the fresh
 // marginals over the non-zero bins, bias update b /= marg/mean (in place), convergence test,
 // scale / iteration bookkeeping -- all on the device.
-__global__ void __launch_bounds__(1024)
-ice_dense_update_kernel(IceDenseArgs A) {
+__device__ __forceinline__ void ice_dense_update(const IceDenseArgs& A) {
     __shared__ double red[32];
     __shared__ long long redll[32];
     const int p = blockIdx.x;
@@ -796,7 +884,7 @@ ice_dense_update_kernel(IceDenseArgs A) {
         if (c == 0) {   // nothing left to balance: cooler sets bias = NaN, scale = NaN, var = 0
             if (threadIdx.x == 0) {
                 hc_ice_result r; r.scale = nan; r.var = 0.0; r.iters = k; r.converged = 1;
-                A.results[p] = r; A.done[p] = 1; atomicAdd(A.n_done, 1);
+                A.results[p] = r; ice_mark_done(A, p);
             }
             return;
         }
@@ -832,7 +920,7 @@ ice_dense_update_kernel(IceDenseArgs A) {
             A.dig_exp[p] = E;
             hc_ice_result r; r.scale = mean; r.var = var; r.iters = k; r.converged = var < A.tol;
             A.results[p] = r;
-            if (var < A.tol || k >= A.max_iters) { A.done[p] = 1; atomicAdd(A.n_done, 1); }
+            if (var < A.tol || k >= A.max_iters) { ice_mark_done(A, p); }
         }
         return;
     }
@@ -857,7 +945,7 @@ ice_dense_update_kernel(IceDenseArgs A) {
         if (threadIdx.x == 0) {
             hc_ice_result r; r.scale = nan; r.var = 0.0;
             r.iters = k; r.converged = 1;
-            A.results[p] = r; A.done[p] = 1; atomicAdd(A.n_done, 1);
+            A.results[p] = r; ice_mark_done(A, p);
         }
         return;
     }
@@ -876,12 +964,17 @@ ice_dense_update_kernel(IceDenseArgs A) {
     if (threadIdx.x == 0) {
         hc_ice_result r; r.scale = mean; r.var = var; r.iters = k; r.converged = var < A.tol;
         A.results[p] = r;
-        if (var < A.tol || k >= A.max_iters) { A.done[p] = 1; atomicAdd(A.n_done, 1); }
+        if (var < A.tol || k >= A.max_iters) { ice_mark_done(A, p); }
     }
     if (A.packed) {      // the stream kernel reads the bias as byte planes
         __syncthreads();
         ice_write_digits(bw, n, A.mat_ld[p], A.digits + 8 * lo, A.dig_exp + p, red);
     }
+}
+__global__ void __launch_bounds__(1024)
+ice_dense_update_kernel(IceDenseArgs A) {
+    ice_dense_update(A);
+    ice_iteration_end(A);
 }
 
 // The same update for the packed encoding when every chromosome has at most 8192 padded columns: a thread-block
@@ -890,8 +983,7 @@ ice_dense_update_kernel(IceDenseArgs A) {
 // single-CTA kernel above spends ~25 us per iteration on this (latency: six block barriers, 16 fp64 divisions and
 // 450 KB through one SM); that is a third of an iteration once the matrix pass takes ~50 us.
 constexpr int UPD_CLUSTER = 8;
-__global__ void __cluster_dims__(UPD_CLUSTER, 1, 1) __launch_bounds__(256)
-ice_q8_update_cluster_kernel(IceDenseArgs A) {
+__device__ __forceinline__ void ice_q8_update_cluster(const IceDenseArgs& A) {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     __shared__ double red[8];
@@ -952,7 +1044,7 @@ ice_q8_update_cluster_kernel(IceDenseArgs A) {
     if (c == 0) {   // nothing left to balance: cooler sets bias = NaN, scale = NaN, var = 0
         if (rank == 0 && threadIdx.x == 0) {
             hc_ice_result r; r.scale = nan; r.var = 0.0; r.iters = k; r.converged = 1;
-            A.results[p] = r; A.done[p] = 1; atomicAdd(A.n_done, 1);
+            A.results[p] = r; ice_mark_done(A, p);
         }
         cluster.sync();      // nobody leaves while its shared memory may still be read
         return;
@@ -990,9 +1082,14 @@ ice_q8_update_cluster_kernel(IceDenseArgs A) {
         A.dig_exp[p] = E;
         hc_ice_result r; r.scale = mean; r.var = var; r.iters = k; r.converged = var < A.tol;
         A.results[p] = r;
-        if (var < A.tol || k >= A.max_iters) { A.done[p] = 1; atomicAdd(A.n_done, 1); }
+        if (var < A.tol || k >= A.max_iters) { ice_mark_done(A, p); }
     }
     cluster.sync();          // keep every CTA's shared memory alive until the remote reads are done
+}
+__global__ void __cluster_dims__(UPD_CLUSTER, 1, 1) __launch_bounds__(256)
+ice_q8_update_cluster_kernel(IceDenseArgs A) {
+    ice_q8_update_cluster(A);
+    ice_iteration_end(A);
 }
 
 // user bias (concatenated bins) <-> padded internal layout
@@ -1010,9 +1107,9 @@ ice_pad_bias_kernel(const int64_t* __restrict__ bin_off, const int64_t* __restri
 __global__ void __launch_bounds__(256)
 ice_finalize_kernel(const int64_t* __restrict__ bin_off, const int64_t* __restrict__ pad_off, int nprob,
                     const hc_ice_result* __restrict__ results, int rescale, const double* __restrict__ padded,
-                    double* __restrict__ bias) {
+                    double* __restrict__ bias, const int32_t* __restrict__ abort_flag) {
     const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (g >= bin_off[nprob]) return;
+    if (g >= bin_off[nprob] || *abort_flag) return;
     int p = 0;
     while (p + 1 < nprob && bin_off[p + 1] <= g) ++p;
     const hc_ice_result r = results[p];
@@ -1026,18 +1123,7 @@ ice_finalize_kernel(const int64_t* __restrict__ bin_off, const int64_t* __restri
     bias[g] = b;
 }
 
-// stream-ordered scratch and timing events of one balancing call, released on every exit path
-struct Scratch {
-    cudaStream_t s;
-    std::vector<void*> ptrs;
-    explicit Scratch(cudaStream_t st) : s(st) {}
-    cudaError_t alloc(void** p, size_t bytes) {
-        const cudaError_t e = cudaMallocAsync(p, bytes, s);
-        if (e == cudaSuccess) ptrs.push_back(*p);
-        return e;
-    }
-    ~Scratch() { for (void* p : ptrs) cudaFreeAsync(p, s); }
-};
+// timing events of one balancing call, released on every exit path
 struct EventPair {
     cudaEvent_t a = nullptr, b = nullptr;
     void create() { cudaEventCreate(&a); cudaEventCreate(&b); }
@@ -1057,17 +1143,55 @@ const StreamVariant kVariants[] = {
 // packed kernel: an item is one strip of 16 rows
 const StreamVariant kQ8 = {ice_q8_mma_kernel, 16, Q8_MINB};
 
+// Everything of hc_ice_dense_balance that depends only on the launch shape, kept between calls (per host thread and
+// device): the host tables (work-item descriptors, padded offsets) and their device copies, every scratch buffer, and
+// the instantiated graph of the iteration loop.  Each pointer in A is owned here, so the graph's kernel nodes are the
+// same for every call of the shape and a repeated call neither builds nor uploads anything.
+struct IceDenseCache {
+    // key
+    int packed = -1, nprob = 0, kseg = 0, cluster = 0, timed = 0, kd = 0, max_iters = 0;
+    StreamKernel fn = nullptr;
+    double tol = 0.0;
+    const void* mats = nullptr; const void* mat_off = nullptr;   // int32 kernel only: it streams the caller's tiles
+    std::vector<int32_t> n, ld;
+    // device memory of the shape (one allocation)
+    unsigned char* mem = nullptr;
+    IceDenseArgs A;
+    int32_t* state = nullptr;          // per-call state, reset from `pristine` at the start of every call
+    const int32_t* pristine = nullptr;
+    size_t state_ints = 0;
+    int64_t* ovf_ptr = nullptr; int64_t* qoff = nullptr; int64_t* strip = nullptr; int32_t* lo = nullptr; int32_t* hi = nullptr;
+    int32_t* abort_flag = nullptr;
+    int64_t nbins = 0, strips = 0;
+    int kt_max = 0, grid = 0;
+    // overflow cells (packed encoding): grow-only capacity, kept across shapes
+    int32_t* ovf = nullptr;
+    long long ovf_cap = 0;
+    // the iteration loop as one graph: first iteration, then a WHILE node over the same two kernels
+    cudaGraph_t graph = nullptr;
+    cudaGraphExec_t exec = nullptr;
+    cudaEvent_t ev[2] = {nullptr, nullptr};    // around the first stream launch (HC_ICE_TIME_KERNEL=1)
+    long long* mbox = nullptr;                 // pinned: [0] overflow cells, [1] iterations (int32) of the last call
+    void drop_graph() {
+        if (exec) cudaGraphExecDestroy(exec);
+        if (graph) cudaGraphDestroy(graph);
+        exec = nullptr; graph = nullptr;
+    }
+    void drop() {
+        drop_graph();
+        if (mem) cudaFree(mem);
+        mem = nullptr; packed = -1; n.clear(); ld.clear();
+    }
+};
+
 }  // namespace
 
 extern "C" int hc_ice_dense_marginals(const int32_t* mats, const int64_t* mat_off, const int32_t* mat_n,
                                       const int32_t* mat_ld, const int64_t* bin_off, int32_t nprob,
                                       int32_t ignore_diags, double* nnz_marg, double* marg, void* stream) {
     HC_REQUIRE(nprob > 0 && ignore_diags >= 0, "nprob>0, ignore_diags>=0");
-    int64_t total = 0;
-    HC_CUDA(hc_read_small(&total, bin_off + nprob, sizeof(int64_t), (cudaStream_t)stream));
-    if (total == 0) return HC_OK;
-    const int64_t blocks = (total * 32 + 255) / 256;
-    ice_dense_marginals_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+    // grid-stride over the bins (count read on the device): no wait for the binning that precedes this call
+    ice_dense_marginals_kernel<<<(unsigned)hc_num_sms() * 8, 256, 0, (cudaStream_t)stream>>>(
         mats, mat_off, mat_n, mat_ld, bin_off, nprob, ignore_diags, nnz_marg, marg);
     HC_LAUNCH_CHECK();
     return HC_OK;
@@ -1125,6 +1249,7 @@ extern "C" int hc_ice_filter_bins(const double* nnz_marg, double* marg, int64_t 
     return HC_OK;
 }
 
+
 extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off, const int32_t* mat_n,
                                     const int32_t* mat_ld, const int64_t* bin_off, int32_t nprob,
                                     const int32_t* h_mat_n, const hc_ice_params* P, double* bias,
@@ -1138,9 +1263,9 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
     }
     if (h_info) { h_info->launches = 0; h_info->loop_ms = 0.f; h_info->packed = 0; h_info->pack_ms = 0.f; h_info->overflow_cells = 0; h_info->stream_full_ms = 0.f; h_info->stream_full_launches = 0; }
     if (nbins == 0) return HC_OK;
-    // The iteration loop is replayed as a CUDA graph, which cannot be captured on the legacy default
-    // stream: run on a private stream ordered after the caller's stream (the call synchronises
-    // before returning, so the caller's later work is ordered after it).
+    // The iteration loop is a CUDA graph, which cannot be captured or launched on the legacy default stream: run on a
+    // private stream ordered after the caller's stream (the call synchronises before returning, so the caller's later
+    // work is ordered after it).
     static thread_local cudaStream_t private_stream[64] = {nullptr};
     int dev = 0;
     HC_CUDA(cudaGetDevice(&dev));
@@ -1184,104 +1309,56 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
     // padded internal vectors: problem p owns [pad_off[p], pad_off[p] + ld_p), 128-byte aligned, so the
     // kernel can read the bias of any 4-column group with two aligned 16-byte loads and never
     // needs a column bound check (matrix padding columns are zero, padded bias entries are zero)
+    // (the one wait of a call on the device: the leading dimensions exist only in device memory)
     std::vector<int32_t> h_ld(nprob);
     HC_CUDA(hc_read_small(h_ld.data(), mat_ld, sizeof(int32_t) * nprob, s));
-    std::vector<int64_t> h_pad(nprob + 1, 0);
     for (int p = 0; p < nprob; ++p) {
         if (h_ld[p] < h_mat_n[p] || (h_ld[p] & 127) != 0) {
             hc_set_error("hc_ice_dense_balance: ld must be >= n and a multiple of 128 elements (matrix %d: n=%d ld=%d)",
                          p, h_mat_n[p], h_ld[p]);
             return HC_ERR_ARG;
         }
-        h_pad[p + 1] = h_pad[p] + h_ld[p];
     }
-    const int64_t npad = h_pad[nprob];
-    int nseg_max = 1;
-    for (int p = 0; p < nprob; ++p) nseg_max = std::max(nseg_max, ((h_ld[p] >> 5) + kseg - 1) / kseg);
+    // update kernel: the 8-CTA cluster version needs every chromosome to fit 8 x 256 x 4 padded columns
+    bool cluster_update = packed;
+    for (int p = 0; p < nprob; ++p) cluster_update = cluster_update && h_ld[p] <= UPD_CLUSTER * 256 * 4;
+    // HC_ICE_TIME_KERNEL=1 (set by bench.py): the stream-kernel launch of the first iteration, in which every
+    // chromosome is active, is bracketed by a pair of events (event-record nodes in the graph), so that its duration
+    // can be read back separately from the update kernel and the launch gaps
+    const bool timed = h_info != nullptr && getenv("HC_ICE_TIME_KERNEL") != nullptr && atoi(getenv("HC_ICE_TIME_KERNEL")) != 0;
 
-    // ---- work items, largest chromosomes first ---------------------------------------------------
-    std::vector<int> order(nprob);
-    for (int p = 0; p < nprob; ++p) order[p] = p;
-    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return h_mat_n[a] > h_mat_n[b]; });
-    // packed kernel: the descriptors of every item (4 x int4 each, see ice_q8_mma_kernel) are built once; the items
-    // of chromosome p are the ids [desc_lo[p], desc_hi[p])
-    std::vector<int4> item_desc;
-    std::vector<int> desc_lo(nprob, 0), desc_hi(nprob, 0);
-    if (packed) {
-        auto lohi = [](int64_t v, int& a, int& b) { a = (int)(uint32_t)(v & 0xffffffffll); b = (int)(v >> 32); };
-        std::vector<int64_t> h_qoff(nprob, 0), h_binoff(nprob + 1, 0);
-        int64_t qb = 0;
+    static thread_local IceDenseCache caches[64];
+    IceDenseCache& C = caches[dev];
+    if (!C.mbox) HC_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&C.mbox), 2 * sizeof(long long), cudaHostAllocDefault));
+    if (timed)
+        for (auto& e : C.ev) if (e == nullptr) HC_CUDA(cudaEventCreate(&e));
+    const bool hit = C.mem != nullptr && C.packed == (int)packed && C.nprob == nprob && C.kseg == kseg && C.fn == V.fn &&
+                     C.cluster == (int)cluster_update && C.timed == (int)timed && C.kd == P->ignore_diags &&
+                     C.max_iters == P->max_iters && C.tol == P->tol && C.mats == (packed ? nullptr : (const void*)mats) &&
+                     C.mat_off == (packed ? nullptr : (const void*)mat_off) &&
+                     std::equal(h_mat_n, h_mat_n + nprob, C.n.begin(), C.n.end()) && C.ld == h_ld;
+    if (!hit) {
+        // ---- a new launch shape: host tables, device buffers ---------------------------------------
+        C.drop();
+        std::vector<int64_t> h_pad(nprob + 1, 0);
+        for (int p = 0; p < nprob; ++p) h_pad[p + 1] = h_pad[p] + h_ld[p];
+        const int64_t npad = h_pad[nprob];
+        int nseg_max = 1, kt_max = 0, nonempty = 0;
         for (int p = 0; p < nprob; ++p) {
-            h_qoff[p] = qb;
-            qb += (int64_t)((h_mat_n[p] + 15) / 16) * 16 * h_ld[p];
-            h_binoff[p + 1] = h_binoff[p] + h_mat_n[p];
+            nseg_max = std::max(nseg_max, ((h_ld[p] >> 5) + kseg - 1) / kseg);
+            kt_max = std::max(kt_max, h_ld[p] >> 5);
+            nonempty += h_mat_n[p] > 0;
         }
-        for (int p : order) {
-            const int n = h_mat_n[p], KT = h_ld[p] >> 5;
-            desc_lo[p] = (int)(item_desc.size() / 4);
-            for (int r0 = 0; r0 < n; r0 += V.rg)
-                for (int k0 = 0; k0 < KT; k0 += kseg) {
-                    int4 d0, d1, d2, d3;
-                    lohi(h_qoff[p] + ((int64_t)(r0 / 16) * KT + k0) * 512, d0.x, d0.y);
-                    lohi((int64_t)(k0 / kseg) * npad + h_pad[p] + r0, d0.z, d0.w);
-                    lohi(8 * h_pad[p] + (int64_t)k0 * 256, d1.x, d1.y);
-                    lohi(h_binoff[p] + r0, d1.z, d1.w);
-                    d2 = make_int4(p, (int)h_pad[p], r0, std::min(V.rg, n - r0));
-                    d3 = make_int4(std::min(kseg, KT - k0), k0 / kseg, KT, 0);
-                    item_desc.push_back(d0); item_desc.push_back(d1); item_desc.push_back(d2); item_desc.push_back(d3);
-                }
-            desc_hi[p] = (int)(item_desc.size() / 4);
-        }
-    }
-    // the live work list of the unconverged chromosomes: packed, their descriptor ids (item_prob); int32, row groups of
-    // ~item_kb KB, a multiple of RG rows each (chromosome, first row, rows)
-    std::vector<int32_t> h_done(nprob, 0);
-    std::vector<int32_t> item_prob, item_row0, item_nrows;
-    auto build_items = [&]() {
-        item_prob.clear(); item_row0.clear(); item_nrows.clear();
-        for (int p : order) {
-            const int n = h_mat_n[p];
-            if (n == 0 || h_done[p]) continue;
-            if (packed) {
-                for (int id = desc_lo[p]; id < desc_hi[p]; ++id) item_prob.push_back(id);
-                continue;
-            }
-            int rows = (int)((int64_t)item_kb * 1024 / ((int64_t)h_ld[p] * 4));
-            rows = std::max(V.rg, rows / V.rg * V.rg);
-            for (int r0 = 0; r0 < n; r0 += rows) {
-                item_prob.push_back(p); item_row0.push_back(r0); item_nrows.push_back(std::min(rows, n - r0));
-            }
-        }
-    };
-    build_items();
-    const size_t max_items = item_prob.size();
-
-    Scratch scratch(s);
-    double* d_vec = nullptr;     // [npad] bias | [npad] marg | [nprob+1] pad_off (as int64)
-    HC_CUDA(scratch.alloc((void**)&d_vec, (2 * (size_t)npad + nprob + 1) * sizeof(double)));
-    double* biasp = d_vec;
-    double* marg = d_vec + npad;
-    int64_t* d_pad = reinterpret_cast<int64_t*>(d_vec + 2 * npad);
-    HC_CUDA(cudaMemsetAsync(d_vec, 0, 2 * (size_t)npad * sizeof(double), s));
-    HC_CUDA(cudaMemcpyAsync(d_pad, h_pad.data(), (nprob + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-    ice_pad_bias_kernel<<<(unsigned)((nbins + 255) / 256), 256, 0, s>>>(bin_off, d_pad, nprob, bias, biasp);
-    HC_LAUNCH_CHECK();
-
-    // ---- packed encoding of the tiles (once per call) ------------------------------------------
-    uint8_t* d_q8 = nullptr;           // tiles | digits (8 B per padded column) behind them
-    int64_t* d_ovf_ptr = nullptr;      // [nbins+1] ptr | q_off[nprob] | strip_off[nprob+1] | lo[nbins] hi[nbins] exp[nprob] (int32)
-    int32_t* d_ovf = nullptr;          // col[novf] | val[novf]
-    uint8_t* d_digits = nullptr;
-    double* d_part = nullptr;          // [npad][nseg_max] partial row sums
-    int64_t* d_qoff = nullptr;
-    int32_t* d_exp = nullptr;
-    long long novf = 0;
-    EventPair evp;
-    cudaEvent_t& evp0 = evp.a;
-    cudaEvent_t& evp1 = evp.b;
-    if (packed) {
-        if (h_info) { evp.create(); cudaEventRecord(evp0, s); }
-        std::vector<int64_t> h_q(2 * (size_t)nprob + 1);     // q_off[nprob] | strip_off[nprob+1]
+        // work items, largest chromosomes first.  Packed: the descriptors of every item (4 x int4 each, see
+        // ice_q8_mma_kernel); int32: row groups of ~item_kb KB, a multiple of RG rows each (chromosome, first row, rows).
+        // The items of the chromosome at position i of `order` are [rng_lo[i], rng_hi[i]) of the full list; the live
+        // list (item_prob ...) is the full list less the converged chromosomes, rewritten on the device.
+        std::vector<int> order(nprob);
+        for (int p = 0; p < nprob; ++p) order[p] = p;
+        std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return h_mat_n[a] > h_mat_n[b]; });
+        std::vector<int4> item_desc;
+        std::vector<int32_t> full_prob, full_row0, full_nrows, rng(3 * (size_t)nprob + 3 * (size_t)nprob, 0);
+        std::vector<int64_t> h_q(2 * (size_t)nprob + 1, 0);     // q_off[nprob] | strip_off[nprob+1]
         int64_t qbytes = 0, strips = 0;
         for (int p = 0; p < nprob; ++p) {
             h_q[p] = qbytes;
@@ -1291,233 +1368,274 @@ extern "C" int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off,
             strips += sp;
         }
         h_q[2 * (size_t)nprob] = strips;
-        HC_CUDA(scratch.alloc((void**)&d_q8, (size_t)qbytes + 8 * (size_t)npad * (1 + (size_t)nseg_max) + 16));
-        d_digits = d_q8 + ((qbytes + 15) & ~15ll);
-        d_part = reinterpret_cast<double*>(d_digits + 8 * (size_t)npad);
+        auto lohi = [](int64_t v, int& a, int& b) { a = (int)(uint32_t)(v & 0xffffffffll); b = (int)(v >> 32); };
+        int64_t binoff = 0;
+        std::vector<int64_t> h_binoff(nprob + 1, 0);
+        for (int p = 0; p < nprob; ++p) { h_binoff[p] = binoff; binoff += h_mat_n[p]; }
+        for (int i = 0; i < nprob; ++i) {
+            const int p = order[i], n = h_mat_n[p];
+            rng[i] = p;
+            rng[nprob + i] = (int)full_prob.size();
+            if (packed) {
+                const int KT = h_ld[p] >> 5;
+                for (int r0 = 0; r0 < n; r0 += V.rg)
+                    for (int k0 = 0; k0 < KT; k0 += kseg) {
+                        int4 d0, d1, d2, d3;
+                        lohi(h_q[p] + ((int64_t)(r0 / 16) * KT + k0) * 512, d0.x, d0.y);
+                        lohi((int64_t)(k0 / kseg) * npad + h_pad[p] + r0, d0.z, d0.w);
+                        lohi(8 * h_pad[p] + (int64_t)k0 * 256, d1.x, d1.y);
+                        lohi(h_binoff[p] + r0, d1.z, d1.w);
+                        d2 = make_int4(p, (int)h_pad[p], r0, std::min(V.rg, n - r0));
+                        d3 = make_int4(std::min(kseg, KT - k0), k0 / kseg, KT, 0);
+                        item_desc.push_back(d0); item_desc.push_back(d1); item_desc.push_back(d2); item_desc.push_back(d3);
+                        full_prob.push_back((int)full_prob.size()); full_row0.push_back(0); full_nrows.push_back(0);
+                    }
+            } else if (n > 0) {
+                int rows = (int)((int64_t)item_kb * 1024 / ((int64_t)h_ld[p] * 4));
+                rows = std::max(V.rg, rows / V.rg * V.rg);
+                for (int r0 = 0; r0 < n; r0 += rows) {
+                    full_prob.push_back(p); full_row0.push_back(r0); full_nrows.push_back(std::min(rows, n - r0));
+                }
+            }
+            rng[2 * nprob + i] = (int)full_prob.size();
+        }
+        for (int p = 0; p < nprob; ++p) { rng[4 * nprob + p] = h_mat_n[p]; rng[5 * nprob + p] = h_ld[p]; }   // mat_n | mat_ld
+        const size_t M = full_prob.size();
+        const int grid = hc_num_sms() * V.minb;    // persistent: every resident slot filled exactly once
+        const unsigned int queue_start = (unsigned)grid * 8u;
+        // per-call state: live items (3 x M) | done[nprob] | n_done | queue | iter | nitems | upd_cnt | changed | abort
+        const size_t st = 3 * M + (size_t)nprob;
+        const size_t S = st + 7;
+        std::vector<int32_t> h_state(S, 0);
+        std::copy(full_prob.begin(), full_prob.end(), h_state.begin());
+        std::copy(full_row0.begin(), full_row0.end(), h_state.begin() + M);
+        std::copy(full_nrows.begin(), full_nrows.end(), h_state.begin() + 2 * M);
+        h_state[st + 1] = (int32_t)queue_start;
+        h_state[st + 3] = (int32_t)M;
+        std::vector<hc_ice_result> h_res(nprob);      // empty problems never get work: their result stays this one
+        for (int p = 0; p < nprob; ++p) { h_res[p].scale = NAN; h_res[p].var = 0.0; h_res[p].iters = 0; h_res[p].converged = 1; }
+
+        size_t off = 0;
+        auto take = [&](size_t bytes) { const size_t o = off; off = (off + bytes + 255) & ~(size_t)255; return o; };
         const size_t ptr_bytes = ((size_t)nbins + 1 + 2 * (size_t)nprob + 1 + (size_t)((nbins + 1023) / 1024) + 1) * sizeof(int64_t);
-        HC_CUDA(scratch.alloc((void**)&d_ovf_ptr, ptr_bytes + (2 * (size_t)nbins + nprob) * sizeof(int32_t)));
-        d_qoff = d_ovf_ptr + nbins + 1;
-        int64_t* d_strip = d_qoff + nprob;
-        int32_t* d_lo = reinterpret_cast<int32_t*>(reinterpret_cast<unsigned char*>(d_ovf_ptr) + ptr_bytes);
-        int32_t* d_hi = d_lo + nbins;
-        d_exp = d_hi + nbins;
-        HC_CUDA(cudaMemcpyAsync(d_qoff, h_q.data(), h_q.size() * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-        HC_CUDA(cudaMemsetAsync(d_ovf_ptr, 0, ((size_t)nbins + 1) * sizeof(int64_t), s));
-        HC_CUDA(cudaMemsetAsync(d_lo, 0x7f, (size_t)nbins * sizeof(int32_t), s));
-        HC_CUDA(cudaMemsetAsync(d_hi, 0xff, (size_t)nbins * sizeof(int32_t), s));
-        HC_CUDA(cudaStreamSynchronize(s));      // h_q goes out of scope
-        int kt_max = 0;
-        for (int p = 0; p < nprob; ++p) kt_max = std::max(kt_max, h_ld[p] >> 5);
-        ice_pack_tiles_kernel<<<dim3((unsigned)((strips * 32 + 255) / 256), (unsigned)((kt_max + 7) / 8)), 256, 0, s>>>(
-            mats, mat_off, mat_n, mat_ld, d_qoff, d_strip, bin_off, nprob, P->ignore_diags, d_q8,
-            reinterpret_cast<unsigned long long*>(d_ovf_ptr), d_lo, d_hi);
+        const size_t o_vec = take((2 * (size_t)npad + nprob + 1) * sizeof(double));     // bias | marg | pad_off (int64)
+        const size_t o_q8 = take(packed ? (size_t)qbytes + 8 * (size_t)npad * (1 + (size_t)nseg_max) + 16 : 0);   // tiles | digits | part
+        // ptr[nbins+1] | q_off[nprob] | strip_off[nprob+1] | bsum | lo[nbins] hi[nbins] exp[nprob] (int32)
+        const size_t o_ptr = take(packed ? ptr_bytes + (2 * (size_t)nbins + nprob) * sizeof(int32_t) : 0);
+        const size_t o_state = take(S * sizeof(int32_t));
+        const size_t o_pristine = take(S * sizeof(int32_t));
+        const size_t o_tab = take(rng.size() * sizeof(int32_t));
+        const size_t o_desc = take(item_desc.size() * sizeof(int4));
+        const size_t o_res = take((size_t)nprob * sizeof(hc_ice_result));
+        HC_CUDA(cudaMalloc(reinterpret_cast<void**>(&C.mem), off));
+        unsigned char* m = C.mem;
+        IceDenseArgs A = {};
+        A.bias = reinterpret_cast<double*>(m + o_vec);
+        A.marg = A.bias + npad;
+        int64_t* d_pad = reinterpret_cast<int64_t*>(A.bias + 2 * npad);
+        A.pad_off = d_pad;
+        C.state = reinterpret_cast<int32_t*>(m + o_state);
+        C.pristine = reinterpret_cast<const int32_t*>(m + o_pristine);
+        C.state_ints = S;
+        int32_t* tab = reinterpret_cast<int32_t*>(m + o_tab);
+        A.mats = packed ? nullptr : mats; A.mat_off = packed ? nullptr : mat_off;
+        A.mat_n = tab + 4 * nprob; A.mat_ld = tab + 5 * nprob;
+        A.item_prob = C.state; A.item_row0 = C.state + M; A.item_nrows = C.state + 2 * M;
+        A.done = C.state + 3 * M;
+        A.n_done = C.state + st;
+        A.queue = reinterpret_cast<unsigned int*>(C.state + st + 1);
+        A.iter = C.state + st + 2;
+        A.nitems = reinterpret_cast<const unsigned int*>(C.state + st + 3);
+        A.upd_cnt = reinterpret_cast<unsigned int*>(C.state + st + 4);
+        A.changed = C.state + st + 5;
+        C.abort_flag = C.state + st + 6;
+        A.results = reinterpret_cast<hc_ice_result*>(m + o_res);
+        A.tol = P->tol; A.kd = P->ignore_diags; A.max_iters = P->max_iters; A.nprob = nprob; A.queue_start = queue_start;
+        A.packed = packed ? 1 : 0; A.kseg = kseg; A.nseg_max = nseg_max; A.npad = npad;
+        A.nonempty = nonempty;
+        A.rng = tab; A.rng_off = tab + 3 * nprob;
+        A.full_row0 = C.pristine + M; A.full_nrows = C.pristine + 2 * M;
+        A.loop_end = 1;
+        if (packed) {
+            uint8_t* q8 = m + o_q8;
+            A.q8 = q8;
+            A.digits = q8 + ((qbytes + 15) & ~15ll);
+            A.part = reinterpret_cast<double*>(A.digits + 8 * (size_t)npad);
+            C.ovf_ptr = reinterpret_cast<int64_t*>(m + o_ptr);
+            C.qoff = C.ovf_ptr + nbins + 1;
+            C.strip = C.qoff + nprob;
+            C.lo = reinterpret_cast<int32_t*>(m + o_ptr + ptr_bytes);
+            C.hi = C.lo + nbins;
+            A.dig_exp = C.hi + nbins;
+            A.q_off = C.qoff;
+            A.ovf_ptr = C.ovf_ptr;
+            A.desc = reinterpret_cast<const int4*>(m + o_desc);
+            HC_CUDA(cudaMemcpyAsync(C.qoff, h_q.data(), h_q.size() * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+            HC_CUDA(cudaMemcpyAsync(m + o_desc, item_desc.data(), item_desc.size() * sizeof(int4), cudaMemcpyHostToDevice, s));
+        }
+        HC_CUDA(cudaMemcpyAsync(d_pad, h_pad.data(), (nprob + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+        HC_CUDA(cudaMemcpyAsync(m + o_pristine, h_state.data(), S * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        HC_CUDA(cudaMemcpyAsync(tab, rng.data(), rng.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        HC_CUDA(cudaMemcpyAsync(A.results, h_res.data(), h_res.size() * sizeof(hc_ice_result), cudaMemcpyHostToDevice, s));
+        HC_CUDA(cudaStreamSynchronize(s));      // the host tables go out of scope
+        C.A = A;
+        C.packed = packed; C.nprob = nprob; C.kseg = kseg; C.fn = V.fn; C.cluster = cluster_update; C.timed = timed;
+        C.kd = P->ignore_diags; C.max_iters = P->max_iters; C.tol = P->tol;
+        C.mats = A.mats; C.mat_off = A.mat_off;
+        C.n.assign(h_mat_n, h_mat_n + nprob); C.ld = h_ld;
+        C.nbins = nbins; C.strips = strips; C.kt_max = kt_max; C.grid = grid;
+    }
+    IceDenseArgs& A = C.A;
+    if (packed && C.ovf == nullptr) {
+        C.ovf_cap = std::max(4 * (long long)nbins, 1024ll);
+        HC_CUDA(cudaMalloc(reinterpret_cast<void**>(&C.ovf), 2 * (size_t)C.ovf_cap * sizeof(int32_t)));
+    }
+    A.ovf_col = C.ovf; A.ovf_val = C.ovf ? C.ovf + C.ovf_cap : nullptr;
+    // the bias vector (its byte planes for the packed kernel) is the only data that should live in L1
+    cudaFuncSetAttribute(V.fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
+    auto launch_update = [&]() {
+        if (C.cluster) ice_q8_update_cluster_kernel<<<nprob * UPD_CLUSTER, 256, 0, s>>>(A);
+        else ice_dense_update_kernel<<<nprob, 1024, 0, s>>>(A);
+    };
+    // The loop as one graph: the first iteration (all chromosomes active; its stream launch bracketed by the timing
+    // events), then a WHILE node whose body is ICE_BODY_ITERS iterations.  The condition is set by the last CTA of the
+    // update launch that ends the first iteration and each body (ice_iteration_end, which also compacts the work list),
+    // so the loop needs no host poll; iterations past the last convergence in a body find every chromosome done (about
+    // 5 us each).  Measured on B200 (C2, 86 iterations): a body of one iteration costs ~2 us more per iteration than 4
+    // or 8 (loop 5.61 ms against 5.47 / 5.44 ms).
+    constexpr int ICE_BODY_ITERS = 4;
+    auto build_graph = [&]() -> cudaError_t {
+        cudaGraph_t g = nullptr;
+        cudaError_t e = cudaGraphCreate(&g, 0);
+        cudaGraphConditionalHandle h = 0;
+        if (e == cudaSuccess) e = cudaGraphConditionalHandleCreate(&h, g, 1, cudaGraphCondAssignDefault);
+        IceDenseArgs GA = A, GB = A;          // GB: the update launches inside a body that do not end it
+        GA.cond = GB.cond = h; GA.has_cond = GB.has_cond = 1; GA.loop_end = 1; GB.loop_end = 0;
+        void* args[1] = {&GA};
+        void* args_mid[1] = {&GB};
+        cudaKernelNodeParams ks = {}, ku = {};
+        ks.func = reinterpret_cast<void*>(C.fn); ks.gridDim = dim3(C.grid); ks.blockDim = dim3(256); ks.kernelParams = args;
+        ku.func = C.cluster ? reinterpret_cast<void*>(ice_q8_update_cluster_kernel) : reinterpret_cast<void*>(ice_dense_update_kernel);
+        ku.gridDim = dim3(C.cluster ? nprob * UPD_CLUSTER : nprob); ku.blockDim = dim3(C.cluster ? 256 : 1024); ku.kernelParams = args;
+        cudaKernelNodeParams ku_mid = ku;
+        ku_mid.kernelParams = args_mid;
+        cudaGraphNode_t prev = nullptr, node = nullptr;
+        if (e == cudaSuccess && C.timed) { e = cudaGraphAddEventRecordNode(&node, g, nullptr, 0, C.ev[0]); prev = node; }
+        if (e == cudaSuccess) { e = cudaGraphAddKernelNode(&node, g, prev ? &prev : nullptr, prev ? 1 : 0, &ks); prev = node; }
+        if (e == cudaSuccess && C.timed) { e = cudaGraphAddEventRecordNode(&node, g, &prev, 1, C.ev[1]); prev = node; }
+        if (e == cudaSuccess) { e = cudaGraphAddKernelNode(&node, g, &prev, 1, &ku); prev = node; }
+        cudaGraphNodeParams cp = {};
+        cp.type = cudaGraphNodeTypeConditional;
+        cp.conditional.handle = h; cp.conditional.type = cudaGraphCondTypeWhile; cp.conditional.size = 1;
+        if (e == cudaSuccess) e = cudaGraphAddNode(&node, g, &prev, 1, &cp);
+        if (e == cudaSuccess) {
+            cudaGraph_t body = cp.conditional.phGraph_out[0];
+            cudaGraphNode_t bs = nullptr, bp = nullptr;
+            for (int u = 0; u < ICE_BODY_ITERS && e == cudaSuccess; ++u) {
+                e = cudaGraphAddKernelNode(&bs, body, bp ? &bp : nullptr, bp ? 1 : 0, &ks);
+                if (e == cudaSuccess) e = cudaGraphAddKernelNode(&bp, body, &bs, 1, u + 1 < ICE_BODY_ITERS ? &ku_mid : &ku);
+            }
+        }
+        if (e == cudaSuccess) e = cudaGraphInstantiate(&C.exec, g, 0);
+        if (e != cudaSuccess) { if (g) cudaGraphDestroy(g); C.exec = nullptr; (void)cudaGetLastError(); return e; }
+        C.graph = g;
+        return cudaSuccess;
+    };
+
+    float loop_ms = 0.f, pack_ms = 0.f, stream_ms = 0.f;
+    int iters = 0;
+    long long novf = 0;
+    for (;;) {      // twice only when the overflow cells outgrow their arrays
+        HC_CUDA(cudaMemcpyAsync(C.state, C.pristine, C.state_ints * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
+        HC_CUDA(cudaMemsetAsync(A.bias, 0, 2 * (size_t)A.npad * sizeof(double), s));
+        ice_pad_bias_kernel<<<(unsigned)((nbins + 255) / 256), 256, 0, s>>>(bin_off, A.pad_off, nprob, bias, A.bias);
         HC_LAUNCH_CHECK();
-        {
+
+        // ---- packed encoding of the tiles (once per call) ------------------------------------------
+        EventPair evp;
+        if (packed) {
+            if (h_info) { evp.create(); cudaEventRecord(evp.a, s); }
+            HC_CUDA(cudaMemsetAsync(C.ovf_ptr, 0, ((size_t)nbins + 1) * sizeof(int64_t), s));
+            HC_CUDA(cudaMemsetAsync(C.lo, 0x7f, (size_t)nbins * sizeof(int32_t), s));
+            HC_CUDA(cudaMemsetAsync(C.hi, 0xff, (size_t)nbins * sizeof(int32_t), s));
+            ice_pack_tiles_kernel<<<dim3((unsigned)((C.strips * 32 + 255) / 256), (unsigned)((C.kt_max + 7) / 8)), 256, 0, s>>>(
+                mats, mat_off, mat_n, mat_ld, C.qoff, C.strip, bin_off, nprob, P->ignore_diags, const_cast<uint8_t*>(A.q8),
+                reinterpret_cast<unsigned long long*>(C.ovf_ptr), C.lo, C.hi);
+            HC_LAUNCH_CHECK();
             const int nb = (int)((nbins + 1023) / 1024);
-            int64_t* d_bsum = d_strip + nprob + 1;       // nb + 1 entries behind the strip table
-            ice_ovf_blocksum_kernel<<<nb, 256, 0, s>>>(d_ovf_ptr, nbins, d_bsum);
+            int64_t* d_bsum = C.strip + nprob + 1;       // nb + 1 entries behind the strip table
+            ice_ovf_blocksum_kernel<<<nb, 256, 0, s>>>(C.ovf_ptr, nbins, d_bsum);
             HC_LAUNCH_CHECK();
             ice_ovf_scan_blocks_kernel<<<1, 1024, 0, s>>>(d_bsum, nb);
             HC_LAUNCH_CHECK();
-            ice_ovf_scan_kernel<<<nb, 256, 0, s>>>(d_ovf_ptr, nbins, d_bsum, nb);
+            ice_ovf_scan_kernel<<<nb, 256, 0, s>>>(C.ovf_ptr, nbins, d_bsum, nb);
             HC_LAUNCH_CHECK();
-        }
-        HC_CUDA(hc_read_small(&novf, d_ovf_ptr + nbins, sizeof(long long), s));
-        HC_CUDA(scratch.alloc((void**)&d_ovf, 2 * (size_t)std::max(novf, 1ll) * sizeof(int32_t)));
-        if (novf > 0) {
             ice_pack_ovf_kernel<<<(unsigned)((nbins * 32 + 255) / 256), 256, 0, s>>>(
-                mats, mat_off, mat_n, mat_ld, bin_off, nprob, P->ignore_diags, d_ovf_ptr, d_lo, d_hi, d_ovf, d_ovf + novf);
+                mats, mat_off, mat_n, mat_ld, bin_off, nprob, P->ignore_diags, C.ovf_ptr, C.lo, C.hi,
+                const_cast<int32_t*>(A.ovf_col), const_cast<int32_t*>(A.ovf_val), C.ovf_cap, A, C.abort_flag);
             HC_LAUNCH_CHECK();
+            ice_digits_kernel<<<nprob, 1024, 0, s>>>(A);      // byte planes of the initial bias
+            HC_LAUNCH_CHECK();
+            if (evp.a) cudaEventRecord(evp.b, s);
         }
-    }
-    int32_t* d_tab = nullptr;    // 3 item tables | done[nprob] | n_done | queue | iter | nitems | pad to 16 B | item descriptors (packed)
-    const size_t desc_at = (3 * max_items + (size_t)nprob + 4 + 3) & ~(size_t)3;
-    const size_t tab_ints = desc_at + (packed ? 16 * max_items : 0);
-    HC_CUDA(scratch.alloc((void**)&d_tab, tab_ints * sizeof(int32_t)));
-    auto upload_items = [&]() -> cudaError_t {
-        const size_t n = item_prob.size();
-        const int32_t n32 = (int32_t)n;
-        cudaError_t e = cudaMemcpyAsync(d_tab + 3 * max_items + nprob + 3, &n32, sizeof(int32_t), cudaMemcpyHostToDevice, s);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d_tab, item_prob.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, s);
-        // the packed kernel reads only the id list; its descriptors are uploaded once, below
-        if (e == cudaSuccess && !packed) e = cudaMemcpyAsync(d_tab + max_items, item_row0.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, s);
-        if (e == cudaSuccess && !packed) e = cudaMemcpyAsync(d_tab + 2 * max_items, item_nrows.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);   // the host vectors may be rebuilt afterwards
-        return e;
-    };
-    HC_CUDA(cudaMemsetAsync(d_tab + 3 * max_items, 0, ((size_t)nprob + 3) * sizeof(int32_t), s));
-    if (packed) HC_CUDA(cudaMemcpyAsync(d_tab + desc_at, item_desc.data(), item_desc.size() * sizeof(int4), cudaMemcpyHostToDevice, s));
-    HC_CUDA(upload_items());
-    const int grid = hc_num_sms() * V.minb;    // persistent: every resident slot filled exactly once
-    const unsigned int queue_start = (unsigned)grid * 8u;
-    HC_CUDA(cudaMemcpyAsync(d_tab + 3 * max_items + nprob + 1, &queue_start, sizeof(unsigned int), cudaMemcpyHostToDevice, s));
 
-    IceDenseArgs A;
-    A.mats = mats; A.mat_off = mat_off; A.mat_n = mat_n; A.mat_ld = mat_ld; A.pad_off = d_pad;
-    A.item_prob = d_tab; A.item_row0 = d_tab + max_items; A.item_nrows = d_tab + 2 * max_items;
-    A.done = d_tab + 3 * max_items;
-    A.n_done = A.done + nprob;
-    A.queue = reinterpret_cast<unsigned int*>(A.n_done + 1);
-    A.iter = A.n_done + 2;
-    A.nitems = reinterpret_cast<const unsigned int*>(A.n_done + 3);
-    A.bias = biasp; A.marg = marg; A.results = results;
-    A.tol = P->tol; A.kd = P->ignore_diags; A.max_iters = P->max_iters; A.nprob = nprob; A.queue_start = queue_start;
-    A.q8 = d_q8; A.q_off = d_qoff; A.digits = d_digits; A.dig_exp = d_exp; A.packed = packed ? 1 : 0;
-    A.desc = reinterpret_cast<const int4*>(d_tab + desc_at); A.kseg = kseg; A.part = d_part; A.nseg_max = nseg_max; A.npad = npad;
-    A.bin_off = bin_off; A.ovf_ptr = d_ovf_ptr; A.ovf_col = d_ovf; A.ovf_val = d_ovf ? d_ovf + novf : nullptr;
-    if (packed) {
-        ice_digits_kernel<<<nprob, 1024, 0, s>>>(A);      // byte planes of the initial bias
-        HC_LAUNCH_CHECK();
-        if (evp0) cudaEventRecord(evp1, s);
-    }
-
-    int nonempty = 0;
-    for (int p = 0; p < nprob; ++p) nonempty += h_mat_n[p] > 0;
-    if (nonempty != nprob) {   // empty problems never get work: give them a defined result
-        std::vector<hc_ice_result> h_res(nprob);
-        for (int p = 0; p < nprob; ++p) { h_res[p].scale = NAN; h_res[p].var = 0.0; h_res[p].iters = 0; h_res[p].converged = 1; }
-        HC_CUDA(cudaMemcpyAsync(results, h_res.data(), sizeof(hc_ice_result) * nprob, cudaMemcpyHostToDevice, s));
-        HC_CUDA(cudaStreamSynchronize(s));
-    }
-    // the bias vector (its byte planes for the packed kernel) is the only data that should live in L1
-    const size_t smem = 0;
-    cudaFuncSetAttribute(V.fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1);
-    // update kernel: the 8-CTA cluster version needs every chromosome to fit 8 x 256 x 4 padded columns
-    bool cluster_update = packed;
-    for (int p = 0; p < nprob; ++p) cluster_update = cluster_update && h_ld[p] <= UPD_CLUSTER * 256 * 4;
-    auto launch_update = [&]() {
-        if (cluster_update) ice_q8_update_cluster_kernel<<<nprob * UPD_CLUSTER, 256, 0, s>>>(A);
-        else ice_dense_update_kernel<<<nprob, 1024, 0, s>>>(A);
-    };
-    const int poll = P->poll_every > 0 ? P->poll_every : 8;
-    int launches = 0, h_ndone = 0, seen_done = 0;
-    int rc = HC_OK;
-    // `poll` iterations (stream + update kernel each) captured once and replayed: the iteration index,
-    // the work-list length and every convergence decision live in device memory, so the graph is static
-    // (plain launches only when capture or instantiation fails).
-    cudaGraphExec_t gexec = nullptr;
-    // The captured graph is kept between calls (per host thread): the next call with the same launch shape only
-    // rewrites the kernel parameters of its nodes (cudaGraphExecKernelNodeSetParams) instead of capturing and
-    // instantiating again -- ~0.4 ms of host time per call on C2.
-    // HC_ICE_TIME_KERNEL=1 (set by bench.py): the first stream-kernel launch of every graph replay is bracketed by a pair
-    // of events, so that its duration can be read back separately from the update kernel and the launch gaps (external
-    // event-record nodes inside the graph; bracketing all 8 launches of a replay cost ~11 us per iteration)
-    struct GraphCache {
-        cudaGraphExec_t exec = nullptr;
-        cudaGraph_t graph = nullptr;
-        std::vector<cudaGraphNode_t> knodes;
-        StreamKernel fn = nullptr;     // the packed kernel or one of the int32 kernels
-        int grid = 0, poll = 0, nprob = 0, cluster = 0, timed = 0, dev = -1;
-        cudaEvent_t ev[2] = {nullptr, nullptr};
-        void drop() {
-            if (exec) cudaGraphExecDestroy(exec);
-            if (graph) cudaGraphDestroy(graph);
-            exec = nullptr; graph = nullptr; knodes.clear();
-        }
-    };
-    static thread_local GraphCache gc;
-    const bool timed = h_info != nullptr && getenv("HC_ICE_TIME_KERNEL") != nullptr && atoi(getenv("HC_ICE_TIME_KERNEL")) != 0;
-    struct { std::vector<cudaEvent_t> ev; } sev;
-    if (timed) {
-        for (auto& e : gc.ev) if (e == nullptr && cudaEventCreate(&e) != cudaSuccess) { e = nullptr; (void)cudaGetLastError(); }
-        if (gc.ev[0] && gc.ev[1]) sev.ev.assign(gc.ev, gc.ev + 2);
-    }
-    double stream_ms_sum = 0.0;
-    int stream_ms_n = 0;
-    {
-        const bool hit = gc.exec != nullptr && gc.fn == V.fn && gc.grid == grid && gc.poll == poll && gc.nprob == nprob &&
-                         gc.cluster == (int)cluster_update && gc.timed == (int)!sev.ev.empty() && gc.dev == dev;
+        if (!C.exec && build_graph() != cudaSuccess) C.exec = nullptr;   // plain launches below
+        EventPair evl;                              // device time of the iteration loop, for the roofline
+        if (h_info) { evl.create(); cudaEventRecord(evl.a, s); }
         cudaError_t e = cudaSuccess;
-        if (hit) {
-            for (cudaGraphNode_t node : gc.knodes) {
-                cudaKernelNodeParams kp;
-                e = cudaGraphKernelNodeGetParams(node, &kp);
-                void* args[1] = {&A};
-                kp.kernelParams = args;
-                if (e == cudaSuccess) e = cudaGraphExecKernelNodeSetParams(gc.exec, node, &kp);
-                if (e != cudaSuccess) break;
-            }
-            if (e != cudaSuccess) { (void)cudaGetLastError(); gc.drop(); }
-        } else gc.drop();               // another launch shape: capture again
-        if (gc.exec == nullptr) {
-            e = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal);
-            if (e == cudaSuccess) {
+        if (C.exec) e = cudaGraphLaunch(C.exec, s);
+        else {
+            // without the graph: launch pairs, the host polls the done counter every `poll` iterations
+            const int poll = P->poll_every > 0 ? P->poll_every : 8;
+            for (int k0 = 0; k0 < P->max_iters && e == cudaSuccess; k0 += poll) {
                 for (int i = 0; i < poll; ++i) {
-                    if (i == 0 && !sev.ev.empty()) cudaEventRecordWithFlags(sev.ev[0], s, cudaEventRecordExternal);
-                    V.fn<<<grid, 256, smem, s>>>(A);
-                    if (i == 0 && !sev.ev.empty()) cudaEventRecordWithFlags(sev.ev[1], s, cudaEventRecordExternal);
+                    if (k0 + i == 0 && C.timed) cudaEventRecord(C.ev[0], s);
+                    C.fn<<<C.grid, 256, 0, s>>>(A);
+                    if (k0 + i == 0 && C.timed) cudaEventRecord(C.ev[1], s);
                     launch_update();
                 }
-                e = cudaStreamEndCapture(s, &gc.graph);
+                int32_t nd = 0;
+                e = hc_read_small(&nd, A.n_done, sizeof(int32_t), s);   // not a memcpy: see hc_read_small
+                if (e == cudaSuccess && nd >= A.nonempty) break;
             }
-            if (e == cudaSuccess) e = cudaGraphInstantiate(&gc.exec, gc.graph, 0);
-            if (e == cudaSuccess) {
-                size_t nn = 0;
-                e = cudaGraphGetNodes(gc.graph, nullptr, &nn);
-                std::vector<cudaGraphNode_t> nodes(nn);
-                if (e == cudaSuccess && nn) e = cudaGraphGetNodes(gc.graph, nodes.data(), &nn);
-                for (size_t k = 0; e == cudaSuccess && k < nn; ++k) {
-                    cudaGraphNodeType t;
-                    e = cudaGraphNodeGetType(nodes[k], &t);
-                    if (e == cudaSuccess && t == cudaGraphNodeTypeKernel) gc.knodes.push_back(nodes[k]);
-                }
-            }
-            if (e != cudaSuccess) { gc.drop(); (void)cudaGetLastError(); }   // plain launches below
-            else { gc.fn = V.fn; gc.grid = grid; gc.poll = poll; gc.nprob = nprob; gc.cluster = (int)cluster_update;
-                   gc.timed = (int)!sev.ev.empty(); gc.dev = dev; }
         }
-        gexec = gc.exec;
+        if (evl.a) cudaEventRecord(evl.b, s);
+        if (e == cudaSuccess) {
+            ice_finalize_kernel<<<(unsigned)((nbins + 255) / 256), 256, 0, s>>>(bin_off, A.pad_off, nprob, A.results,
+                                                                               P->rescale_marginals, A.bias, bias, C.abort_flag);
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) e = cudaMemcpyAsync(results, A.results, (size_t)nprob * sizeof(hc_ice_result), cudaMemcpyDeviceToDevice, s);
+        if (e == cudaSuccess && packed) e = cudaMemcpyAsync(C.mbox, C.ovf_ptr + nbins, sizeof(long long), cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(C.mbox + 1, A.iter, sizeof(int32_t), cudaMemcpyDeviceToHost, s);
+        const cudaError_t es = cudaStreamSynchronize(s);
+        if (e == cudaSuccess) e = es;
+        if (e != cudaSuccess) { hc_set_error("hc_ice_dense_balance: %s", cudaGetErrorString(e)); return HC_ERR_CUDA; }
+        iters = *reinterpret_cast<const int32_t*>(C.mbox + 1);
+        novf = packed ? C.mbox[0] : 0;
+        hc_count_launch(2 * iters + 1);
+        if (h_info) {
+            cudaEventElapsedTime(&loop_ms, evl.a, evl.b);
+            if (evp.a) cudaEventElapsedTime(&pack_ms, evp.a, evp.b);
+            if (C.timed && cudaEventElapsedTime(&stream_ms, C.ev[0], C.ev[1]) != cudaSuccess) { stream_ms = 0.f; (void)cudaGetLastError(); }
+        }
+        if (novf <= C.ovf_cap) break;
+        // the overflow arrays were too small: nothing was streamed and the caller's bias is untouched; grow, run again
+        cudaFree(C.ovf);
+        C.ovf = nullptr;
+        C.ovf_cap = novf + novf / 4;
+        HC_CUDA(cudaMalloc(reinterpret_cast<void**>(&C.ovf), 2 * (size_t)C.ovf_cap * sizeof(int32_t)));
+        A.ovf_col = C.ovf; A.ovf_val = C.ovf + C.ovf_cap;
+        C.drop_graph();     // its kernel nodes hold the old pointers
     }
-    EventPair evl;                              // device time of the iteration loop, for the roofline
-    cudaEvent_t& ev0 = evl.a;
-    cudaEvent_t& ev1 = evl.b;
-    if (h_info) { evl.create(); cudaEventRecord(ev0, s); }
-    for (int k0 = 0; k0 < P->max_iters; k0 += poll) {
-        cudaError_t e = cudaSuccess;
-        if (gexec) e = cudaGraphLaunch(gexec, s);
-        else for (int i = 0; i < poll; ++i) {
-            if (i == 0 && !sev.ev.empty()) cudaEventRecord(sev.ev[0], s);
-            V.fn<<<grid, 256, smem, s>>>(A);
-            if (i == 0 && !sev.ev.empty()) cudaEventRecord(sev.ev[1], s);
-            launch_update();
-        }
-        hc_count_launch(2 * poll);
-        launches += 2 * poll;
-        if (e == cudaSuccess) e = hc_read_small(&h_ndone, A.n_done, sizeof(int32_t), s);   // not a memcpy: see hc_read_small
-        if (e == cudaSuccess && h_ndone == 0 && !sev.ev.empty()) {
-            // no problem has finished yet: the bracketed launch streamed every matrix of the batch
-            float ms = 0.f;
-            if (cudaEventElapsedTime(&ms, sev.ev[0], sev.ev[1]) == cudaSuccess) { stream_ms_sum += ms; ++stream_ms_n; }
-            else (void)cudaGetLastError();
-        }
-        if (e == cudaSuccess && h_ndone >= nonempty) break;
-        if (e == cudaSuccess && h_ndone != seen_done) {
-            // drop the converged chromosomes from the work list (their items would only be skipped)
-            seen_done = h_ndone;
-            e = hc_read_small(h_done.data(), A.done, sizeof(int32_t) * nprob, s);
-            if (e == cudaSuccess) { build_items(); e = upload_items(); }
-        }
-        if (e != cudaSuccess) { hc_set_error("hc_ice_dense_balance: %s", cudaGetErrorString(e)); rc = HC_ERR_CUDA; break; }
-    }
-    if (h_info && ev0) cudaEventRecord(ev1, s);
-    if (rc == HC_OK) {
-        const int64_t blocks = (nbins + 255) / 256;
-        ice_finalize_kernel<<<(unsigned)blocks, 256, 0, s>>>(bin_off, d_pad, nprob, results, P->rescale_marginals, biasp, bias);
-        hc_count_launch();
-        ++launches;
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) { hc_set_error("hc_ice_dense_balance: %s", cudaGetErrorString(e)); rc = HC_ERR_CUDA; }
-    }
-    cudaError_t e = cudaStreamSynchronize(s);
-    if (rc == HC_OK && e != cudaSuccess) { hc_set_error("hc_ice_dense_balance: %s", cudaGetErrorString(e)); rc = HC_ERR_CUDA; }
     if (h_info) {
-        h_info->launches = launches;
-        if (ev0 && e == cudaSuccess) cudaEventElapsedTime(&h_info->loop_ms, ev0, ev1);
+        h_info->launches = 2 * iters + 1;
+        h_info->loop_ms = loop_ms;
         h_info->packed = packed ? 1 : 0;
         h_info->overflow_cells = novf;
-        h_info->stream_full_launches = stream_ms_n;
-        h_info->stream_full_ms = stream_ms_n ? (float)(stream_ms_sum / stream_ms_n) : 0.f;
-        if (evp0 && e == cudaSuccess) cudaEventElapsedTime(&h_info->pack_ms, evp0, evp1);
+        h_info->stream_full_launches = stream_ms > 0.f ? 1 : 0;
+        h_info->stream_full_ms = stream_ms;
+        h_info->pack_ms = pack_ms;
     }
-    return rc;
+    return HC_OK;
 }

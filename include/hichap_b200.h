@@ -166,7 +166,8 @@ typedef struct hc_ice_params {
     int32_t ignore_diags;  /* HiCHap passes 1 */
     int32_t max_iters;     /* 200  */
     int32_t rescale_marginals; /* 1 */
-    int32_t poll_every;    /* host polls the device-side done counter every this many launches */
+    int32_t poll_every;    /* dense ICE without its CUDA graph (graph creation failed) and CSR ICE: the host polls the
+                              device-side done counter every this many iterations; the dense graph loop polls nothing */
 } hc_ice_params;
 
 /* Filter marginals of a dense batch of symmetric matrices (one balancing problem per matrix,
@@ -208,13 +209,15 @@ typedef struct hc_ice_run_info {
 /* Iterate every problem of the dense batch to convergence, independently (own loop, scale and
  * early exit -- cooler's _balance_cisonly; one problem == _balance_genomewide).
  * bias: in = initial bias from the filters, out = final weights (NaN for masked bins, divided
- * by sqrt(scale) when rescale_marginals).  All scratch is stream-ordered and library-owned (ABI v1 took a
+ * by sqrt(scale) when rescale_marginals).  All scratch is library-owned (ABI v1 took a
  * `work` pointer here that was never used; v2 drops it).  The reduction over the
  * marginals, the bias update, the rescale and the convergence test all run on the device
- * (stream kernel + per-chromosome update kernel, replayed as a CUDA graph); the host only polls a
- * done counter.  By default the tiles are first re-encoded into uint8 + an overflow list (exact; a
- * quarter of the bytes per iteration; HC_ICE_PACKED=0 streams the int32 tiles instead) in stream-ordered
- * scratch of 1 byte per tile element.  Every mat_ld must be a multiple of 128 elements (512-byte rows). */
+ * (stream kernel + per-chromosome update kernel).  The loop is one launch of a CUDA graph whose WHILE node is ended by
+ * the device once every problem is done or max_iters is reached; the shape's tables, scratch and graph are kept
+ * between calls (per host thread and device), so a repeated call waits on the device once (the mat_ld read) before
+ * its final synchronisation.  By default the tiles are first re-encoded into uint8 + an overflow list (exact; a
+ * quarter of the bytes per iteration; HC_ICE_PACKED=0 streams the int32 tiles instead) in library-owned scratch of
+ * 1 byte per tile element.  Every mat_ld must be a multiple of 128 elements (512-byte rows). */
 int hc_ice_dense_balance(const int32_t* mats, const int64_t* mat_off, const int32_t* mat_n,
                          const int32_t* mat_ld, const int64_t* bin_off, int32_t nprob,
                          const int32_t* h_mat_n, const hc_ice_params* h_params, double* bias,
